@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py — headline benchmark of the B200-native MuZero/Hanoi acting engine.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--mode bf16|fp32|fp32x3]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--mode bf16|fp32|fp32x3] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 \
         --master-port P bench.py --gpus N --steps K --warmup W
 
@@ -16,6 +16,8 @@ so the default 20 timed steps cover more than a second of device time.
 the env words coming from pinned host memory and the step's results (the 32-byte records of its 16 moves, the new env
 words) read back to pinned host memory before the next step starts.
 One JSON line on stdout (rank 0); progress goes to stderr.
+`--dump-outputs DIR` (rank 0) writes what the last timed step handed its caller -- the move records of its moves and the
+env words it left -- as DIR/<name>.npy; the inputs are seeded, so two builds can be compared output for output.
 """
 from __future__ import annotations
 
@@ -38,6 +40,7 @@ DISCOUNT, ALPHA, EPS, TEMPERATURE = 0.8, 0.25, 0.25, 1.0
 FLOP_PER_SIM = 203_776  # SURVEY.md §3.3 / §8d: 101,888 MAC of g + reward/policy/value heads, un-padded
 ENV_BYTES_PER_STEP, ENV_BYTES_PER_RANDOM_STEP = 14, 13  # SURVEY.md §8d: word r/w 8 + action 1 + reward 4 + flags 1
 METRIC, UNIT = "mcts_simulations_per_second", "sims/s"
+DUMP_BUDGET_BYTES = 64_000_000  # --dump-outputs: above this, a fixed, seeded sample of the games is written
 
 
 def tree_bytes_per_sim(depth, latent_bytes=128):
@@ -383,6 +386,38 @@ def network_accuracy(net, n, dev, rows=4096):
     return out
 
 
+def dump_outputs(out_dir, sp, n_moves):
+    """Writes the outputs of the last n_moves SelfPlay.move() calls: every field of their move records (dist.unpack_records)
+    as [move, game] arrays (visits [move, game, 6]), the env words the last move left ([game]) and the global id of every
+    game row (game.npy), all float32 / float64 (exact for every integer field).  Above DUMP_BUDGET_BYTES the rows are a
+    fixed, seeded sample of the games.  The record ring must hold n_moves slots."""
+    import numpy as np
+    import torch
+
+    from muzero_hanoi_b200 import _lib
+
+    assert sp.T >= n_moves
+    per_game = n_moves * (8 + 8 + 4 + 6 * 4 + 3 * 4) + 8 + 8
+    games = np.arange(sp.B)
+    if per_game * sp.B > DUMP_BUDGET_BYTES:
+        games = np.sort(np.random.default_rng(0).choice(sp.B, DUMP_BUDGET_BYTES // per_game, replace=False))
+    idx = torch.as_tensor(games, device=sp.device)
+    slots = torch.as_tensor([(sp.moves_done - n_moves + k) % sp.T for k in range(n_moves)], device=sp.device)
+    raw = sp.records.index_select(0, slots).index_select(1, idx).cpu().numpy()  # uint8 [move, game, 32]
+    rec = raw.view(np.dtype(_lib.RECORD_DTYPE))[..., 0]
+    arrays = {"root_q": rec["root_q"].astype(np.float64), "state": rec["state"].astype(np.float64),
+              "reward": rec["reward"].astype(np.float32), "visits": rec["visits"].astype(np.float32),
+              "action": rec["action"].astype(np.float32), "flags": rec["flags"].astype(np.float32),
+              "game_lo": rec["game_lo"].astype(np.float32),
+              "env_words": sp.env.words.index_select(0, idx).cpu().numpy().view(np.uint32).astype(np.float64),
+              "game": (sp.game_offset + games).astype(np.float64)}
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+    log(f"[bench] wrote {len(arrays)} arrays ({sum(a.nbytes for a in arrays.values()) / 1e6:.1f} MB, {len(games)} of {sp.B} games "
+        f"x {n_moves} moves) to {out_dir}")
+
+
 def run_ours(args):
     import ctypes as C
 
@@ -425,9 +460,12 @@ def run_ours(args):
     if schedule is None:
         schedule = int(args.schedule)
 
+    # --dump-outputs: a record ring that holds every move of a step, so that the last timed step's records are still there
+    ring_slots = max(4, MOVES_PER_STEP) if args.dump_outputs else 4
+
     def make_selfplay(games, offset, sched=schedule):
-        sp_ = SelfPlay(N_DISKS, MAX_STEPS, games, S, weights, DISCOUNT, ALPHA, EPS, TEMPERATURE, seed=1234, ring_slots=4, device=dev,
-                       latent_dtype=latent_dtype, game_offset=offset)
+        sp_ = SelfPlay(N_DISKS, MAX_STEPS, games, S, weights, DISCOUNT, ALPHA, EPS, TEMPERATURE, seed=1234, ring_slots=ring_slots,
+                       device=dev, latent_dtype=latent_dtype, game_offset=offset)
         sp_.mcts.store.set_schedule(sched)
         return sp_
 
@@ -480,6 +518,8 @@ def run_ours(args):
     sims_per_s = world * B * S * moves / (ms * 1e-3)
     depth = mean_leaf_depth(sp)
     log(f"[bench] {ms / args.steps:.2f} ms/step ({ms / moves:.3f} ms/move) -> {sims_per_s:.3e} sims/s; mean leaf depth {depth:.2f}")
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, sp, MOVES_PER_STEP)
 
     # ---- per-kernel device time over one step (CUDA-event pairs recorded by the library on its launch streams)
     def kernel_profile(sp_, sched):
@@ -812,7 +852,13 @@ def main():
     ap.add_argument("--moves-per-step", type=int, default=MOVES_PER_STEP, help="moves of every game per timed step (profiling runs use 1)")
     ap.add_argument("--schedule", default=os.environ.get("HMZ_BENCH_SCHEDULE", "auto"),
                     help="hmz_search_t.schedule: auto | persistent | server | k (stream groups, 1..16; 128 + k = server with k tree groups)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the last timed step's outputs (move records, env words) as DIR/<name>.npy, at most 64 MB (rank 0)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs needs --impl ours")
     MOVES_PER_STEP = max(1, args.moves_per_step)
     claim_stdout()
     if args.impl == "reference":

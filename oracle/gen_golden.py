@@ -25,6 +25,16 @@ GOLDEN = os.path.join(ROOT, "tests", "golden")
 REWARD_CODE = {0: 0, 100: 1, -100 / 1000: 2}
 
 
+def savez_lzma(path, arrays):
+    """np.savez with LZMA members instead of deflate (np.load reads either): the N=10 tables stay well under 1 MB."""
+    import zipfile
+
+    with zipfile.ZipFile(path, "w", compression=zipfile.ZIP_LZMA) as z:
+        for name, a in arrays.items():
+            with z.open(name + ".npy", "w", force_zip64=True) as f:
+                np.lib.format.write_array(f, np.asanyarray(a), allow_pickle=False)
+
+
 # ------------------------------------------------------------------ env + solver
 def gen_env_tables(ref):
     out = {}
@@ -76,7 +86,7 @@ def gen_env_tables(ref):
         print(f"env table N={n}: {n_states * 6 * len(variants)} transitions ok")
     out["max_steps"] = np.int64(max_steps)
     out["counter_before"] = np.array([17, max_steps - 1])
-    np.savez_compressed(os.path.join(GOLDEN, "env_tables.npz"), **out)
+    savez_lzma(os.path.join(GOLDEN, "env_tables.npz"), out)
     # known-answer anchors quoted by the reference (acting_ablations.py:53-60, generate_all_figures.py:78)
     assert [ref.hanoi_solver(s) for s in ((2, 2, 0), (0, 0, 2), (1, 2, 2), (0, 0, 0))] == [7, 3, 1, 7]
 

@@ -171,6 +171,10 @@ class PortHanoi:
     def current_state(self):
         return list(self.c_state)
 
+    def _move_allowed(self, move):
+        """env/hanoi.py:123-139 on the current state."""
+        return move_allowed(self.c_state, move)
+
     def step(self, action):
         assert self.reset_check, "Need to reset env before taking a step"
         moved, stored, ctr, rwd, done, illegal, rc = step_state(
