@@ -390,6 +390,15 @@ int hmz_episode_record(const uint32_t* words, const int32_t* action, const int32
  * finished (HMZ_FLAG_DONE), else 0. */
 int hmz_episode_close(const uint8_t* flags, const int32_t* cur_slot, int64_t n_games, uint8_t* ep_flags, int32_t* ep_len,
                       void* stream);
+/* The episode store filled from move records, e.g. the all-gather of every rank's move: exactly the ep_* writes of
+ * hmz_selfplay_move, for n_games records, record i being global game game_offset + i.  slot = the counter bits of
+ * record.state (clamped to t_max - 1); state / action / flags / visits / root_q are stored there, cur_slot[i] = slot,
+ * ep_len[i] = slot + 1 if HMZ_FLAG_DONE else 0, ep_exp (nullable) = the integer play-policy exponent clamp(1/T, 1, 5) of
+ * `temperature` (HMZ_ERR_UNSUPPORTED if it is not an integer).  A record whose game_lo != (game_offset + i) & 0xFFFF
+ * writes nothing and adds 1 to *mismatch (device int32).  records 16-byte aligned. */
+int hmz_episode_ingest(const hmz_move_record_t* records, int64_t n_games, uint64_t game_offset, int n_disks, int t_max,
+                       double temperature, uint32_t* ep_state, uint8_t* ep_action, uint8_t* ep_flags, uint16_t* ep_visits,
+                       double* ep_root_q, int32_t* cur_slot, int32_t* ep_len, uint8_t* ep_exp, int32_t* mismatch, void* stream);
 /* compute_n_step_returns (utils.py:28-72) and the priorities |f32(return) - f32(rootQ)|
  * (Muzero.py:197-200) of every finished episode (ep_len[g] > 0): returns float64 / priority float32
  * [t_max][n_games].  discount_pow[i] = discount ** i for i in [0, n_step], computed by the HOST libm

@@ -133,6 +133,7 @@ SIGNATURES = {
     "hmz_eval_errors": (_I, [_P, _P, _L, _P, _P]),
     "hmz_episode_record": (_I, [_P, _P, _P, _P, _I, _I, _L, _P, _P, _P, _P, _P, _P, _P]),
     "hmz_episode_close": (_I, [_P, _P, _L, _P, _P, _P]),
+    "hmz_episode_ingest": (_I, [_P, _L, _U64, _I, _I, _D, _P, _P, _P, _P, _P, _P, _P, _P, _P, _P]),
     "hmz_episode_returns": (_I, [_P, _P, _P, _L, _I, _P, _I, _P, _P, _P]),
     "hmz_episode_mc_returns": (_I, [_P, _P, _P, _L, _I, _P, _P, _P, _P]),
     "hmz_episode_rows": (_I, [_P, _P, _L, _L, _I, _P, _P, _P]),

@@ -159,6 +159,38 @@ __global__ void __launch_bounds__(256) selfplay_begin(hmz_search_t s, const floa
   if (a8 == 7) uniform_out[b] = uniform01(seed, game, counter);
 }
 
+// The episode store (include/hmz.h): [t_max][n_games] struct-of-arrays, slot = the game's own step counter.
+struct EpisodeStore {
+  uint32_t* state;
+  uint8_t* action;
+  uint8_t* flags;
+  uint16_t* visits;
+  double* root_q;
+  int32_t* cur_slot;
+  int32_t* len;
+  uint8_t* exp;  // nullable
+  int t_max;
+};
+
+// The episode-store writes of game b's move (hmz_episode_record + hmz_episode_close in one): slot = the counter bits of the
+// env word before the move, clamped to t_max - 1.  The store's two writers, selfplay_finish (from the move itself) and
+// episode_ingest (from its gathered wire record), both go through here so that they cannot drift apart.
+__device__ __forceinline__ void episode_store_move(const EpisodeStore& e, int64_t n, int64_t b, int n_disks, uint32_t w, int action,
+                                                   const int (&visits)[6], double q, uint32_t flags, int exponent) {
+  int t = (int)(w >> (2 * n_disks));
+  if (t >= e.t_max) t = e.t_max - 1;
+  const int64_t at = (int64_t)t * n + b;
+  e.state[at] = w;
+  e.action[at] = (uint8_t)action;
+  e.root_q[at] = q;
+#pragma unroll
+  for (int k = 0; k < 6; ++k) e.visits[at * 6 + k] = (uint16_t)visits[k];
+  e.cur_slot[b] = t;
+  e.flags[at] = (uint8_t)flags;
+  e.len[b] = (flags & HMZ_FLAG_DONE) ? t + 1 : 0;
+  if (e.exp) e.exp[at] = (uint8_t)exponent;
+}
+
 struct FinishArgs {
   hmz_search_t s;
   EnvCfg env;
@@ -169,17 +201,10 @@ struct FinishArgs {
   int32_t* visits;
   double* root_q;
   int32_t* action;
-  uint32_t* ep_state;
-  uint8_t* ep_action;
-  uint8_t* ep_flags;
-  uint16_t* ep_visits;
-  double* ep_root_q;
-  int32_t* ep_cur_slot;
-  int32_t* ep_len;
-  uint8_t* ep_exp;
+  EpisodeStore ep;  // ep.state == nullptr: no episode store
   double temperature;
   uint64_t game_offset;
-  int n_sims, n_disks, ep_t_max, exponent;
+  int n_sims, n_disks, exponent;
 };
 
 // End of a move for every game, one thread each: MCTS/mcts.py:112-126 (root_policy_eval), the move's record, the env step.
@@ -205,21 +230,38 @@ __global__ void __launch_bounds__(256) selfplay_finish(FinishArgs a) {
                           (uint32_t)rp.n[4] | ((uint32_t)rp.n[5] << 16),
                           (uint32_t)rp.action | (o.flags << 8) | ((uint32_t)(game & 0xFFFFu) << 16));
     }
-    if (a.ep_state) {  // episode store: slot = the game's own step counter before the move (hmz_episode_record / _close)
-      int t = (int)(w >> (2 * a.n_disks));
-      if (t >= a.ep_t_max) t = a.ep_t_max - 1;
-      const int64_t at = (int64_t)t * n + b;
-      a.ep_state[at] = w;
-      a.ep_action[at] = (uint8_t)rp.action;
-      a.ep_root_q[at] = q;
-#pragma unroll
-      for (int k = 0; k < 6; ++k) a.ep_visits[at * 6 + k] = (uint16_t)rp.n[k];
-      a.ep_cur_slot[b] = t;
-      a.ep_flags[at] = (uint8_t)o.flags;
-      a.ep_len[b] = (o.flags & HMZ_FLAG_DONE) ? t + 1 : 0;
-      if (a.ep_exp) a.ep_exp[at] = (uint8_t)a.exponent;
-    }
+    if (a.ep.state)  // episode store: slot = the game's own step counter before the move
+      episode_store_move(a.ep, n, b, a.n_disks, w, rp.action, rp.n, q, o.flags, a.exponent);
   }
+}
+
+// Gathered move records -> the episode store, one thread per record: the store writes selfplay_finish makes, read back from
+// the move's 32-byte wire form (two 128-bit loads).  Record b must be global game game_offset + b; one whose game_lo says
+// otherwise writes nothing and is counted in *mismatch.
+__global__ void __launch_bounds__(256) episode_ingest(const hmz_move_record_t* __restrict__ records, int64_t n, uint64_t game_offset,
+                                                     int n_disks, EpisodeStore ep, int exponent, int32_t* __restrict__ mismatch) {
+  const int64_t b = blockIdx.x * (int64_t)blockDim.x + threadIdx.x;
+  if (b >= n) return;
+  const uint4* src = reinterpret_cast<const uint4*>(records + b);
+  const uint4 r0 = __ldcs(src), r1 = __ldcs(src + 1);  // read once: streaming loads
+  if ((r1.w >> 16) != (uint32_t)((game_offset + (uint64_t)b) & 0xFFFFu)) {
+    atomicAdd(mismatch, 1);
+    return;
+  }
+  const int visits[6] = {(int)(r1.x & 0xFFFFu), (int)(r1.x >> 16), (int)(r1.y & 0xFFFFu),
+                         (int)(r1.y >> 16),     (int)(r1.z & 0xFFFFu), (int)(r1.z >> 16)};
+  episode_store_move(ep, n, b, n_disks, r0.z, (int)(r1.w & 0xFFu), visits, __hiloint2double((int)r0.y, (int)r0.x),
+                     (r1.w >> 8) & 0xFFu, exponent);
+}
+
+// clamp(1/T, 1, 5), MCTS/mcts.py:170-172 (1 for T == 0: raw counts); the episode store keeps integer exponents only
+static int play_policy_exponent(const char* who, double temperature, bool store_exp, int* out) {
+  double ex = 1.0;
+  if (temperature > 0.0) ex = 1.0 / temperature < 1.0 ? 1.0 : (1.0 / temperature > 5.0 ? 5.0 : 1.0 / temperature);
+  *out = (int)ex;
+  if (store_exp && (double)*out != ex)
+    return fail(HMZ_ERR_UNSUPPORTED, "%s: the episode store keeps integer play-policy exponents; temperature %g gives %g", who, temperature, ex);
+  return HMZ_OK;
 }
 
 }  // namespace hmz
@@ -295,28 +337,35 @@ int hmz_selfplay_move(const hmz_selfplay_t* sp, uint64_t move_index, void* strea
   fa.visits = sp->visits;
   fa.root_q = sp->root_q;
   fa.action = sp->action;
-  fa.ep_state = sp->ep_state;
-  fa.ep_action = sp->ep_action;
-  fa.ep_flags = sp->ep_flags;
-  fa.ep_visits = sp->ep_visits;
-  fa.ep_root_q = sp->ep_root_q;
-  fa.ep_cur_slot = sp->ep_cur_slot;
-  fa.ep_len = sp->ep_len;
-  fa.ep_exp = sp->ep_exp;
-  {  // clamp(1/T, 1, 5), MCTS/mcts.py:170-172 (1 for T == 0: raw counts); the episode store keeps integer exponents only
-    double ex = 1.0;
-    if (sp->temperature > 0.0) ex = 1.0 / sp->temperature < 1.0 ? 1.0 : (1.0 / sp->temperature > 5.0 ? 5.0 : 1.0 / sp->temperature);
-    fa.exponent = (int)ex;
-    if (sp->ep_exp && (double)fa.exponent != ex)
-      return fail(HMZ_ERR_UNSUPPORTED, "hmz_selfplay_move: the episode store keeps integer play-policy exponents; temperature %g gives %g", sp->temperature, ex);
-  }
+  fa.ep = EpisodeStore{sp->ep_state, sp->ep_action, sp->ep_flags, sp->ep_visits, sp->ep_root_q, sp->ep_cur_slot, sp->ep_len,
+                       sp->ep_exp, sp->ep_t_max};
+  if (int rc = play_policy_exponent("hmz_selfplay_move", sp->temperature, sp->ep_exp != nullptr, &fa.exponent)) return rc;
   fa.temperature = sp->temperature;
   fa.game_offset = sp->game_offset;
   fa.n_sims = sp->n_simulations;
   fa.n_disks = sp->n_disks;
-  fa.ep_t_max = sp->ep_t_max;
   selfplay_finish<<<grid_for(B, 256, 4), 256, 0, st>>>(fa);
   return check_launch("selfplay_finish");
+}
+
+int hmz_episode_ingest(const hmz_move_record_t* records, int64_t n_games, uint64_t game_offset, int n_disks, int t_max,
+                       double temperature, uint32_t* ep_state, uint8_t* ep_action, uint8_t* ep_flags, uint16_t* ep_visits,
+                       double* ep_root_q, int32_t* cur_slot, int32_t* ep_len, uint8_t* ep_exp, int32_t* mismatch, void* stream) {
+  if (!records || !ep_state || !ep_action || !ep_flags || !ep_visits || !ep_root_q || !cur_slot || !ep_len || !mismatch)
+    return fail(HMZ_ERR_INVALID, "hmz_episode_ingest: null pointer");
+  if (n_games < 0 || t_max < 1 || n_disks < 1 || n_disks > HMZ_MAX_DISKS)
+    return fail(HMZ_ERR_INVALID, "hmz_episode_ingest: bad sizes (n_games %lld, t_max %d, n_disks %d)", (long long)n_games, t_max, n_disks);
+  if ((reinterpret_cast<uintptr_t>(records) & 15u) != 0) return fail(HMZ_ERR_INVALID, "hmz_episode_ingest: records must be 16-byte aligned");
+  if (!(temperature >= 0.0 && temperature <= 1.0))  // MCTS/mcts.py:163-166
+    return fail(HMZ_ERR_INVALID, "Expect `temperature` to be in the range [0.0, 1.0], got %g", temperature);
+  int exponent;
+  if (int rc = play_policy_exponent("hmz_episode_ingest", temperature, ep_exp != nullptr, &exponent)) return rc;
+  if (n_games == 0) return HMZ_OK;
+  ProfScope prof_scope(HMZ_PROF_OTHER, stream);
+  const EpisodeStore ep{ep_state, ep_action, ep_flags, ep_visits, ep_root_q, cur_slot, ep_len, ep_exp, t_max};
+  episode_ingest<<<(unsigned)((n_games + 255) / 256), 256, 0, (cudaStream_t)stream>>>(records, n_games, game_offset, n_disks, ep,
+                                                                                     exponent, mismatch);
+  return check_launch("episode_ingest");
 }
 
 }  // extern "C"

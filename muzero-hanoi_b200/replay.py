@@ -39,6 +39,7 @@ class EpisodeStore:
         self.ep_len = torch.zeros(B, dtype=torch.int32, device=dev)
         # play-policy exponent in force when each move was played (SelfPlay fills it); None = use add_episodes' temperature
         self.exp = None
+        self.mismatch = None  # ingest's count of records that were not the game of their row (int32 [1] on the device)
         self.returns = torch.zeros(T, B, dtype=torch.float64, device=dev)
         self.priority = torch.zeros(T, B, dtype=torch.float32, device=dev)
         self.row_base = torch.full((B,), -1, dtype=torch.int64, device=dev)
@@ -56,6 +57,23 @@ class EpisodeStore:
         """After the env step: ep_len[g] = length of the episode that just finished, else 0."""
         check(self.lib.hmz_episode_close(ptr(flags), ptr(self.cur_slot), self.B, ptr(self.flags), ptr(self.ep_len),
                                          current_stream()))
+
+    def ingest(self, records, temperature, game_offset=0):
+        """One move of every game from its move records (uint8 [B, 32], e.g. dist.RecordGather.result(i)): the store
+        writes SelfPlay(episodes=True) makes, with ``temperature`` the one the move was played at.  Record i must be global
+        game ``game_offset + i``; one whose game_lo says otherwise writes nothing and adds 1 to ``self.mismatch``
+        (int32 [1] on the device, never reset here)."""
+        if records.dtype != torch.uint8 or tuple(records.shape) != (self.B, _lib.RECORD_BYTES) or not records.is_contiguous() \
+                or not records.is_cuda:
+            raise ValueError(f"records must be a contiguous uint8 [{self.B}, {_lib.RECORD_BYTES}] device tensor, got "
+                             f"{records.dtype} {tuple(records.shape)} on {records.device}")
+        if self.exp is None:
+            self.exp = torch.ones(self.t_max, self.B, dtype=torch.uint8, device=self.device)
+        if self.mismatch is None:
+            self.mismatch = torch.zeros(1, dtype=torch.int32, device=self.device)
+        check(self.lib.hmz_episode_ingest(ptr(records), self.B, int(game_offset), self.n_disks, self.t_max, float(temperature),
+                                          ptr(self.state), ptr(self.action), ptr(self.flags), ptr(self.visits), ptr(self.root_q),
+                                          ptr(self.cur_slot), ptr(self.ep_len), ptr(self.exp), ptr(self.mismatch), current_stream()))
 
     def post_process(self, n_step, discount):
         """compute_n_step_returns + priorities of every finished episode (ep_len > 0)."""
