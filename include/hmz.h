@@ -458,7 +458,7 @@ int64_t hmz_learner_param_count(int n_disks);
 int64_t hmz_learner_workspace_bytes(int n_disks, int batch, int unroll);
 int hmz_learner_step(float* params, float* grads, float* adam_m, float* adam_v, void* workspace, int n_disks, int batch, int unroll,
                      const float* states, const float* rwds, const int64_t* actions, const float* pi_probs, const float* returns,
-                     const float* priority_w, float lr, float beta1, float beta2, float eps, int64_t step_index,
+                     const float* priority_w, double lr, double beta1, double beta2, double eps, int64_t step_index,
                      float* new_priorities, float* losses_out, int apply_update, void* stream);
 
 #ifdef __cplusplus

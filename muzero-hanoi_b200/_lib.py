@@ -127,7 +127,7 @@ SIGNATURES = {
     "hmz_selfplay_move": (_I, [C.POINTER(SelfPlayDesc), _U64, _P]),
     "hmz_learner_param_count": (_L, [_I]),
     "hmz_learner_workspace_bytes": (_L, [_I, _I, _I]),
-    "hmz_learner_step": (_I, [_P, _P, _P, _P, _P, _I, _I, _I, _P, _P, _P, _P, _P, _P, C.c_float, C.c_float, C.c_float, C.c_float, _L,
+    "hmz_learner_step": (_I, [_P, _P, _P, _P, _P, _I, _I, _I, _P, _P, _P, _P, _P, _P, C.c_double, C.c_double, C.c_double, C.c_double, _L,
                          _P, _P, _I, _P]),
     "hmz_eval_track": (_I, [_P, _I, _L, _P, _P, _P]),
     "hmz_eval_errors": (_I, [_P, _P, _L, _P, _P]),

@@ -92,7 +92,9 @@ __global__ void __launch_bounds__(256) lin_bwd_dx(const float* __restrict__ dY, 
   }
 }
 
-// dW[N,K] += dY[M,N]^T X[M,K];  db[N] += sum_m dY[m,n]   (gradients accumulate over the unroll steps)
+// dW[N,K] += dY[M,N]^T X[M,K];  db[N] += sum_m dY[m,n]   (gradients accumulate over the unroll steps).
+// Each 32-row tile is summed on its own and then added to the running sum, so float32 rounding grows with
+// 32 + M / 32 additions instead of M (the batch is 4,096 rows in the tests).
 __global__ void __launch_bounds__(256) lin_bwd_dw(const float* __restrict__ dY, int ldy, const float* __restrict__ X, int ldx,
                                                   float* __restrict__ dW, float* __restrict__ db, int M, int N, int K) {
   __shared__ float ys[kTile][kTile + 1], xs[kTile][kTile + 1];
@@ -100,6 +102,7 @@ __global__ void __launch_bounds__(256) lin_bwd_dw(const float* __restrict__ dY, 
   const int n0 = blockIdx.y * kTile, k0 = blockIdx.x * kTile;
   float acc[4] = {0.f, 0.f, 0.f, 0.f}, bsum[4] = {0.f, 0.f, 0.f, 0.f};
   for (int m0 = 0; m0 < M; m0 += kTile) {
+    float part[4] = {0.f, 0.f, 0.f, 0.f}, bpart[4] = {0.f, 0.f, 0.f, 0.f};
 #pragma unroll
     for (int i = 0; i < 4; ++i) {
       const int r = ty * 4 + i;  // r = m inside the tile
@@ -113,9 +116,14 @@ __global__ void __launch_bounds__(256) lin_bwd_dw(const float* __restrict__ dY, 
 #pragma unroll
       for (int i = 0; i < 4; ++i) {
         const float y = ys[m][ty * 4 + i];
-        acc[i] = fmaf(y, x, acc[i]);
-        if (blockIdx.x == 0 && tx == 0) bsum[i] += y;
+        part[i] = fmaf(y, x, part[i]);
+        if (blockIdx.x == 0 && tx == 0) bpart[i] += y;
       }
+    }
+#pragma unroll
+    for (int i = 0; i < 4; ++i) {
+      acc[i] += part[i];
+      bsum[i] += bpart[i];
     }
     __syncthreads();
   }
@@ -189,28 +197,29 @@ __global__ void __launch_bounds__(256) normalize_bwd(const float* __restrict__ g
 // first_pred (nullable): |out - target| of unroll step 0 = the new priorities (Muzero.py:253-258).
 __global__ void __launch_bounds__(128) support_loss(const float* __restrict__ logits, const float* __restrict__ target, int t, int unroll,
                                                     const float* __restrict__ coef, float* __restrict__ dlogits,
-                                                    float* __restrict__ loss_acc, float* __restrict__ first_pred, int B) {
+                                                    double* __restrict__ loss_acc, float* __restrict__ first_pred, int B) {
   for (int b = blockIdx.x * blockDim.x + threadIdx.x; b < B; b += gridDim.x * blockDim.x) {
     const float* l = logits + (size_t)b * kSupport;
     float mx = l[0];
     for (int i = 1; i < kSupport; ++i) mx = fmaxf(mx, l[i]);
-    float p[kSupport], den = 0.f;
+    // x = sum_i e_i (i - 16) / sum_i e_i over the unnormalised exponentials, as support_to_scalar (hmz_net.cuh) forms
+    // it: all-equal logits give e_i = 1 and x = 0 exactly (as torch's float32 sum(softmax * linspace) does), so that
+    // row's sign(x) is 0 and it sends no gradient.  Normalising first would leave x a few ulps off 0 with sign -1.
+    float p[kSupport], den = 0.f, num = 0.f;
     for (int i = 0; i < kSupport; ++i) {
       p[i] = expf(l[i] - mx);
       den += p[i];
+      num = fmaf(p[i], (float)(i - (kSupport - 1) / 2), num);
     }
-    float x = 0.f;
-    for (int i = 0; i < kSupport; ++i) {
-      p[i] /= den;
-      x += p[i] * (float)(i - (kSupport - 1) / 2);
-    }
+    const float x = __fdiv_rn(num, den);
+    for (int i = 0; i < kSupport; ++i) p[i] /= den;
     // MuZeroNet._signed_parabolic in the reference's float32 operation order (see signed_parabolic, hmz_net.cuh)
     const float root = __fsqrt_rn(__fadd_rn(1.0f, __fmul_rn(0.004f, __fadd_rn(1.001f, fabsf(x)))));
     const float z = __fsub_rn(__fdiv_rn(__fdiv_rn(root, 2.0f), 0.001f), 500.0f);
     const float sg = x > 0.f ? 1.f : (x < 0.f ? -1.f : 0.f);
     const float out = __fmul_rn(sg, __fsub_rn(__fmul_rn(z, z), 1.0f));
     const float diff = out - target[(size_t)b * unroll + t];
-    atomicAdd(loss_acc, diff * diff);
+    atomicAdd(loss_acc, (double)(diff * diff));
     if (first_pred && t == 0) first_pred[b] = fabsf(diff);
     // d out / d x = sign(x)^2 * 2 z / root  (0 at x == 0, where torch.sign has value and gradient 0)
     const float gx = coef[b] * 2.f * diff * (sg * sg) * 2.f * z / root;
@@ -222,7 +231,7 @@ __global__ void __launch_bounds__(128) support_loss(const float* __restrict__ lo
 //   loss_b += -sum_k t_k log_softmax(l)_k;  dlogits = coef_b (softmax(l) sum_k t_k - t)
 __global__ void __launch_bounds__(128) policy_loss(const float* __restrict__ logits, const float* __restrict__ pi_target, int t, int unroll,
                                                    const float* __restrict__ coef, float* __restrict__ dlogits,
-                                                   float* __restrict__ loss_acc, int B) {
+                                                   double* __restrict__ loss_acc, int B) {
   for (int b = blockIdx.x * blockDim.x + threadIdx.x; b < B; b += gridDim.x * blockDim.x) {
     const float* l = logits + (size_t)b * kActions;
     const float* tg = pi_target + ((size_t)b * unroll + t) * kActions;
@@ -239,7 +248,7 @@ __global__ void __launch_bounds__(128) policy_loss(const float* __restrict__ log
       loss -= tg[i] * (l[i] - lse);
       dlogits[(size_t)b * kActions + i] = coef[b] * (expf(l[i] - lse) * tsum - tg[i]);
     }
-    atomicAdd(loss_acc, loss);
+    atomicAdd(loss_acc, (double)loss);
   }
 }
 
@@ -249,26 +258,33 @@ __global__ void __launch_bounds__(256) make_coef(const float* __restrict__ w, fl
     coef[b] = (w ? w[b] : 1.f) / ((float)B * (float)unroll);
 }
 
-// torch.optim.Adam (default betas / eps, no weight decay, networks.py:69): step_index = 1 for the first update
+// torch.optim.Adam (default betas / eps, no weight decay, networks.py:69), single-tensor form:
+//   exp_avg.lerp_(grad, 1 - beta1);  exp_avg_sq.mul_(beta2).addcmul_(grad, grad, value=1 - beta2);
+//   denom = exp_avg_sq.sqrt() / sqrt(bias2) + eps;  param.addcdiv_(exp_avg, denom, value=-lr / bias1)
+// Every scalar is a double on the host (1 - beta1 in double, not 1 - (float)beta1) rounded once to float32 here.
 __global__ void __launch_bounds__(256) adam_step(float* __restrict__ p, const float* __restrict__ g, float* __restrict__ m,
-                                                 float* __restrict__ v, int64_t n, float lr, float beta1, float beta2, float eps,
-                                                 float bias1, float bias2_sqrt) {
+                                                 float* __restrict__ v, int64_t n, float one_m_beta1, float beta2, float one_m_beta2,
+                                                 float eps, float bias2_sqrt, float neg_step) {
   for (int64_t i = blockIdx.x * (int64_t)blockDim.x + threadIdx.x; i < n; i += (int64_t)gridDim.x * blockDim.x) {
     const float gi = g[i];
-    const float mi = m[i] + (1.f - beta1) * (gi - m[i]);  // torch: exp_avg.lerp_(grad, 1 - beta1)
-    const float vi = beta2 * v[i] + (1.f - beta2) * gi * gi;
+    const float mi = m[i] + one_m_beta1 * (gi - m[i]);
+    const float vi = v[i] * beta2 + one_m_beta2 * gi * gi;
     m[i] = mi;
     v[i] = vi;
     const float denom = sqrtf(vi) / bias2_sqrt + eps;
-    p[i] -= (lr / bias1) * (mi / denom);
+    p[i] += neg_step * (mi / denom);
   }
 }
 
 __global__ void __launch_bounds__(256) zero_f32(float* __restrict__ p, int64_t n) {
   for (int64_t i = blockIdx.x * (int64_t)blockDim.x + threadIdx.x; i < n; i += (int64_t)gridDim.x * blockDim.x) p[i] = 0.f;
 }
-__global__ void scale_losses(float* __restrict__ losses, float inv_b) {
-  if (threadIdx.x < 3) losses[threadIdx.x] *= inv_b;
+__global__ void zero_f64(double* __restrict__ p, int n) {
+  if ((int)threadIdx.x < n) p[threadIdx.x] = 0.0;
+}
+// losses_out = the double sums / B, rounded once
+__global__ void scale_losses(const double* __restrict__ sums, float* __restrict__ losses_out, double inv_b) {
+  if (threadIdx.x < 3) losses_out[threadIdx.x] = (float)(sums[threadIdx.x] * inv_b);
 }
 
 // ---- flat parameter layout: the 20 tensors of MuZeroNet.state_dict() in state_dict order, torch [out][in] ----
@@ -334,7 +350,7 @@ int64_t hmz_learner_workspace_bytes(int n_disks, int batch, int unroll) {
 
 int hmz_learner_step(float* params, float* grads, float* adam_m, float* adam_v, void* workspace, int n_disks, int batch, int unroll,
                      const float* states, const float* rwds, const int64_t* actions, const float* pi_probs, const float* returns,
-                     const float* priority_w, float lr, float beta1, float beta2, float eps, int64_t step_index,
+                     const float* priority_w, double lr, double beta1, double beta2, double eps, int64_t step_index,
                      float* new_priorities, float* losses_out, int apply_update, void* stream) {
   ProfScope prof_scope(HMZ_PROF_OTHER, stream);
   if (!params || !grads || !workspace || !states || !rwds || !actions || !pi_probs || !returns || !losses_out || batch < 1 ||
@@ -379,7 +395,7 @@ int hmz_learner_step(float* params, float* grads, float* adam_m, float* adam_v, 
   float* g_l33b = take(kSupport);
   float* g_l6 = take(kActions);
   float* coef = take(1);
-  float* loss3 = ws;  // value, reward, policy loss sums
+  double* loss3 = (double*)(((uintptr_t)ws + 7) & ~(uintptr_t)7);  // value, reward, policy loss sums (in the 64-byte tail)
 
   auto fwd = [&](const float* X, int ldx, const float* W, const float* b, float* Y, int ldy, int N, int Kd, int relu) {
     lin_fwd<<<gemm_grid(N, B), 256, 0, st>>>(X, ldx, W, b, Y, ldy, B, N, Kd, relu);
@@ -403,7 +419,7 @@ int hmz_learner_step(float* params, float* grads, float* adam_m, float* adam_v, 
   };
 
   zero_f32<<<grid_for(L.total, 256, 8), 256, 0, st>>>(grads, L.total);
-  zero_f32<<<1, 32, 0, st>>>(loss3, 3);
+  zero_f64<<<1, 32, 0, st>>>(loss3, 3);
   make_coef<<<grid_for(B, 256, 1), 256, 0, st>>>(priority_w, coef, B, K);
   // ---- forward
   mlp_fwd(L.rep, states, hid_rep, h_raw0);
@@ -437,14 +453,12 @@ int hmz_learner_step(float* params, float* grads, float* adam_m, float* adam_v, 
   // representation: h_0 has no hook
   normalize_bwd<<<grid_for(B, 256, 1), 256, 0, st>>>(g_h, 1.0f, h_raw0, arg0, g_hraw, B, 0);
   mlp_bwd(L.rep, states, hid_rep, g_hraw, g_hid, nullptr, d_in, 0);
-  scale_losses<<<1, 32, 0, st>>>(loss3, 1.0f / (float)B);
-  if (cudaMemcpyAsync(losses_out, loss3, 3 * sizeof(float), cudaMemcpyDeviceToDevice, st) != cudaSuccess)
-    return fail(HMZ_ERR_CUDA, "hmz_learner_step: loss copy failed");
+  scale_losses<<<1, 32, 0, st>>>(loss3, losses_out, 1.0 / (double)B);
   if (apply_update) {
     // torch evaluates the bias corrections and the step size in double on the host
-    const double bias1 = 1.0 - std::pow((double)beta1, (double)step_index), bias2 = 1.0 - std::pow((double)beta2, (double)step_index);
-    adam_step<<<grid_for(L.total, 256, 8), 256, 0, st>>>(params, grads, adam_m, adam_v, L.total, lr, beta1, beta2, eps, (float)bias1,
-                                                         (float)std::sqrt(bias2));
+    const double bias1 = 1.0 - std::pow(beta1, (double)step_index), bias2 = 1.0 - std::pow(beta2, (double)step_index);
+    adam_step<<<grid_for(L.total, 256, 8), 256, 0, st>>>(params, grads, adam_m, adam_v, L.total, (float)(1.0 - beta1), (float)beta2,
+                                                         (float)(1.0 - beta2), (float)eps, (float)std::sqrt(bias2), (float)(-lr / bias1));
   }
   (void)g_x;
   return check_launch("hmz_learner_step");
