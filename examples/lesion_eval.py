@@ -33,11 +33,18 @@ def main():
     print("trained: mean episode length of the last 20 loops %.1f" % np.mean([h[1] for h in hist[-20:]]))
     net.load_state_dict({k: v.cpu() for k, v in mz.learner.state_dict().items()})
     budgets = [5, 10, 30, 80]
-    for name, flags in [("intact", (False, False, False)), ("policy lesion", (True, False, False)),
-                        ("value lesion", (False, True, False)), ("reward lesion", (False, False, True)),
-                        ("policy + value lesion", (True, True, False))]:
+    settings = [("intact", (False, False, False)), ("policy lesion", (True, False, False)), ("value lesion", (False, True, False)),
+                ("reward lesion", (False, False, True)), ("policy + value lesion", (True, True, False))]
+    # the whole grid (networks x budgets) as one batch of searches; each condition's numbers are those of
+    # acting.get_results(weights, N, 200, episodes, [budget], 0.0, seed=3)
+    conditions = []
+    for _, flags in settings:
         lesioned = acting.ablate_networks(*flags, copy.deepcopy(net))  # acting_ablations.py:29-45
-        data = acting.get_results(PackedWeights(lesioned.state_dict(), N), N, 200, args.episodes, budgets, 0.0, seed=3)
+        weights = PackedWeights(lesioned.state_dict(), N)
+        conditions += [dict(weights=weights, n_simulations=n, episode=args.episodes) for n in budgets]
+    results = acting.get_results_grid(conditions, N, 200, 0.0, seed=3)
+    for k, (name, _) in enumerate(settings):
+        data = [row for r in results[k * len(budgets):(k + 1) * len(budgets)] for row in r]
         print("%-22s " % name + "  ".join("S=%d: %.2f" % (n, e) for n, e in data))
 
 

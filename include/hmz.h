@@ -283,6 +283,41 @@ int hmz_search_run(const hmz_search_t* s, const void* weights, int mode, int n_s
                    const double* ucb_table, double discount, void* stream);
 /* (Scheduling is chosen per call by hmz_search_t.schedule.) */
 
+/* ------------------------------------------------------------------ heterogeneous batches ---
+ * One search batch over several networks and simulation budgets (the lesion-experiment grid of
+ * acting_ablations.get_results run as one batch).  The batch is cut into blocks of 256 searches:
+ *   - every block uses ONE weight set: sets are packed (hmz_weights_pack, same n_disks and mode) into one
+ *     device blob at a fixed stride, set k at weights + k * weight_stride;
+ *   - every search has its own budget, in [1, host_block_budget[its block]];
+ *   - blocks are ordered by non-increasing budget, so simulation s runs over a prefix of the batch: the
+ *     blocks whose budget is greater than s.
+ * A search with budget b runs simulations 0 .. b-1 exactly as hmz_search_run with n_simulations = b
+ * would run it alone; its node records and latents above record b are unspecified afterwards. */
+typedef struct hmz_multi {
+  const uint16_t* block_set;         /* device [n_searches / 256]: weight set of each block, in [0, n_sets)       */
+  const uint16_t* budget;            /* device [n_searches]: simulations of each search (nullable for initial) */
+  const int32_t* host_block_budget;  /* HOST [n_searches / 256]: max budget of each block, non-increasing        */
+  int64_t weight_stride;             /* bytes between sets: >= hmz_weights_packed_bytes, a multiple of 256      */
+  int32_t n_sets;                    /* weight sets in the blob (>= 1)                                          */
+  int32_t n_disks;                   /* disk count the sets were packed for                                     */
+} hmz_multi_t;
+
+/* hmz_net_initial from packed env words with each block's weight set (n = n_searches of m, a multiple of 256;
+ * host_block_budget and budget are not read). */
+int hmz_net_initial_multi(const void* weights, const hmz_multi_t* m, int mode, const uint32_t* words, void* latents_out,
+                          int64_t out_rows_per_item, int latent_dtype, float* p0, float* v0, int64_t n, void* stream);
+/* hmz_search_run over a heterogeneous batch: simulation s launches the select -> MLP -> backup chain over the
+ * blocks whose budget is greater than s; within them a search backs up simulation s only if s < budget and
+ * selects the next leaf only if s + 1 < budget.  s->n_records >= host_block_budget[0] + 1.  Schedules: 0 and
+ * k in [1, 16] (stream groups of whole blocks); HMZ_SCHEDULE_PERSISTENT / _SERVER: HMZ_ERR_UNSUPPORTED. */
+int hmz_search_run_multi(const hmz_search_t* s, const hmz_multi_t* m, const void* weights, int mode, const double* ucb_table,
+                         double discount, void* stream);
+/* hmz_search_root_policy with root_q = root_W / budget[b] per search; pow_table (nullable) has
+ * host_block_budget[0] + 1 rows. */
+int hmz_search_root_policy_multi(const hmz_search_t* s, const hmz_multi_t* m, double temperature, int deterministic,
+                                 const double* uniforms, const double* pow_table, int32_t* visits, double* pi, double* root_q,
+                                 int32_t* action, void* stream);
+
 /* Tooling only: with HMZ_TC_TIMELINE=1 in the environment, CTA 0 of the tensor-core kernel records
  * clock64() at its phase boundaries; this copies the 96 marks of the last launch to the host. */
 int hmz_debug_tc_timeline(unsigned long long* host_out);
@@ -322,6 +357,11 @@ int hmz_debug_div_check(uint64_t n_samples, uint64_t seed, unsigned long long* c
 int hmz_rng_dirichlet(double* out, int64_t n, double alpha, uint64_t seed, uint64_t counter, uint64_t item_offset, void* stream);
 /* One uniform double in [0, 1) per item (the draw of np.random.choice, MCTS/mcts.py:120). */
 int hmz_rng_uniform(double* out, int64_t n, uint64_t seed, uint64_t counter, uint64_t item_offset, void* stream);
+/* The same draw with its key given per item: out[i] = the uniform of item item[i] at counter counter_hi[i] | counter_lo,
+ * i.e. element item[i] - o of hmz_rng_uniform(seed, counter_hi[i] | counter_lo, item_offset o).  Items of different
+ * streams (a batch of several experiments) draw in one launch. */
+int hmz_rng_uniform_keyed(double* out, int64_t n, uint64_t seed, const uint64_t* counter_hi, uint64_t counter_lo,
+                          const uint64_t* item, void* stream);
 /* Tests only: n_blocks raw Philox4x32-10 blocks; counters_keys uint32 [n_blocks][6] = counter words 0..3, key words
  * 0..1; out uint32 [n_blocks][4] (known-answer vectors of Salmon et al. 2011). */
 int hmz_debug_philox(const uint32_t* counters_keys, uint32_t* out, int n_blocks, void* stream);

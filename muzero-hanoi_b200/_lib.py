@@ -79,8 +79,19 @@ class SelfPlayDesc(C.Structure):
         ("goal_peg", C.c_int32), ("n_simulations", C.c_int32), ("ep_t_max", C.c_int32), ("reset_word", C.c_uint32),
         ("reserved", C.c_int32)]
 
+
+class MultiDesc(C.Structure):
+    """hmz_multi_t — a heterogeneous search batch: one weight set per 256-search block, one budget per search."""
+
+    _fields_ = [("block_set", C.c_void_p), ("budget", C.c_void_p), ("host_block_budget", C.c_void_p), ("weight_stride", C.c_int64),
+                ("n_sets", C.c_int32), ("n_disks", C.c_int32)]
+
+
+BLOCK = 256  # searches per block of a heterogeneous batch (one weight set each)
+
 _P, _I, _L, _U32, _U64, _D = C.c_void_p, C.c_int, C.c_int64, C.c_uint32, C.c_uint64, C.c_double
 _SD = C.POINTER(SearchDesc)
+_MD = C.POINTER(MultiDesc)
 
 # name -> (restype, argtypes); mirrors include/hmz.h one to one
 SIGNATURES = {
@@ -121,6 +132,10 @@ SIGNATURES = {
     "hmz_debug_tree_timeline": (_I, [C.c_longlong, _P]),
     "hmz_debug_div_check": (_I, [_U64, _U64, _P, _P]),
     "hmz_search_run": (_I, [_SD, _P, _I, _I, _P, _D, _P]),
+    "hmz_net_initial_multi": (_I, [_P, _MD, _I, _P, _P, _L, _I, _P, _P, _L, _P]),
+    "hmz_search_run_multi": (_I, [_SD, _MD, _P, _I, _P, _D, _P]),
+    "hmz_search_root_policy_multi": (_I, [_SD, _MD, _D, _I, _P, _P, _P, _P, _P, _P, _P]),
+    "hmz_rng_uniform_keyed": (_I, [_P, _L, _U64, _P, _U64, _P, _P]),
     "hmz_rng_dirichlet": (_I, [_P, _L, _D, _U64, _U64, _U64, _P]),
     "hmz_rng_uniform": (_I, [_P, _L, _U64, _U64, _U64, _P]),
     "hmz_debug_philox": (_I, [_P, _P, _I, _P]),

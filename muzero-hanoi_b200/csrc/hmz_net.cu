@@ -166,8 +166,16 @@ __device__ __forceinline__ void run_heads(NetSmem& s, const float* __restrict__ 
   if (row_ok) v[row0 + m] = support_to_scalar([&](int i) { return s.lg[i * kRowStride + m]; });
 }
 
+// Heterogeneous batches (hmz_multi_t): the weight set of this CTA's 256-row block (kRows divides 256).
+__device__ __forceinline__ const float* set_weights(const float* W, const uint16_t* block_set, int64_t weight_stride) {
+  if (block_set == nullptr) return W;
+  const int64_t block = (int64_t)blockIdx.x * kRows / 256;
+  return reinterpret_cast<const float*>(reinterpret_cast<const char*>(W) + (int64_t)block_set[block] * weight_stride);
+}
+
 __global__ void __launch_bounds__(kNetThreads, 3)
-net_recurrent_fp32(const float* __restrict__ W, const void* __restrict__ lat_in, int64_t in_rows_per_item,
+net_recurrent_fp32(const float* __restrict__ W_base, const uint16_t* __restrict__ block_set, int64_t weight_stride,
+                   const void* __restrict__ lat_in, int64_t in_rows_per_item,
                    const uint16_t* __restrict__ in_row, const uint8_t* __restrict__ actions, void* lat_out,
                    int64_t out_rows_per_item, int64_t out_row, int latent_dtype, float* __restrict__ r,
                    float* __restrict__ p, float* __restrict__ v, int64_t n) {
@@ -175,6 +183,7 @@ net_recurrent_fp32(const float* __restrict__ W, const void* __restrict__ lat_in,
   NetSmem& s = *reinterpret_cast<NetSmem*>(smem_raw);
   using L = Fp32Layout;
   const int64_t row0 = (int64_t)blockIdx.x * kRows;
+  const float* __restrict__ W = set_weights(W_base, block_set, weight_stride);
   {  // gather the parent latents: lane <-> row, warp <-> 8-feature chunk
     const int m = threadIdx.x & 31, c = threadIdx.x >> 5;
     int64_t item = row0 + m;
@@ -216,13 +225,14 @@ net_recurrent_fp32(const float* __restrict__ W, const void* __restrict__ lat_in,
 }
 
 __global__ void __launch_bounds__(kNetThreads, 3)
-net_initial_fp32(const float* __restrict__ W, int n_disks, const uint32_t* __restrict__ words,
+net_initial_fp32(const float* __restrict__ W_base, const uint16_t* __restrict__ block_set, int64_t weight_stride, int n_disks, const uint32_t* __restrict__ words,
                  const float* __restrict__ obs, void* lat_out, int64_t out_rows_per_item, int latent_dtype,
                  float* __restrict__ p0, float* __restrict__ v0, int64_t n) {
   extern __shared__ __align__(16) unsigned char smem_raw[];
   NetSmem& s = *reinterpret_cast<NetSmem*>(smem_raw);
   using L = Fp32Layout;
   const int64_t row0 = (int64_t)blockIdx.x * kRows;
+  const float* __restrict__ W = set_weights(W_base, block_set, weight_stride);
   const int width = 3 * n_disks;
   const float* w1 = W + L::rep_w1;
   const float* b1 = W + L::rep_b1(n_disks);
@@ -365,6 +375,62 @@ int hmz_net_initial(const void* weights, int mode, int n_disks, const uint32_t* 
                     void* latents_out, int64_t out_rows_per_item, int latent_dtype, float* p0, float* v0, int64_t n,
                     void* stream) {
   ProfScope prof_scope(HMZ_PROF_NET_INITIAL, stream);
+  return net_initial_sets(weights, nullptr, 0, mode, n_disks, words, obs, latents_out, out_rows_per_item, latent_dtype, p0, v0, n,
+                          stream);
+}
+
+int hmz_net_initial_multi(const void* weights, const hmz_multi_t* m, int mode, const uint32_t* words, void* latents_out,
+                          int64_t out_rows_per_item, int latent_dtype, float* p0, float* v0, int64_t n, void* stream) {
+  ProfScope prof_scope(HMZ_PROF_NET_INITIAL, stream);
+  if (int rc = check_multi(m, n, mode, 0, false, "hmz_net_initial_multi")) return rc;
+  if (n > 0 && !words) return fail(HMZ_ERR_INVALID, "hmz_net_initial_multi: null words");
+  return net_initial_sets(weights, m->block_set, m->weight_stride, mode, m->n_disks, words, nullptr, latents_out, out_rows_per_item,
+                          latent_dtype, p0, v0, n, stream);
+}
+
+int hmz_net_recurrent(const void* weights, int mode, const void* latents_in, int64_t in_rows_per_item,
+                      const uint16_t* in_row, const uint8_t* actions, void* latents_out, int64_t out_rows_per_item,
+                      int64_t out_row, int latent_dtype, float* r, float* p, float* v, int64_t n, void* stream) {
+  ProfScope prof_scope(HMZ_PROF_NET_RECURRENT, stream);
+  return net_recurrent_sets(weights, nullptr, 0, mode, latents_in, in_rows_per_item, in_row, actions, latents_out, out_rows_per_item,
+                            out_row, latent_dtype, r, p, v, n, stream);
+}
+
+}  // extern "C"
+
+namespace hmz {
+
+int check_multi(const hmz_multi_t* m, int64_t n_searches, int mode, int n_records, bool need_budget, const char* who) {
+  if (!m) return fail(HMZ_ERR_INVALID, "%s: null hmz_multi_t", who);
+  if (n_searches < 0 || n_searches % 256 != 0)
+    return fail(HMZ_ERR_INVALID, "%s: n_searches=%lld is not a multiple of 256", who, (long long)n_searches);
+  if (m->n_sets < 1) return fail(HMZ_ERR_INVALID, "%s: n_sets=%d < 1", who, m->n_sets);
+  if (mode >= 0) {  // the entry point reads weights (mode < 0: the root policy reads none)
+    const int64_t need = hmz_weights_packed_bytes(m->n_disks, mode);
+    if (need < 0) return fail(HMZ_ERR_INVALID, "%s: no packed layout for n_disks=%d, mode=%d", who, m->n_disks, mode);
+    // >= one packed set, and a multiple of 256 bytes so that every set keeps the alignment of the blob's bulk copies
+    if (m->weight_stride < need || m->weight_stride % 256 != 0)
+      return fail(HMZ_ERR_INVALID, "%s: weight_stride=%lld must be >= %lld and a multiple of 256", who, (long long)m->weight_stride,
+                  (long long)need);
+    if (n_searches > 0 && !m->block_set) return fail(HMZ_ERR_INVALID, "%s: null block_set", who);
+  }
+  if (!need_budget || n_searches == 0) return HMZ_OK;
+  if (!m->budget || !m->host_block_budget) return fail(HMZ_ERR_INVALID, "%s: null budget / host_block_budget", who);
+  const int64_t blocks = n_searches / 256;
+  for (int64_t k = 0; k < blocks; ++k) {
+    const int32_t b = m->host_block_budget[k];
+    if (b < 1 || b + 1 > n_records)
+      return fail(HMZ_ERR_INVALID, "%s: block %lld budget %d outside [1, n_records - 1 = %d]", who, (long long)k, b, n_records - 1);
+    if (k > 0 && b > m->host_block_budget[k - 1])
+      return fail(HMZ_ERR_INVALID, "%s: block budgets must not increase (block %lld: %d after %d)", who, (long long)k, b,
+                  m->host_block_budget[k - 1]);
+  }
+  return HMZ_OK;
+}
+
+int net_initial_sets(const void* weights, const uint16_t* block_set, int64_t weight_stride, int mode, int n_disks,
+                     const uint32_t* words, const float* obs, void* latents_out, int64_t out_rows_per_item, int latent_dtype,
+                     float* p0, float* v0, int64_t n, void* stream) {
   if (n == 0) return HMZ_OK;
   if (!weights || (!words && !obs) || !latents_out || !p0 || !v0 || n < 0 || n_disks < 1 || n_disks > HMZ_MAX_DISKS ||
       out_rows_per_item < 1 || (latent_dtype != HMZ_LATENT_F32 && latent_dtype != HMZ_LATENT_BF16))
@@ -374,22 +440,24 @@ int hmz_net_initial(const void* weights, int mode, int n_disks, const uint32_t* 
   // throughput mode with packed env words: the tcgen05 kernel (bf16 representation + policy + value);
   // float observations (drop-in B = 1 views, arbitrary input vectors) keep the float32 kernel below
   if (mode == HMZ_MODE_BF16 && words != nullptr)
-    return tc_net_initial(weights, n_disks, words, latents_out, out_rows_per_item, latent_dtype, p0, v0, n, (cudaStream_t)stream);
+    return tc_net_initial(weights, n_disks, words, latents_out, out_rows_per_item, latent_dtype, p0, v0, n, (cudaStream_t)stream,
+                          block_set, weight_stride);
   if (mode == HMZ_MODE_FP32X3 && words != nullptr)  // float32 accuracy on tcgen05, like the recurrent inference of this mode
-    return x3::net_initial(weights, n_disks, words, latents_out, out_rows_per_item, latent_dtype, p0, v0, n, (cudaStream_t)stream);
+    return x3::net_initial(weights, n_disks, words, latents_out, out_rows_per_item, latent_dtype, p0, v0, n, (cudaStream_t)stream,
+                           block_set, weight_stride);
   if (int rc = ensure_smem_optin()) return rc;
   const unsigned grid = (unsigned)((n + kRows - 1) / kRows);
   const int64_t w32_off = mode == HMZ_MODE_BF16 ? tc_fp32_offset_bytes() : (mode == HMZ_MODE_FP32X3 ? x3::fp32_offset_bytes() : 0);
   const float* w32 = reinterpret_cast<const float*>(reinterpret_cast<const char*>(weights) + w32_off);
   net_initial_fp32<<<grid, kNetThreads, sizeof(NetSmem), (cudaStream_t)stream>>>(
-      w32, n_disks, words, obs, latents_out, out_rows_per_item, latent_dtype, p0, v0, n);
+      w32, block_set, weight_stride, n_disks, words, obs, latents_out, out_rows_per_item, latent_dtype, p0, v0, n);
   return check_launch("net_initial_fp32");
 }
 
-int hmz_net_recurrent(const void* weights, int mode, const void* latents_in, int64_t in_rows_per_item,
-                      const uint16_t* in_row, const uint8_t* actions, void* latents_out, int64_t out_rows_per_item,
-                      int64_t out_row, int latent_dtype, float* r, float* p, float* v, int64_t n, void* stream) {
-  ProfScope prof_scope(HMZ_PROF_NET_RECURRENT, stream);
+int net_recurrent_sets(const void* weights, const uint16_t* block_set, int64_t weight_stride, int mode, const void* latents_in,
+                       int64_t in_rows_per_item, const uint16_t* in_row, const uint8_t* actions, void* latents_out,
+                       int64_t out_rows_per_item, int64_t out_row, int latent_dtype, float* r, float* p, float* v, int64_t n,
+                       void* stream) {
   if (n == 0) return HMZ_OK;
   if (!weights || !latents_in || !actions || !latents_out || !r || !p || !v || n < 0 || in_rows_per_item < 1 ||
       out_rows_per_item < 1 || out_row < 0 || out_row >= out_rows_per_item ||
@@ -397,17 +465,17 @@ int hmz_net_recurrent(const void* weights, int mode, const void* latents_in, int
     return fail(HMZ_ERR_INVALID, "hmz_net_recurrent: bad arguments");
   if (mode == HMZ_MODE_BF16)
     return tc_net_recurrent(weights, latents_in, in_rows_per_item, in_row, actions, latents_out, out_rows_per_item,
-                            out_row, latent_dtype, r, p, v, n, (cudaStream_t)stream);
+                            out_row, latent_dtype, r, p, v, n, (cudaStream_t)stream, block_set, weight_stride);
   if (mode == HMZ_MODE_FP32X3)
     return x3::net_recurrent(weights, latents_in, in_rows_per_item, in_row, actions, latents_out, out_rows_per_item, out_row,
-                             latent_dtype, r, p, v, n, (cudaStream_t)stream);
+                             latent_dtype, r, p, v, n, (cudaStream_t)stream, block_set, weight_stride);
   if (mode != HMZ_MODE_FP32) return fail(HMZ_ERR_INVALID, "hmz_net_recurrent: unknown mode %d", mode);
   if (int rc = ensure_smem_optin()) return rc;
   const unsigned grid = (unsigned)((n + kRows - 1) / kRows);
   net_recurrent_fp32<<<grid, kNetThreads, sizeof(NetSmem), (cudaStream_t)stream>>>(
-      (const float*)weights, latents_in, in_rows_per_item, in_row, actions, latents_out, out_rows_per_item, out_row,
+      (const float*)weights, block_set, weight_stride, latents_in, in_rows_per_item, in_row, actions, latents_out, out_rows_per_item, out_row,
       latent_dtype, r, p, v, n);
   return check_launch("net_recurrent_fp32");
 }
 
-}  // extern "C"
+}  // namespace hmz

@@ -166,7 +166,8 @@ int tc_head_split_allowed() { return tl_split_allowed; }
 
 int tc_net_recurrent(const void* weights, const void* lat_in, int64_t in_rows_per_item, const uint16_t* in_row,
                      const uint8_t* actions, void* lat_out, int64_t out_rows_per_item, int64_t out_row,
-                     int latent_dtype, float* r, float* p, float* v, int64_t n, cudaStream_t stream) {
+                     int latent_dtype, float* r, float* p, float* v, int64_t n, cudaStream_t stream, const uint16_t* block_set,
+                     int64_t weight_stride) {
   int smem = 0, n_pairs = 0;
   if (int rc = tc_prepare(&smem)) return rc;
   unsigned grid = tc_grid(n, &n_pairs, tc_passes());
@@ -176,6 +177,8 @@ int tc_net_recurrent(const void* weights, const void* lat_in, int64_t in_rows_pe
   a.head_split = (split_on && tl_split_allowed && 3 * n_pairs <= sm_count()) ? 3 : 1;
   if (a.head_split == 3) grid = 3u * (unsigned)n_pairs;
   a.wsec = (const uint8_t*)weights;
+  a.block_set = block_set;
+  a.weight_stride = weight_stride;
   a.lat_in = lat_in;
   a.in_rows_per_item = in_rows_per_item;
   a.in_row = in_row;
@@ -197,12 +200,15 @@ int tc_net_recurrent(const void* weights, const void* lat_in, int64_t in_rows_pe
 }
 
 int tc_net_initial(const void* weights, int n_disks, const uint32_t* words, void* lat_out, int64_t out_rows_per_item,
-                   int latent_dtype, float* p0, float* v0, int64_t n, cudaStream_t stream) {
+                   int latent_dtype, float* p0, float* v0, int64_t n, cudaStream_t stream, const uint16_t* block_set,
+                   int64_t weight_stride) {
   int smem = 0, n_pairs = 0;
   if (int rc = tc_prepare(&smem)) return rc;
   const unsigned grid = tc_grid(n, &n_pairs);
   tc::v4::TcArgs a{};
   a.wsec = (const uint8_t*)weights;
+  a.block_set = block_set;
+  a.weight_stride = weight_stride;
   a.in_rows_per_item = 1;
   a.words = words;
   a.n_disks = n_disks;

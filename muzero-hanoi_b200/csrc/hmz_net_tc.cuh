@@ -352,6 +352,8 @@ struct TcArgs {
                               // chain of a pass shrinks from four networks to two while idle SMs do the redundant work; else 1
   int timeline;               // tooling / PDL switches of the stand-alone kernels
   unsigned long long* gantt;  // tooling (hmz_debug_gantt), nullable
+  const uint16_t* block_set;  // nullable (stand-alone kernels only): weight set of each tile pair (hmz_multi_t), at
+  int64_t weight_stride;      // wsec + block_set[pair] * weight_stride
 };
 
 // Hand-off state of the persistent search kernel (hmz_persist.cu), in global memory; zeroed before every launch.
@@ -581,7 +583,9 @@ __device__ __forceinline__ void net_tc_body(const TcArgs& a, const PersistCtl& p
     // holds the reward / policy blocks; cnt = loads issued into a slot so far (a reload waits for the previous use's MMAs).
     uint32_t cnt[2][2] = {{0u, 0u}, {0u, 0u}};
     int issued = 0;
-    for (int pass = 0; pass < n_pass; ++pass) {
+    PassIter load_it{first_pair(0), 0};  // the pair of the pass whose blocks are loaded (the MMA warps may still run the one before)
+    for (int pass = 0; pass < n_pass; ++pass, next_item(load_it)) {
+      const uint8_t* __restrict__ wpass = (!kPersist && a.block_set != nullptr) ? wsec + (int64_t)a.block_set[load_it.pair] * a.weight_stride : wsec;
 #pragma unroll
       for (int i = 0; i < 8; ++i) {
         if (kInitial && (i >> 1) == 1) continue;  // no reward head at the root
@@ -596,7 +600,7 @@ __device__ __forceinline__ void net_tc_body(const TcArgs& a, const PersistCtl& p
         if (u >= 1u) mbar_wait(&s.bar_wfree[kind][slot], (u - 1u) & 1u);
         const uint32_t off = (kInitial && i < 2) ? (i == 0 ? kWh1 : kWh2) : c_block_off[i];  // representation_net at the root
         uint8_t* dst = kind ? (slot ? s.ws1 : s.ws0) : s.wf[slot];
-        if (elect_one()) tma_load(dst, wsec + off, c_block_bytes[i], &s.bar_wfull[kind][slot]);
+        if (elect_one()) tma_load(dst, wpass + off, c_block_bytes[i], &s.bar_wfull[kind][slot]);
         __syncwarp();
         cnt[kind][slot] = u + 1u;
       }

@@ -86,6 +86,8 @@ struct Args {
                    // then ONE head each (reward + the latent rows / value / policy), as in the bf16 kernel: the dependent chain
                    // of a launch shrinks from sixteen chunks to eight while idle SMs do the redundant work; else 1
   int timeline;  // tooling (HMZ_X3_TIMELINE=1): CTA 0 records clock64() at the phase boundaries of its first tile
+  const uint16_t* block_set;  // nullable: weight set of each 256-row block (hmz_multi_t), at wsec + block_set[tile / 2] * weight_stride
+  int64_t weight_stride;
 };
 
 static __device__ unsigned long long g_x3_timeline[160];
@@ -325,7 +327,12 @@ __global__ void __launch_bounds__(kThreads, 1) net_x3(const __grid_constant__ Ar
     auto load = [&](uint32_t G, bool second) {  // chunk counter of this CTA: slot G & 1, use G >> 1
       const int g = chunk_of((int)(G % (uint32_t)n_steps));
       const uint32_t slot = G & 1u, use = G >> 1;
-      const uint8_t* blk = a.wsec + (size_t)((kInitial && g < 4) ? kRepBlock0 + g : g) * kBlockStride;
+      const uint8_t* wsec = a.wsec;
+      if (a.block_set != nullptr) {  // the tile this chunk belongs to: the CTA's (G / n_steps)-th
+        const int tile = cta + (int)(G / (uint32_t)n_steps) * n_cta;
+        wsec += (int64_t)a.block_set[tile >> 1] * a.weight_stride;
+      }
+      const uint8_t* blk = wsec + (size_t)((kInitial && g < 4) ? kRepBlock0 + g : g) * kBlockStride;
       if (!second) {
         if (use >= 1u) mbar_wait(&s.bar_w1free[slot], (use - 1u) & 1u);
         if (G < (uint32_t)n_steps) X3_TL(128 + g);
@@ -726,11 +733,13 @@ static int prepare(int* smem_bytes) {
 
 int net_recurrent(const void* weights, const void* lat_in, int64_t in_rows_per_item, const uint16_t* in_row,
                   const uint8_t* actions, void* lat_out, int64_t out_rows_per_item, int64_t out_row, int latent_dtype,
-                  float* r, float* p, float* v, int64_t n, cudaStream_t stream) {
+                  float* r, float* p, float* v, int64_t n, cudaStream_t stream, const uint16_t* block_set, int64_t weight_stride) {
   int smem = 0;
   if (int rc = prepare(&smem)) return rc;
   Args a{};
   a.wsec = (const uint8_t*)weights;
+  a.block_set = block_set;
+  a.weight_stride = weight_stride;
   a.lat_in = lat_in;
   a.in_rows_per_item = in_rows_per_item;
   a.in_row = in_row;
@@ -757,11 +766,13 @@ int net_recurrent(const void* weights, const void* lat_in, int64_t in_rows_per_i
 }
 
 int net_initial(const void* weights, int n_disks, const uint32_t* words, void* lat_out, int64_t out_rows_per_item,
-                int latent_dtype, float* p0, float* v0, int64_t n, cudaStream_t stream) {
+                int latent_dtype, float* p0, float* v0, int64_t n, cudaStream_t stream, const uint16_t* block_set, int64_t weight_stride) {
   int smem = 0;
   if (int rc = prepare(&smem)) return rc;
   Args a{};
   a.wsec = (const uint8_t*)weights;
+  a.block_set = block_set;
+  a.weight_stride = weight_stride;
   a.in_rows_per_item = 1;
   a.words = words;
   a.n_disks = n_disks;

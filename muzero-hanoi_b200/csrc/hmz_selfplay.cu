@@ -109,6 +109,13 @@ __global__ void __launch_bounds__(256) rng_uniform(double* __restrict__ out, int
     out[i] = uniform01(seed, item_offset + (uint64_t)i, counter);
 }
 
+__global__ void __launch_bounds__(256) rng_uniform_keyed(double* __restrict__ out, int64_t n, uint64_t seed,
+                                                        const uint64_t* __restrict__ counter_hi, uint64_t counter_lo,
+                                                        const uint64_t* __restrict__ item) {
+  for (int64_t i = blockIdx.x * (int64_t)blockDim.x + threadIdx.x; i < n; i += (int64_t)gridDim.x * blockDim.x)
+    out[i] = uniform01(seed, item[i], counter_hi[i] | counter_lo);
+}
+
 // Tests: raw Philox4x32-10 blocks (known-answer vectors of Salmon et al. 2011, Random123 kat_vectors).
 __global__ void philox_blocks(const uint32_t* __restrict__ ctr_key, uint32_t* __restrict__ out, int n) {
   const int i = blockIdx.x * blockDim.x + threadIdx.x;
@@ -284,6 +291,15 @@ int hmz_rng_uniform(double* out, int64_t n, uint64_t seed, uint64_t counter, uin
   if (!out || n < 0) return fail(HMZ_ERR_INVALID, "hmz_rng_uniform: bad arguments");
   rng_uniform<<<grid_for(n, 256, 8), 256, 0, (cudaStream_t)stream>>>(out, n, seed, counter, item_offset);
   return check_launch("rng_uniform");
+}
+
+int hmz_rng_uniform_keyed(double* out, int64_t n, uint64_t seed, const uint64_t* counter_hi, uint64_t counter_lo,
+                          const uint64_t* item, void* stream) {
+  ProfScope prof_scope(HMZ_PROF_OTHER, stream);
+  if (n == 0) return HMZ_OK;
+  if (!out || !counter_hi || !item || n < 0) return fail(HMZ_ERR_INVALID, "hmz_rng_uniform_keyed: bad arguments");
+  rng_uniform_keyed<<<grid_for(n, 256, 8), 256, 0, (cudaStream_t)stream>>>(out, n, seed, counter_hi, counter_lo, item);
+  return check_launch("rng_uniform_keyed");
 }
 
 int hmz_debug_philox(const uint32_t* counters_keys, uint32_t* out, int n_blocks, void* stream) {

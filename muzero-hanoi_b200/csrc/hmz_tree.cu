@@ -174,7 +174,8 @@ __global__ void __launch_bounds__(256) search_root_policy(hmz_search_t s, int n_
                                                          int deterministic, const double* __restrict__ uniforms,
                                                          const double* __restrict__ pow_table, int pow_table_len,
                                                          int32_t* __restrict__ visits, double* __restrict__ pi,
-                                                         double* __restrict__ root_q, int32_t* __restrict__ action) {
+                                                         double* __restrict__ root_q, int32_t* __restrict__ action,
+                                                         const uint16_t* __restrict__ budget) {
   for (int64_t b = blockIdx.x * (int64_t)blockDim.x + threadIdx.x; b < s.n_searches;
        b += (int64_t)gridDim.x * blockDim.x) {
     const RootPolicy rp = root_policy_eval(s.nodes + b * s.n_records, temperature, deterministic, deterministic ? 0.0 : uniforms[b],
@@ -187,7 +188,8 @@ __global__ void __launch_bounds__(256) search_root_policy(hmz_search_t s, int n_
 #pragma unroll
       for (int a = 0; a < 6; ++a) pi[b * 6 + a] = rp.prob[a];
     }
-    if (root_q) root_q[b] = n_sims > 0 ? __ddiv_rn(s.root_W[b], (double)n_sims) : 0.0;  // Node.Q (node.py:125-131)
+    const int n = budget != nullptr ? (int)budget[b] : n_sims;  // (per search in a heterogeneous batch)
+    if (root_q) root_q[b] = n > 0 ? __ddiv_rn(s.root_W[b], (double)n) : 0.0;  // Node.Q (node.py:125-131)
     if (action) action[b] = rp.action;
   }
 }
@@ -470,7 +472,24 @@ int hmz_search_root_policy(const hmz_search_t* s, int n_simulations, double temp
   if (s->n_searches == 0) return HMZ_OK;
   if (!deterministic && !uniforms) return fail(HMZ_ERR_INVALID, "hmz_search_root_policy: sampling needs uniforms");
   search_root_policy<<<grid_for(s->n_searches, 256, 4), 256, 0, (cudaStream_t)stream>>>(
-      *s, n_simulations, temperature, deterministic, uniforms, pow_table, n_simulations + 1, visits, pi, root_q, action);
+      *s, n_simulations, temperature, deterministic, uniforms, pow_table, n_simulations + 1, visits, pi, root_q, action, nullptr);
+  return check_launch("search_root_policy");
+}
+
+int hmz_search_root_policy_multi(const hmz_search_t* s, const hmz_multi_t* m, double temperature, int deterministic,
+                                 const double* uniforms, const double* pow_table, int32_t* visits, double* pi, double* root_q,
+                                 int32_t* action, void* stream) {
+  ProfScope prof_scope(HMZ_PROF_ROOT_POLICY, stream);
+  if (!s) return fail(HMZ_ERR_INVALID, "hmz_search_root_policy_multi: null search descriptor");
+  if (int rc = check_multi(m, s->n_searches, -1, s->n_records, true, "hmz_search_root_policy_multi")) return rc;
+  if (!(temperature >= 0.0 && temperature <= 1.0))
+    return fail(HMZ_ERR_INVALID, "Expect `temperature` to be in the range [0.0, 1.0], got %g", temperature);
+  if (s->n_searches == 0) return HMZ_OK;
+  if (!deterministic && !uniforms) return fail(HMZ_ERR_INVALID, "hmz_search_root_policy_multi: sampling needs uniforms");
+  if (int rc = check_search(s, "hmz_search_root_policy_multi")) return rc;
+  const int max_budget = m->host_block_budget[0];
+  search_root_policy<<<grid_for(s->n_searches, 256, 4), 256, 0, (cudaStream_t)stream>>>(
+      *s, max_budget, temperature, deterministic, uniforms, pow_table, max_budget + 1, visits, pi, root_q, action, m->budget);
   return check_launch("search_root_policy");
 }
 
@@ -548,11 +567,18 @@ static int debug_skip() {
   return e ? atoi(e) : 0;
 }
 
+// Weight sets and budgets of one group's searches in a heterogeneous batch (hmz_search_run_multi); all null otherwise.
+struct GroupSets {
+  const uint16_t* block_set;  // of the group's first block
+  int64_t weight_stride;
+  const uint16_t* budget;     // of the group's first search
+};
+
 // One simulation of one group: [select (first simulation only)] -> g+f MLP -> fused backup + next select.
 // capture_stride / capture_lo: searches per capture row (the whole batch) and this group's first search in it.
 static int run_one_sim(const hmz_search_t* s, const SimScratch& sc, const void* weights, int mode, int sim,
                        int n_simulations, const double* ucb_table, double discount, void* stream, int64_t capture_stride,
-                       int64_t capture_lo) {
+                       int64_t capture_lo, const GroupSets& sets = GroupSets{}) {
   const int64_t B = s->n_searches;
   cudaStream_t st = (cudaStream_t)stream;
   if (sim == 0) {
@@ -565,17 +591,19 @@ static int run_one_sim(const hmz_search_t* s, const SimScratch& sc, const void* 
   // tooling (tools/persist_probe.py): HMZ_DEBUG_SKIP=1 leaves out the network launches, =2 the tree launches — timing of
   // one kernel family alone under the group schedule; the search results are meaningless then
   const int skip = debug_skip();
-  if (!(skip & 1))
-    if (int rc = hmz_net_recurrent(weights, mode, s->latents, s->n_records, sc.lp, sc.la, s->latents, s->n_records, sim + 1,
-                                   s->latent_dtype, sc.r, sc.p, sc.v, B, stream))
+  if (!(skip & 1)) {
+    ProfScope prof_scope(HMZ_PROF_NET_RECURRENT, stream);
+    if (int rc = net_recurrent_sets(weights, sets.block_set, sets.weight_stride, mode, s->latents, s->n_records, sc.lp, sc.la,
+                                    s->latents, s->n_records, sim + 1, s->latent_dtype, sc.r, sc.p, sc.v, B, stream))
       return rc;
+  }
   if (skip & 2) return HMZ_OK;
   ProfScope prof_scope(HMZ_PROF_EXPAND_BACKUP, stream);
   const int do_select = (sim + 1 < n_simulations ? 1 : 0) | (pdl_prewait() << 1) | ((pdl_tree_at() & 3) << 2);
   const float *cr = sc.r, *cp = sc.p, *cv = sc.v;
   TreeScratch ts{sc.lp, sc.la, sc.depth, sc.path, sc.wild, cr, cp, cv,
                  s->capture ? s->capture + ((size_t)sim * (size_t)capture_stride + (size_t)capture_lo) * 8 : nullptr,
-                 gantt_next(1, gantt_context_tag())};
+                 gantt_next(1, gantt_context_tag()), sets.budget};
   cudaError_t e = launch_pdl(2, g_tree_tl_search >= 0 ? search_backup_select<true, true> : search_backup_select<false, true>,
                              dim3(search_grid(B)), dim3(kTreeThreads), 0, st, *s, sim, ucb_table, discount, ts, do_select);
   if (e != cudaSuccess) return fail(HMZ_ERR_CUDA, "search_backup_select launch: %s", cudaGetErrorString(e));
@@ -753,6 +781,77 @@ static int search_run_direct(const hmz_search_t* s, const void* weights, int mod
   return rc;
 }
 
+// Heterogeneous batch (hmz_multi_t): the launch-per-simulation schedule of search_run_direct, where simulation `sim` launches
+// over the active prefix only — the blocks whose budget exceeds sim.  Stream groups keep the fixed slices (whole blocks) of the
+// whole batch; a group whose slice has left the prefix issues nothing, so in the late simulations fewer groups overlap.
+static int search_run_multi(const hmz_search_t* s, const hmz_multi_t* m, const void* weights, int mode, const double* ucb_table,
+                            double discount, void* stream) {
+  // argument errors first, before check_search makes its first CUDA call
+  if (!s) return fail(HMZ_ERR_INVALID, "hmz_search_run_multi: null search descriptor");
+  if (int rc = check_multi(m, s->n_searches, mode, s->n_records, true, "hmz_search_run_multi")) return rc;
+  if (s->schedule == HMZ_SCHEDULE_PERSISTENT || s->schedule >= HMZ_SCHEDULE_SERVER)
+    return fail(HMZ_ERR_UNSUPPORTED, "hmz_search_run_multi: only the stream-group schedules (0, 1..16) serve heterogeneous batches");
+  int groups = s->schedule;
+  if (groups < 0 || groups > 16) return fail(HMZ_ERR_INVALID, "hmz_search_run_multi: schedule %d is not a group count in [0, 16]", groups);
+  if (s->n_searches > 0 && (!weights || !ucb_table || !s->workspace || !s->latents))
+    return fail(HMZ_ERR_INVALID, "hmz_search_run_multi: null argument");
+  if (int rc = check_search(s, "hmz_search_run_multi")) return rc;
+  if (s->n_searches == 0) return HMZ_OK;
+  const int64_t B = s->n_searches, n_blocks = B / 256;
+  const int64_t Bp = (B + 63) / 64 * 64;
+  const int max_budget = m->host_block_budget[0];
+  if (groups == 0) groups = B >= 49152 ? 4 : (B >= 12288 ? 2 : 1);  // as hmz_search_run
+  const int64_t per = ((B + groups - 1) / groups + 255) / 256 * 256;  // whole blocks: a block's weight set is per tile pair
+  groups = (int)((B + per - 1) / per);
+  GroupStreams* gs = nullptr;
+  cudaStream_t main_stream = (cudaStream_t)stream;
+  if (groups > 1) {
+    if (int rc = get_group_streams(groups, &gs)) return rc;
+    if (cudaEventRecord(gs->fork, main_stream) != cudaSuccess) return fail(HMZ_ERR_CUDA, "cudaEventRecord(fork) failed");
+  }
+  hmz_search_t sub[16];
+  SimScratch sc[16];
+  GroupSets gsets[16];
+  const size_t lat_elem = s->latent_dtype == HMZ_LATENT_F32 ? 4 : 2;
+  for (int g = 0; g < groups; ++g) {
+    const int64_t lo = g * per, hi = (lo + per < B) ? lo + per : B;
+    sub[g] = *s;
+    sub[g].nodes = s->nodes + lo * s->n_records;
+    sub[g].latents = (char*)s->latents + (size_t)lo * s->n_records * kLatentWidth * lat_elem;
+    sub[g].root_prior = s->root_prior + lo * 6;
+    sub[g].root_W = s->root_W + lo;
+    sub[g].minmax = s->minmax + 2 * lo;
+    sub[g].n_searches = hi - lo;
+    sc[g] = carve_scratch(s->workspace, Bp, lo);
+    gsets[g] = GroupSets{m->block_set + lo / 256, m->weight_stride, m->budget + lo};
+    if (groups > 1 && cudaStreamWaitEvent(gs->stream[g], gs->fork, 0) != cudaSuccess) return fail(HMZ_ERR_CUDA, "cudaStreamWaitEvent failed");
+  }
+  int rc = HMZ_OK;
+  if (groups > 1) tc_allow_head_split(0);
+  int64_t active_blocks = n_blocks;
+  for (int sim = 0; sim < max_budget && rc == HMZ_OK; ++sim) {
+    while (active_blocks > 0 && m->host_block_budget[active_blocks - 1] <= sim) --active_blocks;
+    const int64_t active = active_blocks * 256;
+    for (int g = 0; g < groups && rc == HMZ_OK; ++g) {
+      const int64_t lo = g * per;
+      if (lo >= active) break;  // this and every later slice have left the prefix
+      hmz_search_t part = sub[g];
+      if (part.n_searches > active - lo) part.n_searches = active - lo;
+      gantt_set_context(g, sim);
+      rc = run_one_sim(&part, sc[g], weights, mode, sim, max_budget, ucb_table, discount, groups > 1 ? (void*)gs->stream[g] : stream, B,
+                       lo, gsets[g]);
+    }
+  }
+  if (groups > 1) {
+    tc_allow_head_split(1);
+    for (int g = 0; g < groups; ++g) {  // always join, even after an error, so the caller's stream stays ordered
+      cudaEventRecord(gs->done[g], gs->stream[g]);
+      cudaStreamWaitEvent(main_stream, gs->done[g], 0);
+    }
+  }
+  return rc;
+}
+
 // ---- optional CUDA-graph replay of the whole search (HMZ_GRAPH=1) -------------------------------------------
 // The launch sequence of one hmz_search_run call (groups x simulations x 2 kernels, programmatic edges
 // included) is captured once per distinct argument set on an internal stream and replayed; the caller's stream
@@ -841,6 +940,11 @@ int hmz_search_run(const hmz_search_t* s, const void* weights, int mode, int n_s
   if (graph_mode() && s && s->n_searches > 0 && n_simulations > 0 && g_prof_on.load() == 0 && g_tree_tl_search < 0)
     return search_run_graph(s, weights, mode, n_simulations, ucb_table, discount, stream);
   return search_run_direct(s, weights, mode, n_simulations, ucb_table, discount, stream);
+}
+
+int hmz_search_run_multi(const hmz_search_t* s, const hmz_multi_t* m, const void* weights, int mode, const double* ucb_table,
+                         double discount, void* stream) {
+  return search_run_multi(s, m, weights, mode, ucb_table, discount, stream);
 }
 
 }  // extern "C"

@@ -516,6 +516,8 @@ struct TreeScratch {
   const float* v;
   float* capture;  // nullable: [n_searches][8] row of THIS simulation
   unsigned long long* gantt;  // tooling (hmz_debug_gantt), nullable
+  const uint16_t* budget;     // nullable: simulations of each search (hmz_search_run_multi); the search backs up simulation
+                              // sim only if sim < budget and selects for sim + 1 only if sim + 1 < budget
 };
 
 // Hand-off words of the server schedule (hmz_persist.cu), one 32-byte sector per 256-search tile pair each.
@@ -567,7 +569,8 @@ __device__ __forceinline__ void tree_phase(const hmz_search_t& s, int sim, const
   PathBatch pb;
   pb.slot[0] = make_uint4(0u, 0u, 0u, 0u);
   bool wild = false, was_wild = false;
-  const bool do_backup = !(do_select & 16);  // bit 4: selection only (the first selection of a search: sim = -1)
+  const int budget = (valid && sc.budget != nullptr) ? (int)sc.budget[b] : 0x7FFFFFFF;
+  const bool do_backup = !(do_select & 16) && sim < budget;  // bit 4: selection only (the first selection of a search: sim = -1)
   if (valid) {
     if (kTrusted && half == 0) was_wild = wild = wild_flags[b] != 0;
     mn = s.minmax[2 * b];
@@ -638,9 +641,10 @@ __device__ __forceinline__ void tree_phase(const hmz_search_t& s, int sim, const
   if (kTrusted) wild = __shfl_sync(0xffffffffu, (int)wild, (threadIdx.x & 31) & ~1) != 0;
   tree_mark<kTL>(40, tl, (uint32_t)__double2loint(mn));
   const double* rp = s.root_prior_is_f64 ? s.root_prior + b * 6 : nullptr;
-  const Leaf leaf = select_leaf<kTL, kTrusted, TB>(nodes, rp, mn, mx, sim + 1, ucb_table, discount, half, nullptr, 0, path, tl, valid, wild, tb);
+  const bool sel = valid && sim + 1 < budget;  // (a search past its budget stays in the warp-uniform walk, masked)
+  const Leaf leaf = select_leaf<kTL, kTrusted, TB>(nodes, rp, mn, mx, sim + 1, ucb_table, discount, half, nullptr, 0, path, tl, sel, wild, tb);
   if (kPdl && signal_at == 2) pdl_launch_dependents();
-  if (half == 0 && valid) {
+  if (half == 0 && sel) {
     leaf_parent[b] = (uint16_t)leaf.parent;
     leaf_action[b] = (uint8_t)leaf.action;
     leaf_depth[b] = (uint16_t)leaf.depth;

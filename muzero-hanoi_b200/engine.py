@@ -318,25 +318,7 @@ class PackedWeights:
         self.lib = _lib.load()
         self.n_disks, self.mode = int(n_disks), int(mode)
         self.device = torch.device(device)
-        arrays = []
-        for key in STATE_DICT_ORDER:
-            t = state_dict[key]
-            a = t.detach().cpu().numpy() if torch.is_tensor(t) else np.asarray(t)
-            arrays.append(np.ascontiguousarray(a, dtype=np.float32))
-        expect = {"representation_net.0.weight": (256, 3 * n_disks), "dynamic_net.0.weight": (256, 70),
-                  "rwd_net.2.weight": (33, 256), "policy_net.2.weight": (6, 256), "value_net.2.weight": (33, 256)}
-        for key, shape in expect.items():
-            got = arrays[STATE_DICT_ORDER.index(key)].shape
-            if got != shape:
-                raise ValueError(f"{key}: expected shape {shape}, got {got} (TD_return=True nets with h1_s=256, "
-                                 "reprs_output_size=64 are supported)")
-        nbytes = int(self.lib.hmz_weights_packed_bytes(self.n_disks, self.mode))
-        if nbytes <= 0:
-            raise _lib.HmzError(_lib.ERR_UNSUPPORTED, f"no packed layout for n_disks={n_disks}, mode={mode}")
-        host = np.zeros(nbytes, dtype=np.uint8)
-        table = (C.c_void_p * 20)(*[a.ctypes.data for a in arrays])
-        check(self.lib.hmz_weights_pack(table, self.n_disks, self.mode, host.ctypes.data))
-        self.blob = torch.from_numpy(host).to(self.device)
+        self.blob = torch.from_numpy(pack_host(state_dict, self.n_disks, self.mode)).to(self.device)
         self.ptr = C.c_void_p(self.blob.data_ptr())
 
     def initial(self, n, *, words=None, obs=None, latents_out, out_rows_per_item, latent_dtype, p0, v0):
@@ -348,6 +330,69 @@ class PackedWeights:
         check(self.lib.hmz_net_recurrent(self.ptr, self.mode, ptr(latents_in), in_rows_per_item, ptr(in_row),
                                          ptr(actions), ptr(latents_out), out_rows_per_item, out_row, latent_dtype,
                                          ptr(r), ptr(p), ptr(v), n, current_stream()))
+
+
+def pack_host(state_dict, n_disks, mode):
+    """hmz_weights_pack of a MuZeroNet state_dict (torch tensors or numpy arrays): the packed blob as host uint8."""
+    lib = _lib.load()
+    arrays = []
+    for key in STATE_DICT_ORDER:
+        t = state_dict[key]
+        a = t.detach().cpu().numpy() if torch.is_tensor(t) else np.asarray(t)
+        arrays.append(np.ascontiguousarray(a, dtype=np.float32))
+    expect = {"representation_net.0.weight": (256, 3 * n_disks), "dynamic_net.0.weight": (256, 70),
+              "rwd_net.2.weight": (33, 256), "policy_net.2.weight": (6, 256), "value_net.2.weight": (33, 256)}
+    for key, shape in expect.items():
+        got = arrays[STATE_DICT_ORDER.index(key)].shape
+        if got != shape:
+            raise ValueError(f"{key}: expected shape {shape}, got {got} (TD_return=True nets with h1_s=256, "
+                             "reprs_output_size=64 are supported)")
+    nbytes = int(lib.hmz_weights_packed_bytes(int(n_disks), int(mode)))
+    if nbytes <= 0:
+        raise _lib.HmzError(_lib.ERR_UNSUPPORTED, f"no packed layout for n_disks={n_disks}, mode={mode}")
+    host = np.zeros(nbytes, dtype=np.uint8)
+    table = (C.c_void_p * 20)(*[a.ctypes.data for a in arrays])
+    check(lib.hmz_weights_pack(table, int(n_disks), int(mode), host.ctypes.data))
+    return host
+
+
+class WeightSets:
+    """Several networks in ONE blob, set k at byte k * stride (hmz_multi_t): the weights of a search batch whose 256-search
+    blocks each play with their own network.  ``nets``: state_dicts and / or PackedWeights of the same n_disks and mode.
+    stride = hmz_weights_packed_bytes rounded up to a multiple of 256; the bytes between two sets are zero."""
+
+    def __init__(self, nets, n_disks, mode=_lib.MODE_FP32, device="cuda"):
+        self.lib = _lib.load()
+        self.n_disks, self.mode, self.n_sets = int(n_disks), int(mode), len(nets)
+        if self.n_sets < 1:
+            raise ValueError("WeightSets needs at least one network")
+        self.device = torch.device(device)
+        nbytes = int(self.lib.hmz_weights_packed_bytes(self.n_disks, self.mode))
+        if nbytes <= 0:
+            raise _lib.HmzError(_lib.ERR_UNSUPPORTED, f"no packed layout for n_disks={n_disks}, mode={mode}")
+        self.set_bytes = nbytes
+        self.stride = (nbytes + 255) // 256 * 256
+        self.blob = torch.zeros(self.n_sets * self.stride, dtype=torch.uint8, device=self.device)
+        for k, net in enumerate(nets):
+            if isinstance(net, PackedWeights):
+                if (net.n_disks, net.mode) != (self.n_disks, self.mode):
+                    raise ValueError(f"set {k}: packed for n_disks={net.n_disks}, mode={net.mode}, not {self.n_disks}, {self.mode}")
+                src = net.blob
+            else:
+                src = torch.from_numpy(pack_host(net, self.n_disks, self.mode))
+            self.blob[k * self.stride: k * self.stride + nbytes].copy_(src)
+        self.ptr = C.c_void_p(self.blob.data_ptr())
+
+    def desc(self, block_set, budget=None, host_block_budget=None):
+        """hmz_multi_t over these sets: block_set int16 device [B / 256], budget int16 device [B] (simulations per search),
+        host_block_budget int32 numpy [B / 256] (non-increasing).  The caller keeps the arrays alive."""
+        return _lib.MultiDesc(block_set=block_set.data_ptr(), budget=budget.data_ptr() if budget is not None else None,
+                              host_block_budget=host_block_budget.ctypes.data if host_block_budget is not None else None,
+                              weight_stride=self.stride, n_sets=self.n_sets, n_disks=self.n_disks)
+
+    def initial(self, n, md, *, words, latents_out, out_rows_per_item, latent_dtype, p0, v0):
+        check(self.lib.hmz_net_initial_multi(self.ptr, C.byref(md), self.mode, ptr(words), ptr(latents_out), out_rows_per_item,
+                                             latent_dtype, ptr(p0), ptr(v0), n, current_stream()))
 
 
 def mix_dirichlet(prior_f32: np.ndarray, noise_f64: np.ndarray, eps=0.25) -> np.ndarray:
@@ -385,6 +430,60 @@ def _run_mcts(self, weights: PackedWeights, *, words=None, obs=None, temperature
 
 
 BatchedMCTS.run_mcts = _run_mcts
+
+
+class MultiMCTS:
+    """B searches (a multiple of 256) over several networks and simulation budgets in ONE launch sequence
+    (hmz_search_run_multi): block k of 256 searches plays with weight set block_set[k], search b runs budget[b] simulations.
+    Each search computes exactly what BatchedMCTS.run_mcts with its own network and n_simulations = budget[b] computes.
+    Searches [0, n) of the store take part in a call, so a caller can drop finished blocks by compacting them away."""
+
+    def __init__(self, discount, root_dirichlet_alpha, max_simulations, B, device="cuda", root_exploration_eps=0.25,
+                 latent_dtype=_lib.LATENT_F32):
+        if int(B) % _lib.BLOCK:
+            raise ValueError(f"B={B} is not a multiple of {_lib.BLOCK}")
+        self.discount = float(discount)
+        self.root_dirichlet_alpha = root_dirichlet_alpha
+        self.root_exploration_eps = root_exploration_eps
+        self.max_simulations, self.B = int(max_simulations), int(B)
+        self.store = SearchStore(B, self.max_simulations + 1, device, latent_dtype)
+        self.lib, self.device = self.store.lib, self.store.device
+        self._table = torch.from_numpy(ucb_table(self.max_simulations + 1)).to(self.device)
+        dev = self.device
+        self.p0 = torch.empty(self.B, 6, dtype=torch.float32, device=dev)
+        self.v0 = torch.empty(self.B, dtype=torch.float32, device=dev)
+        self.visits = torch.zeros(self.B, 6, dtype=torch.int32, device=dev)
+        self.pi = torch.zeros(self.B, 6, dtype=torch.float64, device=dev)
+        self.root_q = torch.zeros(self.B, dtype=torch.float64, device=dev)
+        self.action = torch.zeros(self.B, dtype=torch.int32, device=dev)
+
+    def run_mcts(self, sets: WeightSets, md, n, *, words, temperature=1.0, deterministic=False, noise=None, uniforms=None,
+                 pow_table=None):
+        """MCTS.run_mcts for searches [0, n) (n a multiple of 256): root inference with each block's network, optional
+        Dirichlet mix, the fused heterogeneous search, root policy with root_q = root_W / budget.  md: sets.desc(...) of the
+        n searches.  Returns device views [n] of (action, pi, root_q, visits)."""
+        if not 0.0 <= temperature <= 1.0:
+            raise ValueError(f"Expect `temperature` to be in the range [0.0, 1.0], got {temperature}")
+        n = int(n)
+        st = self.store
+        st.desc.n_searches = n
+        try:
+            sets.initial(n, md, words=words, latents_out=st.latents, out_rows_per_item=st.n_records, latent_dtype=st.latent_dtype,
+                         p0=self.p0, v0=self.v0)
+            use_noise = (not deterministic) and self.root_dirichlet_alpha > 0.0 and self.root_exploration_eps > 0.0
+            if use_noise and noise is None:
+                raise ValueError("Dirichlet noise is an input of the batched engine (`noise`, float64 [n,6])")
+            st.desc.root_prior_is_f64 = int(use_noise)
+            check(self.lib.hmz_search_begin_p0(C.byref(st.desc), ptr(self.p0), ptr(noise) if use_noise else None,
+                                               float(self.root_exploration_eps), current_stream()))
+            check(self.lib.hmz_search_run_multi(C.byref(st.desc), C.byref(md), sets.ptr, sets.mode, ptr(self._table), self.discount,
+                                                current_stream()))
+            check(self.lib.hmz_search_root_policy_multi(C.byref(st.desc), C.byref(md), float(temperature), int(bool(deterministic)),
+                                                        ptr(uniforms), ptr(pow_table), ptr(self.visits), ptr(self.pi),
+                                                        ptr(self.root_q), ptr(self.action), current_stream()))
+        finally:
+            st.desc.n_searches = st.B
+        return self.action[:n], self.pi[:n], self.root_q[:n], self.visits[:n]
 
 
 # ---------------------------------------------------------------------------- self-play
