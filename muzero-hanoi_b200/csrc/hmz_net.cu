@@ -392,8 +392,8 @@ int hmz_net_recurrent(const void* weights, int mode, const void* latents_in, int
                       const uint16_t* in_row, const uint8_t* actions, void* latents_out, int64_t out_rows_per_item,
                       int64_t out_row, int latent_dtype, float* r, float* p, float* v, int64_t n, void* stream) {
   ProfScope prof_scope(HMZ_PROF_NET_RECURRENT, stream);
-  return net_recurrent_sets(weights, nullptr, 0, mode, latents_in, in_rows_per_item, in_row, actions, latents_out, out_rows_per_item,
-                            out_row, latent_dtype, r, p, v, n, stream);
+  return net_recurrent_sets(weights, nullptr, 0, true, mode, latents_in, in_rows_per_item, in_row, actions, latents_out,
+                            out_rows_per_item, out_row, latent_dtype, r, p, v, n, stream);
 }
 
 }  // extern "C"
@@ -454,10 +454,10 @@ int net_initial_sets(const void* weights, const uint16_t* block_set, int64_t wei
   return check_launch("net_initial_fp32");
 }
 
-int net_recurrent_sets(const void* weights, const uint16_t* block_set, int64_t weight_stride, int mode, const void* latents_in,
-                       int64_t in_rows_per_item, const uint16_t* in_row, const uint8_t* actions, void* latents_out,
-                       int64_t out_rows_per_item, int64_t out_row, int latent_dtype, float* r, float* p, float* v, int64_t n,
-                       void* stream) {
+int net_recurrent_sets(const void* weights, const uint16_t* block_set, int64_t weight_stride, bool allow_head_split, int mode,
+                       const void* latents_in, int64_t in_rows_per_item, const uint16_t* in_row, const uint8_t* actions,
+                       void* latents_out, int64_t out_rows_per_item, int64_t out_row, int latent_dtype, float* r, float* p, float* v,
+                       int64_t n, void* stream) {
   if (n == 0) return HMZ_OK;
   if (!weights || !latents_in || !actions || !latents_out || !r || !p || !v || n < 0 || in_rows_per_item < 1 ||
       out_rows_per_item < 1 || out_row < 0 || out_row >= out_rows_per_item ||
@@ -465,10 +465,10 @@ int net_recurrent_sets(const void* weights, const uint16_t* block_set, int64_t w
     return fail(HMZ_ERR_INVALID, "hmz_net_recurrent: bad arguments");
   if (mode == HMZ_MODE_BF16)
     return tc_net_recurrent(weights, latents_in, in_rows_per_item, in_row, actions, latents_out, out_rows_per_item,
-                            out_row, latent_dtype, r, p, v, n, (cudaStream_t)stream, block_set, weight_stride);
+                            out_row, latent_dtype, r, p, v, n, (cudaStream_t)stream, block_set, weight_stride, allow_head_split);
   if (mode == HMZ_MODE_FP32X3)
     return x3::net_recurrent(weights, latents_in, in_rows_per_item, in_row, actions, latents_out, out_rows_per_item, out_row,
-                             latent_dtype, r, p, v, n, (cudaStream_t)stream, block_set, weight_stride);
+                             latent_dtype, r, p, v, n, (cudaStream_t)stream, block_set, weight_stride, allow_head_split);
   if (mode != HMZ_MODE_FP32) return fail(HMZ_ERR_INVALID, "hmz_net_recurrent: unknown mode %d", mode);
   if (int rc = ensure_smem_optin()) return rc;
   const unsigned grid = (unsigned)((n + kRows - 1) / kRows);

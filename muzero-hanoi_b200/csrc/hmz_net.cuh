@@ -49,12 +49,10 @@ void tc_pack(const float* const* tensors, int n_disks, void* out);
 int tc_net_initial(const void* weights, int n_disks, const uint32_t* words, void* lat_out, int64_t out_rows_per_item,
                    int latent_dtype, float* p0, float* v0, int64_t n, cudaStream_t stream, const uint16_t* block_set = nullptr,
                    int64_t weight_stride = 0);
-int tc_head_split_allowed();
-void tc_allow_head_split(int allow);  // per host thread; hmz_search_run clears it while several stream groups are in flight
 int tc_net_recurrent(const void* weights, const void* lat_in, int64_t in_rows_per_item, const uint16_t* in_row,
                      const uint8_t* actions, void* lat_out, int64_t out_rows_per_item, int64_t out_row,
                      int latent_dtype, float* r, float* p, float* v, int64_t n, cudaStream_t stream,
-                     const uint16_t* block_set = nullptr, int64_t weight_stride = 0);
+                     const uint16_t* block_set, int64_t weight_stride, bool allow_head_split);
 
 // float32-accurate tensor-core path (hmz_net_x3.cu, HMZ_MODE_FP32X3): split section + the float32 blob behind it
 namespace x3 {
@@ -63,8 +61,8 @@ int64_t fp32_offset_bytes();
 void pack(const float* const* tensors, int n_disks, void* out);
 int net_recurrent(const void* weights, const void* lat_in, int64_t in_rows_per_item, const uint16_t* in_row,
                   const uint8_t* actions, void* lat_out, int64_t out_rows_per_item, int64_t out_row, int latent_dtype,
-                  float* r, float* p, float* v, int64_t n, cudaStream_t stream, const uint16_t* block_set = nullptr,
-                  int64_t weight_stride = 0);
+                  float* r, float* p, float* v, int64_t n, cudaStream_t stream, const uint16_t* block_set,
+                  int64_t weight_stride, bool allow_head_split);
 int net_initial(const void* weights, int n_disks, const uint32_t* words, void* lat_out, int64_t out_rows_per_item,
                 int latent_dtype, float* p0, float* v0, int64_t n, cudaStream_t stream, const uint16_t* block_set = nullptr,
                 int64_t weight_stride = 0);
@@ -72,14 +70,16 @@ int debug_read_timeline(unsigned long long* host_out);
 }  // namespace x3
 
 // Both inferences with an optional weight set per 256-row block (hmz_multi_t): block_set == nullptr is the plain call;
-// otherwise block k of the batch uses weights + block_set[k] * weight_stride (hmz_net.cu).
+// otherwise block k of the batch uses weights + block_set[k] * weight_stride (hmz_net.cu).  allow_head_split: the tensor-core
+// kernels may spread a small batch over three CTAs per tile (one head each); hmz_search_run forbids it while several stream
+// groups share the machine, as the other groups' launches want the idle SMs.
 int net_initial_sets(const void* weights, const uint16_t* block_set, int64_t weight_stride, int mode, int n_disks,
                      const uint32_t* words, const float* obs, void* latents_out, int64_t out_rows_per_item, int latent_dtype,
                      float* p0, float* v0, int64_t n, void* stream);
-int net_recurrent_sets(const void* weights, const uint16_t* block_set, int64_t weight_stride, int mode, const void* latents_in,
-                       int64_t in_rows_per_item, const uint16_t* in_row, const uint8_t* actions, void* latents_out,
-                       int64_t out_rows_per_item, int64_t out_row, int latent_dtype, float* r, float* p, float* v, int64_t n,
-                       void* stream);
+int net_recurrent_sets(const void* weights, const uint16_t* block_set, int64_t weight_stride, bool allow_head_split, int mode,
+                       const void* latents_in, int64_t in_rows_per_item, const uint16_t* in_row, const uint8_t* actions,
+                       void* latents_out, int64_t out_rows_per_item, int64_t out_row, int latent_dtype, float* r, float* p, float* v,
+                       int64_t n, void* stream);
 // Argument checks of the hmz_multi_t entry points (before any CUDA call); need_budget: budget, host_block_budget and
 // their bounds against n_records are checked too.
 int check_multi(const hmz_multi_t* m, int64_t n_searches, int mode, int n_records, bool need_budget, const char* who);

@@ -159,22 +159,17 @@ static unsigned tc_grid(int64_t n, int* n_pairs, int passes = 1) {
   return (unsigned)(want < sms ? want : sms);
 }
 
-// hmz_search_run with several stream groups: the launches of the other groups want the idle SMs — no head split then
-static thread_local int tl_split_allowed = 1;
-void tc_allow_head_split(int allow) { tl_split_allowed = allow; }
-int tc_head_split_allowed() { return tl_split_allowed; }
-
 int tc_net_recurrent(const void* weights, const void* lat_in, int64_t in_rows_per_item, const uint16_t* in_row,
                      const uint8_t* actions, void* lat_out, int64_t out_rows_per_item, int64_t out_row,
                      int latent_dtype, float* r, float* p, float* v, int64_t n, cudaStream_t stream, const uint16_t* block_set,
-                     int64_t weight_stride) {
+                     int64_t weight_stride, bool allow_head_split) {
   int smem = 0, n_pairs = 0;
   if (int rc = tc_prepare(&smem)) return rc;
   unsigned grid = tc_grid(n, &n_pairs, tc_passes());
   tc::v4::TcArgs a{};
   // small batches: three CTAs per tile pair, one head each (TcArgs::head_split); HMZ_TC_SPLIT=0 switches it off
   static const int split_on = getenv("HMZ_TC_SPLIT") ? atoi(getenv("HMZ_TC_SPLIT")) : 1;
-  a.head_split = (split_on && tl_split_allowed && 3 * n_pairs <= sm_count()) ? 3 : 1;
+  a.head_split = (split_on && allow_head_split && 3 * n_pairs <= sm_count()) ? 3 : 1;
   if (a.head_split == 3) grid = 3u * (unsigned)n_pairs;
   a.wsec = (const uint8_t*)weights;
   a.block_set = block_set;

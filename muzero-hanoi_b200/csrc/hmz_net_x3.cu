@@ -733,7 +733,8 @@ static int prepare(int* smem_bytes) {
 
 int net_recurrent(const void* weights, const void* lat_in, int64_t in_rows_per_item, const uint16_t* in_row,
                   const uint8_t* actions, void* lat_out, int64_t out_rows_per_item, int64_t out_row, int latent_dtype,
-                  float* r, float* p, float* v, int64_t n, cudaStream_t stream, const uint16_t* block_set, int64_t weight_stride) {
+                  float* r, float* p, float* v, int64_t n, cudaStream_t stream, const uint16_t* block_set, int64_t weight_stride,
+                  bool allow_head_split) {
   int smem = 0;
   if (int rc = prepare(&smem)) return rc;
   Args a{};
@@ -754,10 +755,9 @@ int net_recurrent(const void* weights, const void* lat_in, int64_t in_rows_per_i
   a.n = n;
   a.n_tiles = (int)((n + kM - 1) / kM);
   const int sms = sm_count();
-  // small batches: three CTAs per tile, one head each (HMZ_TC_SPLIT=0 switches it off; hmz_search_run clears the permission
-  // while several stream groups share the machine)
+  // small batches: three CTAs per tile, one head each (HMZ_TC_SPLIT=0 switches it off)
   static const int split_on = getenv("HMZ_TC_SPLIT") ? atoi(getenv("HMZ_TC_SPLIT")) : 1;
-  a.head_split = (split_on && tc_head_split_allowed() && 3 * a.n_tiles <= sms) ? 3 : 1;
+  a.head_split = (split_on && allow_head_split && 3 * a.n_tiles <= sms) ? 3 : 1;
   static const int tl = getenv("HMZ_X3_TIMELINE") ? atoi(getenv("HMZ_X3_TIMELINE")) : 0;
   a.timeline = tl;
   const unsigned grid = a.head_split == 3 ? 3u * (unsigned)a.n_tiles : (unsigned)(a.n_tiles < sms ? a.n_tiles : sms);

@@ -142,9 +142,8 @@ static int server_mlp_ctas() {
   return v;
 }
 
-// Launches the resident MLP CTAs on `mlp_stream`; the caller then enqueues the tree launches (server_tree_launch).
-int server_mlp_launch(const hmz_search_t* s, const void* weights, int n_simulations, TreeScratch scratch, void* ctl_mem,
-                      int pairs_per_group, cudaStream_t mlp_stream, ServerCtl* out) {
+// Dynamic shared memory of search_persistent, opted in once per host thread and device.
+static int persist_prepare(int* smem_out) {
   static thread_local int attr_dev = -1;
   int dev = 0;
   if (cudaGetDevice(&dev) != cudaSuccess) return fail(HMZ_ERR_CUDA, "cudaGetDevice failed");
@@ -154,44 +153,76 @@ int server_mlp_launch(const hmz_search_t* s, const void* weights, int n_simulati
       return fail(HMZ_ERR_CUDA, "cudaFuncSetAttribute(search_persistent): %s", cudaGetErrorString(cudaGetLastError()));
     attr_dev = dev;
   }
+  *smem_out = smem;
+  return HMZ_OK;
+}
+
+// The control block of both schedules for n_pairs tile pairs: ticket counter [0], queue tail [256], tree_done [1024, 32 B
+// per pair), the item queue (8 B per slot, a power of two >= 2 n_pairs), then the server schedule's mlp_done (32 B per
+// pair) and group_done (32 B per stream group, up to 16).  Returns its size in bytes; with `c`, also points c's hand-off
+// words into `mem` — mlp_done and group_done only for the server schedule (with mlp_done set, the network body pushes no
+// items to the queue).
+static int64_t ctl_layout(int64_t n_pairs, void* mem, bool server, tc::v4::PersistCtl* c) {
+  int64_t cap = 64;
+  while (cap < 2 * n_pairs) cap <<= 1;
+  const int64_t queue = 1024 + n_pairs * 32, mlp_done = queue + cap * 8 + 256, group_done = mlp_done + n_pairs * 32 + 256;
+  if (c) {
+    char* ctl = (char*)mem;
+    c->tree_head = (uint32_t*)ctl;
+    c->q_tail = (uint32_t*)(ctl + 256);
+    c->tree_done = (uint32_t*)(ctl + 1024);
+    c->queue = (unsigned long long*)(ctl + queue);
+    c->q_mask = (uint32_t)(cap - 1);
+    if (server) {
+      c->mlp_done = (uint32_t*)(ctl + mlp_done);
+      c->group_done = (uint32_t*)(ctl + group_done);
+    }
+  }
+  return group_done + 768;
+}
+
+static int64_t tile_pairs(int64_t n_searches) { return (n_searches + 2 * tc::kM - 1) / (2 * tc::kM); }
+
+// The MLP role's arguments: latents gathered from the leaf's parent record, written to record sim + 1 (the body derives
+// the row).
+static tc::v4::TcArgs mlp_args(const hmz_search_t* s, const void* weights, const TreeScratch& scratch, int n_pairs) {
+  tc::v4::TcArgs a{};
+  a.wsec = (const uint8_t*)weights;
+  a.lat_in = s->latents;
+  a.in_rows_per_item = s->n_records;
+  a.in_row = scratch.leaf_parent;
+  a.actions = scratch.leaf_action;
+  a.lat_out = s->latents;
+  a.out_rows_per_item = s->n_records;
+  a.out_row = 0;
+  a.latent_dtype = s->latent_dtype;
+  a.r_out = const_cast<float*>(scratch.r);
+  a.p_out = const_cast<float*>(scratch.p);
+  a.v_out = const_cast<float*>(scratch.v);
+  a.n = s->n_searches;
+  a.n_pairs = n_pairs;
+  return a;
+}
+
+// Launches the resident MLP CTAs on `mlp_stream`; the caller then enqueues the tree launches (server_tree_launch).
+int server_mlp_launch(const hmz_search_t* s, const void* weights, int n_simulations, TreeScratch scratch, void* ctl_mem,
+                      int pairs_per_group, cudaStream_t mlp_stream, ServerCtl* out) {
+  int smem = 0;
+  if (int rc = persist_prepare(&smem)) return rc;
   PersistArgs a{};
-  const int64_t B = s->n_searches;
-  a.n_pairs = (int)((B + 2 * tc::kM - 1) / (2 * tc::kM));
+  a.n_pairs = (int)tile_pairs(s->n_searches);
   a.n_sims = n_simulations;
   int n_mlp = server_mlp_ctas();
   if (n_mlp > sm_count() - 8) n_mlp = sm_count() - 8;
   if (n_mlp > a.n_pairs) n_mlp = a.n_pairs;
   if (n_mlp < 1) return fail(HMZ_ERR_UNSUPPORTED, "server schedule needs at least 9 SMs");
   a.n_mlp = n_mlp;
-  char* ctl = (char*)ctl_mem;
-  int64_t cap = 64;
-  while (cap < 2 * (int64_t)a.n_pairs) cap <<= 1;
   // (the caller has zeroed the control block and ordered every stream behind that)
-  a.ctl.tree_head = (uint32_t*)ctl;
-  a.ctl.q_tail = (uint32_t*)(ctl + 256);
-  a.ctl.tree_done = (uint32_t*)(ctl + 1024);
-  a.ctl.queue = (unsigned long long*)(ctl + 1024 + (size_t)a.n_pairs * 32);
-  a.ctl.q_mask = (uint32_t)(cap - 1);
+  ctl_layout(a.n_pairs, ctl_mem, true, &a.ctl);
   a.ctl.n_sims = n_simulations;
-  a.ctl.stats = nullptr;
-  a.ctl.mlp_done = (uint32_t*)(ctl + 1024 + (size_t)a.n_pairs * 32 + (size_t)cap * 8 + 256);
-  a.ctl.group_done = (uint32_t*)(ctl + 1024 + (size_t)a.n_pairs * 32 + (size_t)cap * 8 + 256 + (size_t)a.n_pairs * 32 + 256);
   a.ctl.pairs_per_group = pairs_per_group;
   a.ctl.rotate = 1;
-  a.net.wsec = (const uint8_t*)weights;
-  a.net.lat_in = s->latents;
-  a.net.in_rows_per_item = s->n_records;
-  a.net.in_row = scratch.leaf_parent;
-  a.net.actions = scratch.leaf_action;
-  a.net.lat_out = s->latents;
-  a.net.out_rows_per_item = s->n_records;
-  a.net.out_row = 0;
-  a.net.latent_dtype = s->latent_dtype;
-  a.net.r_out = const_cast<float*>(scratch.r);
-  a.net.p_out = const_cast<float*>(scratch.p);
-  a.net.v_out = const_cast<float*>(scratch.v);
-  a.net.n = B;
-  a.net.n_pairs = a.n_pairs;
+  a.net = mlp_args(s, weights, scratch, a.n_pairs);
   // tooling: HMZ_TC_TIMELINE=1 HMZ_TC_TIMELINE_PASS=p records the phase marks of CTA 0's pass p (hmz_debug_persist_timeline)
   a.net.timeline = (getenv("HMZ_TC_TIMELINE") && atoi(getenv("HMZ_TC_TIMELINE")))
                        ? (1 | ((getenv("HMZ_TC_TIMELINE_PASS") ? atoi(getenv("HMZ_TC_TIMELINE_PASS")) : 0) << 8))
@@ -245,12 +276,7 @@ static int choose_n_mlp(int n_pairs, int sms) {
   return best;
 }
 
-int64_t persist_ctl_bytes(int64_t n_searches) {
-  const int64_t n_pairs = (n_searches + 2 * tc::kM - 1) / (2 * tc::kM);
-  int64_t cap = 64;
-  while (cap < 2 * n_pairs) cap <<= 1;
-  return 1024 + n_pairs * 32 + cap * 8 + 256 + n_pairs * 32 + 1024;  // ... + the server schedule's per-pair flags and group counters
-}
+int64_t persist_ctl_bytes(int64_t n_searches) { return ctl_layout(tile_pairs(n_searches), nullptr, false, nullptr); }
 
 bool persist_supported(const hmz_search_t* s, int mode, int n_simulations) {
   return mode == HMZ_MODE_BF16 && n_simulations + 2 <= 2048 && s->n_searches > 0 && s->n_searches <= (int64_t)65535 * 256 &&
@@ -261,20 +287,13 @@ bool persist_supported(const hmz_search_t* s, int mode, int n_simulations) {
 // here.  Returns HMZ_OK or an error; the caller has validated the descriptor (check_search) and the tables.
 int persist_launch(const hmz_search_t* s, const void* weights, int n_simulations, const double* ucb_table, double discount,
                    const CountRow* cnt_table, const TreeScratch& scratch, void* ctl_mem, cudaStream_t stream) {
-  static thread_local int attr_dev = -1;
-  int dev = 0;
-  if (cudaGetDevice(&dev) != cudaSuccess) return fail(HMZ_ERR_CUDA, "cudaGetDevice failed");
-  const int smem = (int)sizeof(tc::v4::Smem) + 1024;
-  if (attr_dev != dev) {
-    if (cudaFuncSetAttribute(search_persistent, cudaFuncAttributeMaxDynamicSharedMemorySize, smem) != cudaSuccess)
-      return fail(HMZ_ERR_CUDA, "cudaFuncSetAttribute(search_persistent): %s", cudaGetErrorString(cudaGetLastError()));
-    attr_dev = dev;
-  }
+  int smem = 0;
+  if (int rc = persist_prepare(&smem)) return rc;
   int sms = sm_count();
   if (persist_sm_limit() > 1 && persist_sm_limit() < sms) sms = persist_sm_limit();
   PersistArgs a{};
   const int64_t B = s->n_searches;
-  a.n_pairs = (int)((B + 2 * tc::kM - 1) / (2 * tc::kM));
+  a.n_pairs = (int)tile_pairs(B);
   a.n_sims = n_simulations;
   a.n_mlp = choose_n_mlp(a.n_pairs, sms);
   // every remaining SM plays the tree role, but never more CTAs than there are slices per simulation: with few searches
@@ -295,40 +314,16 @@ int persist_launch(const hmz_search_t* s, const void* weights, int n_simulations
   a.sc = scratch;
   a.sc.capture = s->capture;
   a.capture_stride = s->capture ? B * 8 : 0;
-  // control block
-  char* ctl = (char*)ctl_mem;
-  int64_t cap = 64;
-  while (cap < 2 * (int64_t)a.n_pairs) cap <<= 1;
-  if (cudaMemsetAsync(ctl, 0, (size_t)persist_ctl_bytes(B), stream) != cudaSuccess) return fail(HMZ_ERR_CUDA, "cudaMemsetAsync(control block) failed");
-  a.ctl.tree_head = (uint32_t*)ctl;
-  a.ctl.q_tail = (uint32_t*)(ctl + 256);
-  a.ctl.tree_done = (uint32_t*)(ctl + 1024);
-  a.ctl.queue = (unsigned long long*)(ctl + 1024 + (size_t)a.n_pairs * 32);
-  a.ctl.q_mask = (uint32_t)(cap - 1);
+  const int64_t ctl_bytes = ctl_layout(a.n_pairs, ctl_mem, false, &a.ctl);
+  if (cudaMemsetAsync(ctl_mem, 0, (size_t)ctl_bytes, stream) != cudaSuccess) return fail(HMZ_ERR_CUDA, "cudaMemsetAsync(control block) failed");
   a.ctl.n_sims = n_simulations;
-  a.ctl.stats = nullptr;
   if (tc::v4::kPersistStats && persist_stats_on()) {
     void* sp = nullptr;
     if (cudaGetSymbolAddress(&sp, g_persist_stats) != cudaSuccess || cudaMemsetAsync(sp, 0, sizeof(unsigned long long) * 16, stream) != cudaSuccess)
       return fail(HMZ_ERR_CUDA, "persistent search: statistics buffer unavailable");
     a.ctl.stats = (unsigned long long*)sp;
   }
-  // MLP arguments: latents gathered from the leaf's parent record, written to record sim + 1 (the body derives the row)
-  a.net.wsec = (const uint8_t*)weights;
-  a.net.lat_in = s->latents;
-  a.net.in_rows_per_item = s->n_records;
-  a.net.in_row = scratch.leaf_parent;
-  a.net.actions = scratch.leaf_action;
-  a.net.lat_out = s->latents;
-  a.net.out_rows_per_item = s->n_records;
-  a.net.out_row = 0;
-  a.net.latent_dtype = s->latent_dtype;
-  a.net.r_out = const_cast<float*>(scratch.r);
-  a.net.p_out = const_cast<float*>(scratch.p);
-  a.net.v_out = const_cast<float*>(scratch.v);
-  a.net.n = B;
-  a.net.n_pairs = a.n_pairs;
-  a.net.timeline = 0;
+  a.net = mlp_args(s, weights, scratch, a.n_pairs);
   void* params[] = {&a};
   const cudaError_t e = cudaLaunchCooperativeKernel((const void*)search_persistent, dim3((unsigned)(a.n_mlp + n_tree)), dim3(kPersistThreads),
                                                     params, (size_t)smem, stream);

@@ -311,6 +311,46 @@ static unsigned search_grid(int64_t n_searches) {
   return (unsigned)((n_searches + kSearchesPerBlock - 1) / kSearchesPerBlock);
 }
 
+// hmz_search_run's scratch in the caller's workspace (hmz_search_workspace_bytes), from its first 256-byte boundary: per
+// search of the batch padded to 64 searches, p[6] r v, leaf_parent / action / depth, the sticky "wild" flag and kPathCap
+// path elements of 32 B; then, at the next 256-byte boundary, the hand-off block of the persistent and server schedules
+// (persist_ctl_bytes).
+constexpr int64_t kScratchBytesPerSearch = 40 + 32 * kPathCap;
+static int64_t padded_searches(int64_t n_searches) { return (n_searches + 63) / 64 * 64; }
+
+struct SimScratch {
+  float *p, *r, *v;
+  uint16_t *lp, *depth;
+  uint8_t *la, *wild;
+  uint4* path;
+  void* ctl;  // the hand-off block (whole batch)
+};
+// The scratch of a batch of n_searches, from its search `lo` on.
+static SimScratch carve_scratch(void* workspace, int64_t n_searches, int64_t lo) {
+  const int64_t padded_total = padded_searches(n_searches);
+  char* ws = (char*)(((uintptr_t)workspace + 255) & ~(uintptr_t)255);
+  SimScratch sc;
+  sc.p = (float*)ws + lo * 6;
+  sc.r = (float*)(ws + padded_total * 24) + lo;
+  sc.v = (float*)(ws + padded_total * 28) + lo;
+  sc.lp = (uint16_t*)(ws + padded_total * 32) + lo;
+  sc.la = (uint8_t*)(ws + padded_total * 34) + lo;
+  sc.depth = (uint16_t*)(ws + padded_total * 36) + lo;
+  sc.wild = (uint8_t*)(ws + padded_total * 38) + lo;
+  sc.path = (uint4*)(ws + padded_total * 40) + lo * (2 * kPathCap);
+  sc.ctl = ws + (((size_t)padded_total * kScratchBytesPerSearch + 255) & ~(size_t)255);
+  return sc;
+}
+
+// The root policy of every search of `s` after n_simulations; budget (nullable, hmz_multi_t): each search's own count.
+static int root_policy_launch(const hmz_search_t* s, int n_simulations, const uint16_t* budget, double temperature,
+                              int deterministic, const double* uniforms, const double* pow_table, int32_t* visits, double* pi,
+                              double* root_q, int32_t* action, void* stream) {
+  search_root_policy<<<grid_for(s->n_searches, 256, 4), 256, 0, (cudaStream_t)stream>>>(
+      *s, n_simulations, temperature, deterministic, uniforms, pow_table, n_simulations + 1, visits, pi, root_q, action, budget);
+  return check_launch("search_root_policy");
+}
+
 }  // namespace hmz
 
 using namespace hmz;
@@ -390,9 +430,8 @@ const char* hmz_build_flags(void) {
 
 int64_t hmz_search_workspace_bytes(int64_t n_searches) {
   if (n_searches < 0) return -1;
-  // p[6] r v, leaf_parent/action/depth, the sticky "wild" flag, kPathCap path elements of 32 B per search
-  // ... and the hand-off block of the persistent schedule (ticket counter, per-pair counters, item queue)
-  return ((n_searches + 63) / 64) * 64 * (40 + 32 * kPathCap) + 1024 + persist_ctl_bytes(n_searches);
+  // carve_scratch's layout; 1024 covers the two 256-byte alignments
+  return padded_searches(n_searches) * kScratchBytesPerSearch + 1024 + persist_ctl_bytes(n_searches);
 }
 
 int hmz_search_minmax_reset(double* minmax, int64_t n, void* stream) {
@@ -471,9 +510,8 @@ int hmz_search_root_policy(const hmz_search_t* s, int n_simulations, double temp
     return fail(HMZ_ERR_INVALID, "Expect `temperature` to be in the range [0.0, 1.0], got %g", temperature);
   if (s->n_searches == 0) return HMZ_OK;
   if (!deterministic && !uniforms) return fail(HMZ_ERR_INVALID, "hmz_search_root_policy: sampling needs uniforms");
-  search_root_policy<<<grid_for(s->n_searches, 256, 4), 256, 0, (cudaStream_t)stream>>>(
-      *s, n_simulations, temperature, deterministic, uniforms, pow_table, n_simulations + 1, visits, pi, root_q, action, nullptr);
-  return check_launch("search_root_policy");
+  return root_policy_launch(s, n_simulations, nullptr, temperature, deterministic, uniforms, pow_table, visits, pi, root_q,
+                            action, stream);
 }
 
 int hmz_search_root_policy_multi(const hmz_search_t* s, const hmz_multi_t* m, double temperature, int deterministic,
@@ -487,16 +525,8 @@ int hmz_search_root_policy_multi(const hmz_search_t* s, const hmz_multi_t* m, do
   if (s->n_searches == 0) return HMZ_OK;
   if (!deterministic && !uniforms) return fail(HMZ_ERR_INVALID, "hmz_search_root_policy_multi: sampling needs uniforms");
   if (int rc = check_search(s, "hmz_search_root_policy_multi")) return rc;
-  const int max_budget = m->host_block_budget[0];
-  search_root_policy<<<grid_for(s->n_searches, 256, 4), 256, 0, (cudaStream_t)stream>>>(
-      *s, max_budget, temperature, deterministic, uniforms, pow_table, max_budget + 1, visits, pi, root_q, action, m->budget);
-  return check_launch("search_root_policy");
-}
-
-// Tuning switch: HMZ_PERSIST_AUTO=0 keeps the automatic schedule on the launch-per-simulation path.
-static int persist_auto() {
-  static const int v = getenv("HMZ_PERSIST_AUTO") ? atoi(getenv("HMZ_PERSIST_AUTO")) : 0;
-  return v;
+  return root_policy_launch(s, m->host_block_budget[0], m->budget, temperature, deterministic, uniforms, pow_table, visits, pi,
+                            root_q, action, stream);
 }
 
 namespace {
@@ -528,24 +558,44 @@ int get_group_streams(int want, GroupStreams** out) {
   return HMZ_OK;
 }
 
-struct SimScratch {
-  float *p, *r, *v;
-  uint16_t *lp, *depth;
-  uint8_t *la, *wild;
-  uint4* path;
+// Helper streams forked from the caller's stream: begin(n) orders n of them behind the work enqueued on it so far, and the
+// destructor joins every forked one back into it — on every path, errors included, so that the caller's stream stays
+// ordered behind whatever was enqueued on them.
+class StreamFork {
+ public:
+  explicit StreamFork(cudaStream_t caller) : caller_(caller) {}
+  int begin(int n) {
+    if (int rc = get_group_streams(n, &gs_)) return rc;
+    if (cudaEventRecord(gs_->fork, caller_) != cudaSuccess) return fail(HMZ_ERR_CUDA, "cudaEventRecord(fork) failed");
+    for (; forked_ < n; ++forked_)
+      if (cudaStreamWaitEvent(gs_->stream[forked_], gs_->fork, 0) != cudaSuccess) return fail(HMZ_ERR_CUDA, "cudaStreamWaitEvent failed");
+    return HMZ_OK;
+  }
+  cudaStream_t operator[](int g) const { return gs_->stream[g]; }
+  ~StreamFork() {
+    for (int g = 0; g < forked_; ++g) {
+      cudaEventRecord(gs_->done[g], gs_->stream[g]);
+      cudaStreamWaitEvent(caller_, gs_->done[g], 0);
+    }
+  }
+
+ private:
+  cudaStream_t caller_;
+  GroupStreams* gs_ = nullptr;
+  int forked_ = 0;
 };
-SimScratch carve_scratch(void* workspace, int64_t padded_total, int64_t lo) {
-  char* ws = (char*)(((uintptr_t)workspace + 255) & ~(uintptr_t)255);
-  SimScratch sc;
-  sc.p = (float*)ws + lo * 6;
-  sc.r = (float*)(ws + padded_total * 24) + lo;
-  sc.v = (float*)(ws + padded_total * 28) + lo;
-  sc.lp = (uint16_t*)(ws + padded_total * 32) + lo;
-  sc.la = (uint8_t*)(ws + padded_total * 34) + lo;
-  sc.depth = (uint16_t*)(ws + padded_total * 36) + lo;
-  sc.wild = (uint8_t*)(ws + padded_total * 38) + lo;
-  sc.path = (uint4*)(ws + padded_total * 40) + lo * (2 * kPathCap);
-  return sc;
+
+// Searches [lo, hi) of `s` as a descriptor of their own (their scratch: carve_scratch(s->workspace, s->n_searches, lo)).
+hmz_search_t search_slice(const hmz_search_t* s, int64_t lo, int64_t hi) {
+  const size_t lat_elem = s->latent_dtype == HMZ_LATENT_F32 ? 4 : 2;
+  hmz_search_t sub = *s;
+  sub.nodes = s->nodes + lo * s->n_records;
+  sub.latents = (char*)s->latents + (size_t)lo * s->n_records * kLatentWidth * lat_elem;
+  sub.root_prior = s->root_prior + lo * 6;
+  sub.root_W = s->root_W + lo;
+  sub.minmax = s->minmax + 2 * lo;
+  sub.n_searches = hi - lo;
+  return sub;
 }
 }  // namespace
 
@@ -578,7 +628,7 @@ struct GroupSets {
 // capture_stride / capture_lo: searches per capture row (the whole batch) and this group's first search in it.
 static int run_one_sim(const hmz_search_t* s, const SimScratch& sc, const void* weights, int mode, int sim,
                        int n_simulations, const double* ucb_table, double discount, void* stream, int64_t capture_stride,
-                       int64_t capture_lo, const GroupSets& sets = GroupSets{}) {
+                       int64_t capture_lo, const GroupSets& sets, bool allow_head_split) {
   const int64_t B = s->n_searches;
   cudaStream_t st = (cudaStream_t)stream;
   if (sim == 0) {
@@ -593,8 +643,8 @@ static int run_one_sim(const hmz_search_t* s, const SimScratch& sc, const void* 
   const int skip = debug_skip();
   if (!(skip & 1)) {
     ProfScope prof_scope(HMZ_PROF_NET_RECURRENT, stream);
-    if (int rc = net_recurrent_sets(weights, sets.block_set, sets.weight_stride, mode, s->latents, s->n_records, sc.lp, sc.la,
-                                    s->latents, s->n_records, sim + 1, s->latent_dtype, sc.r, sc.p, sc.v, B, stream))
+    if (int rc = net_recurrent_sets(weights, sets.block_set, sets.weight_stride, allow_head_split, mode, s->latents, s->n_records,
+                                    sc.lp, sc.la, s->latents, s->n_records, sim + 1, s->latent_dtype, sc.r, sc.p, sc.v, B, stream))
       return rc;
   }
   if (skip & 2) return HMZ_OK;
@@ -616,24 +666,18 @@ static int run_one_sim(const hmz_search_t* s, const SimScratch& sc, const void* 
 static int search_run_server(const hmz_search_t* s, const void* weights, int n_simulations, const double* ucb_table,
                              double discount, void* stream) {
   const int64_t B = s->n_searches;
-  const int64_t Bp = (B + 63) / 64 * 64;
   int groups = s->schedule - HMZ_SCHEDULE_SERVER;
   if (groups < 0 || groups > 15) return fail(HMZ_ERR_INVALID, "hmz_search_run: bad server schedule %d", s->schedule);
   if (groups == 0) groups = 4;
   const int64_t per = ((B + groups - 1) / groups + 255) / 256 * 256;  // whole tile pairs: the hand-offs are per pair
   groups = (int)((B + per - 1) / per);
-  GroupStreams* gs = nullptr;
-  if (int rc = get_group_streams(groups + 1, &gs)) return rc;
-  cudaStream_t main_stream = (cudaStream_t)stream, mlp_stream = gs->stream[groups];
-  SimScratch sc0 = carve_scratch(s->workspace, Bp, 0);
-  char* ws = (char*)(((uintptr_t)s->workspace + 255) & ~(uintptr_t)255);
-  void* ctl = ws + (((size_t)Bp * (40 + 32 * kPathCap) + 255) & ~(size_t)255);
+  cudaStream_t main_stream = (cudaStream_t)stream;
+  const SimScratch sc0 = carve_scratch(s->workspace, B, 0);
   if (cudaMemsetAsync(sc0.wild, 0, (size_t)B, main_stream) != cudaSuccess ||
-      cudaMemsetAsync(ctl, 0, (size_t)persist_ctl_bytes(B), main_stream) != cudaSuccess)
+      cudaMemsetAsync(sc0.ctl, 0, (size_t)persist_ctl_bytes(B), main_stream) != cudaSuccess)
     return fail(HMZ_ERR_CUDA, "cudaMemsetAsync(server control block) failed");
-  if (cudaEventRecord(gs->fork, main_stream) != cudaSuccess) return fail(HMZ_ERR_CUDA, "cudaEventRecord(fork) failed");
-  for (int g = 0; g <= groups; ++g)
-    if (cudaStreamWaitEvent(gs->stream[g], gs->fork, 0) != cudaSuccess) return fail(HMZ_ERR_CUDA, "cudaStreamWaitEvent failed");
+  StreamFork fork(main_stream);  // streams [0, groups): tree launches; stream `groups`: the MLP CTAs
+  if (int rc = fork.begin(groups + 1)) return rc;
   {  // CUDA loads kernels lazily, and loading one may wait for the device to go idle — which the resident network CTAs
      // never let it: the tree kernel must be loaded BEFORE they are launched
     static thread_local int loaded_dev = -1;
@@ -645,7 +689,7 @@ static int search_run_server(const hmz_search_t* s, const void* weights, int n_s
   }
   ServerCtl sctl{};
   TreeScratch whole{sc0.lp, sc0.la, sc0.depth, sc0.path, sc0.wild, sc0.r, sc0.p, sc0.v, nullptr, nullptr};
-  int rc = server_mlp_launch(s, weights, n_simulations, whole, ctl, (int)(per / 256), mlp_stream, &sctl);
+  int rc = server_mlp_launch(s, weights, n_simulations, whole, sc0.ctl, (int)(per / 256), fork[groups], &sctl);
   // A tree launch that is resident before its pairs' network outputs exist holds its SM slots spinning: the group's
   // stream waits (cuStreamWaitValue32, resolved through the runtime so that libcuda is not a link dependency) until the
   // network CTAs have finished every pair of the group for the previous simulation.  HMZ_SERVER_GATE=0: spin only.
@@ -664,37 +708,75 @@ static int search_run_server(const hmz_search_t* s, const void* weights, int n_s
   }
   hmz_search_t sub[16];
   SimScratch sc[16];
-  const size_t lat_elem = s->latent_dtype == HMZ_LATENT_F32 ? 4 : 2;
   for (int g = 0; g < groups; ++g) {
-    const int64_t lo = g * per, hi = (lo + per < B) ? lo + per : B;
-    sub[g] = *s;
-    sub[g].nodes = s->nodes + lo * s->n_records;
-    sub[g].latents = (char*)s->latents + (size_t)lo * s->n_records * kLatentWidth * lat_elem;
-    sub[g].root_prior = s->root_prior + lo * 6;
-    sub[g].root_W = s->root_W + lo;
-    sub[g].minmax = s->minmax + 2 * lo;
-    sub[g].n_searches = hi - lo;
-    sc[g] = carve_scratch(s->workspace, Bp, lo);
+    const int64_t lo = g * per;
+    sub[g] = search_slice(s, lo, lo + per < B ? lo + per : B);
+    sc[g] = carve_scratch(s->workspace, B, lo);
   }
   // item k: expansion + backup of simulation k - 1 (none for k = 0) and the selection of simulation k (none for k = S)
   for (int k = 0; k <= n_simulations && rc == HMZ_OK; ++k)
     for (int g = 0; g < groups && rc == HMZ_OK; ++g) {
-      ProfScope prof_scope(HMZ_PROF_EXPAND_BACKUP, (void*)gs->stream[g]);
+      ProfScope prof_scope(HMZ_PROF_EXPAND_BACKUP, (void*)fork[g]);
       gantt_set_context(g, k);
       TreeScratch ts{sc[g].lp, sc[g].la, sc[g].depth, sc[g].path, sc[g].wild, sc[g].r, sc[g].p, sc[g].v,
                      (s->capture && k > 0) ? s->capture + ((size_t)(k - 1) * (size_t)B + (size_t)(g * per)) * 8 : nullptr,
                      gantt_next(1, gantt_context_tag())};
       if (gate && k > 0) {
         const unsigned int pairs_g = (unsigned int)((sub[g].n_searches + 255) / 256);
-        if (wait_value(gs->stream[g], (unsigned long long)(uintptr_t)(sctl.group_done + (size_t)g * 8), pairs_g * (unsigned int)k, 0u /* >= */) != 0)
+        if (wait_value(fork[g], (unsigned long long)(uintptr_t)(sctl.group_done + (size_t)g * 8), pairs_g * (unsigned int)k, 0u /* >= */) != 0)
           rc = fail(HMZ_ERR_CUDA, "cuStreamWaitValue32 failed");
       }
       if (rc == HMZ_OK)
-        rc = server_tree_launch(&sub[g], k, n_simulations, ucb_table, discount, ts, sctl, (int)(g * per / 256), gs->stream[g]);
+        rc = server_tree_launch(&sub[g], k, n_simulations, ucb_table, discount, ts, sctl, (int)(g * per / 256), fork[g]);
     }
-  for (int g = 0; g <= groups; ++g) {  // always join, even after an error, so the caller's stream stays ordered
-    cudaEventRecord(gs->done[g], gs->stream[g]);
-    cudaStreamWaitEvent(main_stream, gs->done[g], 0);
+  return rc;
+}
+
+// The stream-group schedules (0, 1..16) of hmz_search_run and hmz_search_run_multi.  Searches never interact, so the
+// batch is cut into groups whose select -> MLP -> backup chains run on separate streams: the latency-bound tree kernels of
+// one group fill the issue slots the tensor-core kernel of another leaves idle.  One group runs on the caller's stream.
+//   m == nullptr   group boundaries are multiples of 128 searches; every simulation runs over the whole batch.
+//   m (hmz_multi_t) group boundaries are whole 256-search blocks (a block's weight set is per tile pair), each group carries
+//                  its weight sets and budgets, and simulation `sim` launches over the active prefix only — the blocks
+//                  whose budget exceeds sim; a group whose slice has left the prefix issues nothing, so in the late
+//                  simulations fewer groups overlap.
+static int search_run_groups(const hmz_search_t* s, const hmz_multi_t* m, const void* weights, int mode, int n_simulations,
+                             const double* ucb_table, double discount, void* stream) {
+  const int64_t B = s->n_searches;
+  int groups = s->schedule;
+  // measured on the B200 (tools/gpu_round.sh groupsweep, S = 100): 8,192 searches 2.08 / 2.12 / 2.17 ms per move with 1 / 2 / 4
+  // groups, 16,384: 2.26 / 2.25 / 2.29, 32,768: 2.53 / 2.52 / 2.58, 65,536: 4.70 / 4.15 / 4.10 (3 groups 4.07, 6: 4.12, 8: 4.17)
+  if (groups == 0) groups = B >= 49152 ? 4 : (B >= 12288 ? 2 : 1);
+  const int64_t unit = m ? 256 : 128;
+  const int64_t per = ((B + groups - 1) / groups + unit - 1) / unit * unit;
+  groups = (int)((B + per - 1) / per);
+  StreamFork fork((cudaStream_t)stream);
+  if (groups > 1)
+    if (int rc = fork.begin(groups)) return rc;
+  hmz_search_t sub[16];
+  SimScratch sc[16];
+  GroupSets sets[16] = {};
+  for (int g = 0; g < groups; ++g) {
+    const int64_t lo = g * per;
+    sub[g] = search_slice(s, lo, lo + per < B ? lo + per : B);
+    sc[g] = carve_scratch(s->workspace, B, lo);
+    if (m) sets[g] = GroupSets{m->block_set + lo / 256, m->weight_stride, m->budget + lo};
+  }
+  int64_t active = B, active_blocks = B / 256;
+  int rc = HMZ_OK;
+  for (int sim = 0; sim < n_simulations && rc == HMZ_OK; ++sim) {
+    if (m) {
+      while (active_blocks > 0 && m->host_block_budget[active_blocks - 1] <= sim) --active_blocks;
+      active = active_blocks * 256;
+    }
+    for (int g = 0; g < groups && g * per < active && rc == HMZ_OK; ++g) {
+      hmz_search_t part = sub[g];
+      if (part.n_searches > active - g * per) part.n_searches = active - g * per;
+      gantt_set_context(g, sim);
+      // several groups in flight: the other groups' launches want the idle SMs — no head split then
+      rc = run_one_sim(&part, sc[g], weights, mode, sim, n_simulations, ucb_table, discount, groups > 1 ? (void*)fork[g] : stream,
+                       B, g * per, sets[g], groups == 1);
+    }
   }
   return rc;
 }
@@ -707,149 +789,25 @@ static int search_run_direct(const hmz_search_t* s, const void* weights, int mod
       n_simulations + 1 > s->n_records)
     return fail(HMZ_ERR_INVALID, "hmz_search_run: bad arguments (n_simulations=%d, n_records=%d)", n_simulations,
                 s->n_records);
-  const int64_t B = s->n_searches;
-  const int64_t Bp = (B + 63) / 64 * 64;
-  // ONE persistent role-specialised kernel for the whole search (hmz_persist.cu): on request, or as the automatic choice
-  // where it is supported (throughput mode) unless HMZ_PERSIST_AUTO=0
   const bool can_persist = persist_supported(s, mode, n_simulations);
-  if (s->schedule == HMZ_SCHEDULE_PERSISTENT && !can_persist)
-    return fail(HMZ_ERR_UNSUPPORTED, "hmz_search_run: the persistent schedule needs HMZ_MODE_BF16 and n_simulations <= 2046");
-  if (s->schedule == HMZ_SCHEDULE_PERSISTENT || (s->schedule == HMZ_SCHEDULE_AUTO && can_persist && persist_auto() && g_tree_tl_search < 0)) {
+  if (s->schedule == HMZ_SCHEDULE_PERSISTENT) {  // ONE persistent role-specialised kernel for the whole search (hmz_persist.cu)
+    if (!can_persist)
+      return fail(HMZ_ERR_UNSUPPORTED, "hmz_search_run: the persistent schedule needs HMZ_MODE_BF16 and n_simulations <= 2046");
     ProfScope prof_scope(HMZ_PROF_SEARCH_PERSISTENT, stream);
-    SimScratch sc = carve_scratch(s->workspace, Bp, 0);
-    if (cudaMemsetAsync(sc.wild, 0, (size_t)B, (cudaStream_t)stream) != cudaSuccess) return fail(HMZ_ERR_CUDA, "cudaMemsetAsync(wild flags) failed");
+    const SimScratch sc = carve_scratch(s->workspace, s->n_searches, 0);
+    if (cudaMemsetAsync(sc.wild, 0, (size_t)s->n_searches, (cudaStream_t)stream) != cudaSuccess) return fail(HMZ_ERR_CUDA, "cudaMemsetAsync(wild flags) failed");
     const CountRow* cnt = count_table_address();
     if (!cnt) return fail(HMZ_ERR_CUDA, "cudaGetSymbolAddress(count table) failed");
-    char* ws = (char*)(((uintptr_t)s->workspace + 255) & ~(uintptr_t)255);
-    void* ctl = ws + (((size_t)Bp * (40 + 32 * kPathCap) + 255) & ~(size_t)255);
     TreeScratch ts{sc.lp, sc.la, sc.depth, sc.path, sc.wild, sc.r, sc.p, sc.v, nullptr, nullptr};
-    return persist_launch(s, weights, n_simulations, ucb_table, discount, cnt, ts, ctl, (cudaStream_t)stream);
+    return persist_launch(s, weights, n_simulations, ucb_table, discount, cnt, ts, sc.ctl, (cudaStream_t)stream);
   }
   if (s->schedule >= HMZ_SCHEDULE_SERVER) {
     if (!can_persist) return fail(HMZ_ERR_UNSUPPORTED, "hmz_search_run: the server schedule needs HMZ_MODE_BF16 and n_simulations <= 2046");
     return search_run_server(s, weights, n_simulations, ucb_table, discount, stream);
   }
-  // Searches never interact, so the batch is cut into groups whose select -> MLP -> backup chains
-  // run on separate streams: the latency-bound tree kernels of one group fill the issue slots the
-  // tensor-core kernel of another leaves idle.  Group boundaries are multiples of 128 searches.
-  int groups = s->schedule;
-  if (groups < 0 || groups > 16) return fail(HMZ_ERR_INVALID, "hmz_search_run: schedule %d is neither a group count in [0, 16] nor HMZ_SCHEDULE_PERSISTENT", groups);
-  // measured on the B200 (tools/gpu_round.sh groupsweep, S = 100): 8,192 searches 2.08 / 2.12 / 2.17 ms per move with 1 / 2 / 4
-  // groups, 16,384: 2.26 / 2.25 / 2.29, 32,768: 2.53 / 2.52 / 2.58, 65,536: 4.70 / 4.15 / 4.10 (3 groups 4.07, 6: 4.12, 8: 4.17)
-  if (groups == 0) groups = B >= 49152 ? 4 : (B >= 12288 ? 2 : 1);
-  const int64_t per = ((B + groups - 1) / groups + 127) / 128 * 128;
-  groups = (int)((B + per - 1) / per);
-  if (groups <= 1) {
-    SimScratch sc = carve_scratch(s->workspace, Bp, 0);
-    for (int sim = 0; sim < n_simulations; ++sim) {
-      gantt_set_context(0, sim);
-      if (int rc = run_one_sim(s, sc, weights, mode, sim, n_simulations, ucb_table, discount, stream, B, 0)) return rc;
-    }
-    return HMZ_OK;
-  }
-  GroupStreams* gs = nullptr;
-  if (int rc = get_group_streams(groups, &gs)) return rc;
-  cudaStream_t main_stream = (cudaStream_t)stream;
-  if (cudaEventRecord(gs->fork, main_stream) != cudaSuccess) return fail(HMZ_ERR_CUDA, "cudaEventRecord(fork) failed");
-  hmz_search_t sub[16];
-  SimScratch sc[16];
-  const size_t lat_elem = s->latent_dtype == HMZ_LATENT_F32 ? 4 : 2;
-  for (int g = 0; g < groups; ++g) {
-    const int64_t lo = g * per, hi = (lo + per < B) ? lo + per : B;
-    sub[g] = *s;
-    sub[g].nodes = s->nodes + lo * s->n_records;
-    sub[g].latents = (char*)s->latents + (size_t)lo * s->n_records * kLatentWidth * lat_elem;
-    sub[g].root_prior = s->root_prior + lo * 6;
-    sub[g].root_W = s->root_W + lo;
-    sub[g].minmax = s->minmax + 2 * lo;
-    sub[g].n_searches = hi - lo;
-    sc[g] = carve_scratch(s->workspace, Bp, lo);
-    if (cudaStreamWaitEvent(gs->stream[g], gs->fork, 0) != cudaSuccess) return fail(HMZ_ERR_CUDA, "cudaStreamWaitEvent failed");
-  }
-  int rc = HMZ_OK;
-  tc_allow_head_split(0);  // the groups' launches share the machine
-  for (int sim = 0; sim < n_simulations && rc == HMZ_OK; ++sim)
-    for (int g = 0; g < groups && rc == HMZ_OK; ++g) {
-      gantt_set_context(g, sim);
-      rc = run_one_sim(&sub[g], sc[g], weights, mode, sim, n_simulations, ucb_table, discount, (void*)gs->stream[g], B, g * per);
-    }
-  tc_allow_head_split(1);
-  for (int g = 0; g < groups; ++g) {  // always join, even after an error, so the caller's stream stays ordered
-    cudaEventRecord(gs->done[g], gs->stream[g]);
-    cudaStreamWaitEvent(main_stream, gs->done[g], 0);
-  }
-  return rc;
-}
-
-// Heterogeneous batch (hmz_multi_t): the launch-per-simulation schedule of search_run_direct, where simulation `sim` launches
-// over the active prefix only — the blocks whose budget exceeds sim.  Stream groups keep the fixed slices (whole blocks) of the
-// whole batch; a group whose slice has left the prefix issues nothing, so in the late simulations fewer groups overlap.
-static int search_run_multi(const hmz_search_t* s, const hmz_multi_t* m, const void* weights, int mode, const double* ucb_table,
-                            double discount, void* stream) {
-  // argument errors first, before check_search makes its first CUDA call
-  if (!s) return fail(HMZ_ERR_INVALID, "hmz_search_run_multi: null search descriptor");
-  if (int rc = check_multi(m, s->n_searches, mode, s->n_records, true, "hmz_search_run_multi")) return rc;
-  if (s->schedule == HMZ_SCHEDULE_PERSISTENT || s->schedule >= HMZ_SCHEDULE_SERVER)
-    return fail(HMZ_ERR_UNSUPPORTED, "hmz_search_run_multi: only the stream-group schedules (0, 1..16) serve heterogeneous batches");
-  int groups = s->schedule;
-  if (groups < 0 || groups > 16) return fail(HMZ_ERR_INVALID, "hmz_search_run_multi: schedule %d is not a group count in [0, 16]", groups);
-  if (s->n_searches > 0 && (!weights || !ucb_table || !s->workspace || !s->latents))
-    return fail(HMZ_ERR_INVALID, "hmz_search_run_multi: null argument");
-  if (int rc = check_search(s, "hmz_search_run_multi")) return rc;
-  if (s->n_searches == 0) return HMZ_OK;
-  const int64_t B = s->n_searches, n_blocks = B / 256;
-  const int64_t Bp = (B + 63) / 64 * 64;
-  const int max_budget = m->host_block_budget[0];
-  if (groups == 0) groups = B >= 49152 ? 4 : (B >= 12288 ? 2 : 1);  // as hmz_search_run
-  const int64_t per = ((B + groups - 1) / groups + 255) / 256 * 256;  // whole blocks: a block's weight set is per tile pair
-  groups = (int)((B + per - 1) / per);
-  GroupStreams* gs = nullptr;
-  cudaStream_t main_stream = (cudaStream_t)stream;
-  if (groups > 1) {
-    if (int rc = get_group_streams(groups, &gs)) return rc;
-    if (cudaEventRecord(gs->fork, main_stream) != cudaSuccess) return fail(HMZ_ERR_CUDA, "cudaEventRecord(fork) failed");
-  }
-  hmz_search_t sub[16];
-  SimScratch sc[16];
-  GroupSets gsets[16];
-  const size_t lat_elem = s->latent_dtype == HMZ_LATENT_F32 ? 4 : 2;
-  for (int g = 0; g < groups; ++g) {
-    const int64_t lo = g * per, hi = (lo + per < B) ? lo + per : B;
-    sub[g] = *s;
-    sub[g].nodes = s->nodes + lo * s->n_records;
-    sub[g].latents = (char*)s->latents + (size_t)lo * s->n_records * kLatentWidth * lat_elem;
-    sub[g].root_prior = s->root_prior + lo * 6;
-    sub[g].root_W = s->root_W + lo;
-    sub[g].minmax = s->minmax + 2 * lo;
-    sub[g].n_searches = hi - lo;
-    sc[g] = carve_scratch(s->workspace, Bp, lo);
-    gsets[g] = GroupSets{m->block_set + lo / 256, m->weight_stride, m->budget + lo};
-    if (groups > 1 && cudaStreamWaitEvent(gs->stream[g], gs->fork, 0) != cudaSuccess) return fail(HMZ_ERR_CUDA, "cudaStreamWaitEvent failed");
-  }
-  int rc = HMZ_OK;
-  if (groups > 1) tc_allow_head_split(0);
-  int64_t active_blocks = n_blocks;
-  for (int sim = 0; sim < max_budget && rc == HMZ_OK; ++sim) {
-    while (active_blocks > 0 && m->host_block_budget[active_blocks - 1] <= sim) --active_blocks;
-    const int64_t active = active_blocks * 256;
-    for (int g = 0; g < groups && rc == HMZ_OK; ++g) {
-      const int64_t lo = g * per;
-      if (lo >= active) break;  // this and every later slice have left the prefix
-      hmz_search_t part = sub[g];
-      if (part.n_searches > active - lo) part.n_searches = active - lo;
-      gantt_set_context(g, sim);
-      rc = run_one_sim(&part, sc[g], weights, mode, sim, max_budget, ucb_table, discount, groups > 1 ? (void*)gs->stream[g] : stream, B,
-                       lo, gsets[g]);
-    }
-  }
-  if (groups > 1) {
-    tc_allow_head_split(1);
-    for (int g = 0; g < groups; ++g) {  // always join, even after an error, so the caller's stream stays ordered
-      cudaEventRecord(gs->done[g], gs->stream[g]);
-      cudaStreamWaitEvent(main_stream, gs->done[g], 0);
-    }
-  }
-  return rc;
+  if (s->schedule < 0 || s->schedule > 16)
+    return fail(HMZ_ERR_INVALID, "hmz_search_run: schedule %d is neither a group count in [0, 16] nor HMZ_SCHEDULE_PERSISTENT", s->schedule);
+  return search_run_groups(s, nullptr, weights, mode, n_simulations, ucb_table, discount, stream);
 }
 
 // ---- optional CUDA-graph replay of the whole search (HMZ_GRAPH=1) -------------------------------------------
@@ -944,7 +902,18 @@ int hmz_search_run(const hmz_search_t* s, const void* weights, int mode, int n_s
 
 int hmz_search_run_multi(const hmz_search_t* s, const hmz_multi_t* m, const void* weights, int mode, const double* ucb_table,
                          double discount, void* stream) {
-  return search_run_multi(s, m, weights, mode, ucb_table, discount, stream);
+  // argument errors first, before check_search makes its first CUDA call
+  if (!s) return fail(HMZ_ERR_INVALID, "hmz_search_run_multi: null search descriptor");
+  if (int rc = check_multi(m, s->n_searches, mode, s->n_records, true, "hmz_search_run_multi")) return rc;
+  if (s->schedule == HMZ_SCHEDULE_PERSISTENT || s->schedule >= HMZ_SCHEDULE_SERVER)
+    return fail(HMZ_ERR_UNSUPPORTED, "hmz_search_run_multi: only the stream-group schedules (0, 1..16) serve heterogeneous batches");
+  if (s->schedule < 0 || s->schedule > 16)
+    return fail(HMZ_ERR_INVALID, "hmz_search_run_multi: schedule %d is not a group count in [0, 16]", s->schedule);
+  if (s->n_searches > 0 && (!weights || !ucb_table || !s->workspace || !s->latents))
+    return fail(HMZ_ERR_INVALID, "hmz_search_run_multi: null argument");
+  if (int rc = check_search(s, "hmz_search_run_multi")) return rc;
+  if (s->n_searches == 0) return HMZ_OK;
+  return search_run_groups(s, m, weights, mode, m->host_block_budget[0], ucb_table, discount, stream);
 }
 
 }  // extern "C"
