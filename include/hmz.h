@@ -501,6 +501,34 @@ int hmz_learner_step(float* params, float* grads, float* adam_m, float* adam_v, 
                      const float* priority_w, double lr, double beta1, double beta2, double eps, int64_t step_index,
                      float* new_priorities, float* losses_out, int apply_update, void* stream);
 
+/* ------------------------------------------------------------------ replay sampling ---------
+ * ReplayRing.priority_sample (buffer.py:96) with priority exponent 1, bit-exact with NumPy given the same uniforms:
+ *   s = np.sum(q) (float32, NumPy's pairwise tree); x = q / s (float32); np.random.choice(num, batch, p=x), i.e. NumPy's
+ *   checks on p = float64(x), cdf = cumsum(p) (float64, left to right, evaluated exactly in parallel), cdf /= cdf[-1],
+ *   indices = searchsorted(cdf, uniforms, side="right"); weights = (float32(1 / size) / x[indices]) ** importance_exponent,
+ *   weights /= max(weights).
+ *   priorities f32 [num] (the filled rows of the ring), uniforms f64 [batch] (np.random.random_sample(batch), the only
+ *   draw choice makes), workspace of hmz_replay_sample_workspace_bytes(num) bytes, indices i64 [batch], weights f32 [batch].
+ *   *status (device int32) ORs in one HMZ_REPLAY_* bit per error NumPy would raise and is never cleared here, so one
+ *   read covers many calls.  The sum check compares the cumulative sum's last value instead of Kahan's sum with the
+ *   threshold (they differ by at most num * 2^-53).  importance_exponent 0, 0.5, 1, 2 and -1 are exact (NumPy's fast
+ *   paths); others use CUDA's powf.  priority_exponent != 1: HMZ_ERR_UNSUPPORTED; num < 1, size < num, batch < 1:
+ *   HMZ_ERR_INVALID; num > 2^27: HMZ_ERR_UNSUPPORTED.
+ * hmz_replay_set_priorities: update_priorities (buffer.py:130): if every new priority is finite and one is > 0,
+ *   priorities[indices[j]] = new_priorities[j] with the last occurrence of a repeated index winning (NumPy's fancy
+ *   assignment); otherwise nothing is written and *status ORs in HMZ_REPLAY_PRIORITY.  Indices outside [0, size) are
+ *   skipped. */
+#define HMZ_REPLAY_NAN 1u      /* ValueError("probabilities contain NaN")           */
+#define HMZ_REPLAY_NEGATIVE 2u /* ValueError("probabilities are not non-negative")  */
+#define HMZ_REPLAY_SUM 4u      /* ValueError("probabilities do not sum to 1")       */
+#define HMZ_REPLAY_PRIORITY 8u /* AssertionError("Priorities must be finite and positive.") */
+int64_t hmz_replay_sample_workspace_bytes(int64_t num);
+int hmz_replay_sample(const float* priorities, int64_t num, int64_t size, double priority_exponent, const double* uniforms,
+                      int64_t batch, double importance_exponent, void* workspace, int64_t* indices, float* weights, int32_t* status,
+                      void* stream);
+int hmz_replay_set_priorities(float* priorities, int64_t size, const int64_t* indices, const float* new_priorities, int64_t batch,
+                              int32_t* status, void* stream);
+
 #ifdef __cplusplus
 }
 #endif

@@ -16,6 +16,7 @@ N_ACTIONS, LATENT, HIDDEN, SUPPORT, MAX_DISKS, NO_CHILD = 6, 64, 256, 33, 12, 0x
 LATENT_F32, LATENT_BF16 = 0, 1
 SCHEDULE_AUTO, SCHEDULE_PERSISTENT, SCHEDULE_SERVER = 0, 64, 128
 MODE_FP32, MODE_BF16, MODE_FP32X3 = 0, 1, 2
+REPLAY_NAN, REPLAY_NEGATIVE, REPLAY_SUM, REPLAY_PRIORITY = 1, 2, 4, 8  # status bits of hmz_replay_sample / _set_priorities
 
 
 class HmzError(RuntimeError):
@@ -153,6 +154,9 @@ SIGNATURES = {
     "hmz_episode_mc_returns": (_I, [_P, _P, _P, _L, _I, _P, _P, _P, _P]),
     "hmz_episode_rows": (_I, [_P, _P, _L, _L, _I, _P, _P, _P]),
     "hmz_episode_unroll": (_I, [_P, _P, _P, _P, _P, _P, _P, _P, _P, _P, _L, _I, _I, _I, _D, _L, _L, _P, _P, _P, _P, _P, _P, _P]),
+    "hmz_replay_sample_workspace_bytes": (_L, [_L]),
+    "hmz_replay_sample": (_I, [_P, _L, _L, _D, _P, _L, _D, _P, _P, _P, _P, _P]),
+    "hmz_replay_set_priorities": (_I, [_P, _L, _P, _P, _L, _P, _P]),
 }
 
 _lock = threading.Lock()

@@ -118,7 +118,7 @@ int hmz_debug_gantt(int enable, unsigned long long* host_out, int max_records, i
 
 const char* hmz_last_error(void) { return hmz::error_buffer(); }
 
-int hmz_version(void) { return 203; }
+int hmz_version(void) { return 204; }
 
 int64_t hmz_launch_count(void) { return (int64_t)hmz::g_launches.load(); }
 

@@ -3,7 +3,7 @@ reference (Muzero.py:209-274, networks.py:118-122) as one libhmz call per batch.
 
 ``Learner`` owns the flat float32 parameter / gradient / Adam-moment buffers (the 20 state_dict tensors in
 state_dict order, torch ``[out][in]`` layout); ``update`` has the reference's ``_update`` signature and return
-values; ``state_dict`` / ``load_state_dict`` move weights to and from a ``MuZeroNet`` (or a PackedWeights for the
+values, ``step`` is the same update left on the device (no read-back); ``state_dict`` / ``load_state_dict`` move weights to and from a ``MuZeroNet`` (or a PackedWeights for the
 acting kernels).  torch is used for memory only.
 """
 from __future__ import annotations
@@ -63,8 +63,10 @@ class Learner:
         return self._split(self.grads)
 
     # -- Muzero._update ------------------------------------------------------------------------------
-    def update(self, states, rwds, actions, pi_probs, returns, priority_w=None, apply_update=True):
-        """-> (new_priorities np.float32[B] or None, value_loss, rwd_loss, policy_loss) like Muzero._update."""
+    def step(self, states, rwds, actions, pi_probs, returns, priority_w=None, apply_update=True):
+        """Enqueues one hmz_learner_step on the current stream and returns device tensors (new_priorities f32[B] or None,
+        losses f32[3] = value, reward, policy loss) without synchronising.  ``losses`` is this Learner's buffer: the next
+        step overwrites it."""
         dev = self.device
         states = torch.as_tensor(states, dtype=torch.float32, device=dev).contiguous()
         B = states.shape[0]
@@ -85,5 +87,11 @@ class Learner:
                                         self.n_disks, B, self.unroll, ptr(states), ptr(rwds), ptr(actions), ptr(pi_probs), ptr(returns),
                                         ptr(w), self.lr, self.betas[0], self.betas[1], self.eps, max(1, self.step_index), ptr(new_p),
                                         ptr(self.losses), int(bool(apply_update)), current_stream()))
-        v_loss, r_loss, p_loss = self.losses.cpu().tolist()
+        return new_p, self.losses
+
+    def update(self, states, rwds, actions, pi_probs, returns, priority_w=None, apply_update=True):
+        """-> (new_priorities np.float32[B] or None, value_loss, rwd_loss, policy_loss) like Muzero._update: step() and
+        the read-back."""
+        new_p, losses = self.step(states, rwds, actions, pi_probs, returns, priority_w, apply_update)
+        v_loss, r_loss, p_loss = losses.cpu().tolist()
         return (None if new_p is None else new_p.cpu().numpy()), v_loss, r_loss, p_loss

@@ -6,6 +6,18 @@ returns (utils.py:28-72), priorities (Muzero.py:197-200) and ``organise_transiti
 (Muzero.py:276-323).  ``ReplayRing`` is ``buffer.Buffer`` (buffer.py) with its arrays resident in HBM:
 same constructor, attributes and methods; ``add_episodes`` is the device-side ``add``.
 torch is used for memory and index gathers only; every computation is a libhmz kernel.
+
+``priority_sample_device`` / ``uniform_sample_device`` / ``update_priorities_device`` draw a training batch and write the
+new priorities back without a host round trip, bit-identical to ``priority_sample`` / ``uniform_sample`` /
+``update_priorities`` given the same NumPy global RandomState.  The host draws only the random numbers: the uniforms
+of ``np.random.choice``, or ``randint``'s indices.  ``hmz_replay_sample`` runs the rest on the device.  It runs NumPy's
+pairwise float32 sum, the division and ``choice``'s checks.  It runs the float64 cumulative sum exactly in parallel:
+inside one binade of the running sum every addition is an integer step on the grid ulp(c), decided by the addend
+alone except at an exact half-ulp tie, so the rows compose as maps of the parity bit and a block scan gives NumPy's
+left-to-right sums (DESIGN §3).  It also runs the search and the importance weights.  Errors NumPy would raise set
+bits of ``status`` (a device int32 that only accumulates); ``check_status`` or ``raise_for_status`` raise them with
+the reference's exception types and messages.  Priority exponents other than 1 are served by ``priority_sample``
+only.
 """
 from __future__ import annotations
 
@@ -117,6 +129,9 @@ class ReplayRing:
         self.priorities = torch.zeros(size, dtype=torch.float32, device=dev)
         self.ptr = 0
         self.is_full = False
+        # device sampling: HMZ_REPLAY_* bits of every error NumPy would have raised since the ring was made (never cleared)
+        self.status = torch.zeros(1, dtype=torch.int32, device=dev)
+        self._ws = None
 
     def __len__(self):
         return self.size if self.is_full else self.ptr
@@ -172,7 +187,7 @@ class ReplayRing:
             self._add(buf, x)
         self._advance(n)
 
-    # -- sampling (buffer.py:85-128): the index draw stays NumPy's, the rows never leave the device -----
+    # -- sampling (buffer.py:85-128) on the host: the index draw is NumPy's, the rows never leave the device -----
     def _sample(self, indx):
         i = torch.as_tensor(indx, dtype=torch.int64, device=self.dev)
         return self.states[i], self.rwds[i], self.actions[i], self.pi_probs[i], self.mc_returns[i]
@@ -199,3 +214,68 @@ class ReplayRing:
             assert np.isfinite(new_priorities).all() and (new_priorities > 0.0).any(), "Priorities must be finite and positive."
             self.priorities[torch.as_tensor(indx, dtype=torch.int64, device=self.dev)] = torch.as_tensor(
                 new_priorities, dtype=torch.float32, device=self.dev)
+
+    # -- sampling without a host round trip ------------------------------------------------------------
+    # The same draws as uniform_sample / priority_sample / update_priorities, enqueued on the current stream with no
+    # synchronisation: the host draws only the random numbers (from NumPy's global RandomState, in the same order) and
+    # copies them from pinned memory; hmz_replay_sample runs priority_sample's sum, division, NumPy's checks, the
+    # cumulative sum, the search and the weights on the device, bit-exact.  Errors NumPy would raise set bits of
+    # self.status instead; check_status() (or raise_for_status on a value read back with other results) raises them.
+    def _to_device(self, a):
+        return torch.from_numpy(np.ascontiguousarray(a)).pin_memory().to(self.dev, non_blocking=True)
+
+    def uniform_sample_device(self, batch_s):
+        """uniform_sample with the indices copied to the device without a synchronise (np.random.choice(arange(num),
+        batch, replace=True) is np.random.randint(0, num, batch): same indices, same draws)."""
+        indx = self._to_device(np.random.randint(0, len(self), int(batch_s)).astype(np.int64))
+        return self._sample(indx)
+
+    def priority_sample_device(self, batch_s, uniforms=None):
+        """priority_sample with indx and the weights as device tensors.  uniforms: float64 [batch_s], the draw of
+        np.random.choice; np.random.random_sample(batch_s) when omitted."""
+        num, batch_s = len(self), int(batch_s)
+        if uniforms is None:
+            uniforms = np.random.random_sample(batch_s)
+        u = uniforms if torch.is_tensor(uniforms) else self._to_device(np.asarray(uniforms, dtype=np.float64))
+        if u.dtype != torch.float64 or u.numel() != batch_s or not u.is_cuda:
+            raise ValueError(f"uniforms must be {batch_s} float64 values")
+        u = u.contiguous()
+        need = int(self.lib.hmz_replay_sample_workspace_bytes(max(num, 1)))
+        if self._ws is None or self._ws.numel() < need:
+            self._ws = torch.empty(need, dtype=torch.uint8, device=self.dev)
+        indx = torch.empty(batch_s, dtype=torch.int64, device=self.dev)
+        weights = torch.empty(batch_s, dtype=torch.float32, device=self.dev)
+        check(self.lib.hmz_replay_sample(ptr(self.priorities), num, self.size, float(self._priority_exponent), ptr(u), batch_s,
+                                         float(self._importance_sampling_exponent), ptr(self._ws), ptr(indx), ptr(weights),
+                                         ptr(self.status), current_stream()))
+        states, rwds, actions, pi_probs, mc_returns = self._sample(indx)
+        return states, rwds, actions, pi_probs, mc_returns, indx, weights
+
+    def update_priorities_device(self, indx, new_priorities):
+        """update_priorities from device tensors: duplicates in indx keep their last value; a batch that fails the
+        reference's assertion writes nothing and sets REPLAY_PRIORITY in self.status."""
+        if indx is None:
+            return
+        i = torch.as_tensor(indx, dtype=torch.int64, device=self.dev).contiguous()
+        p = torch.as_tensor(new_priorities, dtype=torch.float32, device=self.dev).contiguous()
+        if i.numel() != p.numel():
+            raise ValueError(f"{i.numel()} indices but {p.numel()} priorities")
+        check(self.lib.hmz_replay_set_priorities(ptr(self.priorities), self.size, ptr(i), ptr(p), i.numel(), ptr(self.status),
+                                                 current_stream()))
+
+    @staticmethod
+    def raise_for_status(status: int):
+        """The exception the reference would have raised first, for status bits read back from ReplayRing.status."""
+        status = int(status)
+        if status & _lib.REPLAY_NAN:
+            raise ValueError("probabilities contain NaN")
+        if status & _lib.REPLAY_NEGATIVE:
+            raise ValueError("probabilities are not non-negative")
+        if status & _lib.REPLAY_SUM:
+            raise ValueError("probabilities do not sum to 1")
+        if status & _lib.REPLAY_PRIORITY:
+            raise AssertionError("Priorities must be finite and positive.")
+
+    def check_status(self):
+        """Reads the status word (one synchronise) and raises what the reference would have raised."""
+        self.raise_for_status(int(self.status.item()))

@@ -6,7 +6,10 @@ Differences from the sequential reference, all forced by playing B games at once
   * one "loop" plays ``moves_per_loop`` moves of all B games instead of ``n_ep_x_loop`` whole episodes; the episodes
     that finish during a loop are post-processed and (if solved, Muzero.py:98) stored;
   * the temperature schedule (utils.adjust_temperature) is driven by the number of finished episodes per game slot;
-  * acting uses the weights of the last completed update (repacked for the acting kernels once per loop).
+  * acting uses the weights of the last completed update (repacked for the acting kernels once per loop);
+  * the updates of a loop are enqueued without a host round trip (``step``: the replay draw, the learner step and the
+    priority write-back on the device, bit-identical to the reference's NumPy draws); the last update's losses and the
+    replay ring's status are read back once at the end of the loop, so a ring the reference would reject raises there.
 Same hyper-parameters and defaults as training_main.TrainingConfig (training_main.py:17-36).
 
 With ``torch.distributed`` initialised over G > 1 processes (one per GPU, e.g. torchrun) the loop takes the Ape-X /
@@ -52,6 +55,7 @@ class BatchedMuzero:
         self._gather = None      # world > 1: the per-move all-gather of the move records
         self._episodes = None    # world > 1, rank 0: the episode store of all n_games, filled from the gathered records
         self._mismatches = 0     # world > 1, rank 0: gathered records that were not the game of their row (cumulative)
+        self._replay_status = 0  # world > 1, rank 0: the replay ring's status word as read at the end of the loop
 
     def _latent_dtype(self):
         return _lib.LATENT_BF16 if self.acting_mode == _lib.MODE_BF16 else _lib.LATENT_F32
@@ -123,31 +127,54 @@ class BatchedMuzero:
         return finished, (length_sum / finished if finished else float("nan")), stored
 
     def _end_loop(self, row):
-        """world > 1, every rank: rank 0's weights, episode count, whether an update changed the weights and the loop's
-        history row are broadcast, so that every rank repacks its acting weights when one GPU would and returns the same
-        history.  Raises if rank 0 found gathered records out of order."""
-        info = torch.tensor([self.episodes_done, float(self._weights_dirty), self._mismatches, *row[1:]], dtype=torch.float64,
-                            device=self.learner.device)
+        """world > 1, every rank: rank 0's weights, episode count, whether an update changed the weights, the replay
+        ring's status and the loop's history row are broadcast, so that every rank repacks its acting weights when one GPU
+        would, returns the same history and raises what rank 0 raises.  Raises if rank 0 found gathered records out of
+        order or a replay draw / priority write-back that the reference would have rejected."""
+        info = torch.tensor([self.episodes_done, float(self._weights_dirty), self._mismatches, self._replay_status, *row[1:]],
+                            dtype=torch.float64, device=self.learner.device)
         dist.broadcast(self.learner.params, 0)
         dist.broadcast(info, 0)
-        episodes_done, dirty, mismatches, *rest = info.tolist()
+        episodes_done, dirty, mismatches, replay_status, *rest = info.tolist()
         if mismatches:
             raise RuntimeError(f"{int(mismatches)} gathered move records were not the game of their row (game_lo check): the "
                                "all-gathered records are out of order")
+        ReplayRing.raise_for_status(int(replay_status))
         self.episodes_done, self._weights_dirty = int(episodes_done), bool(dirty)
         return (row[0], *rest)
 
-    def update(self):
-        """One Muzero._update on a batch drawn from the replay ring (Muzero.py:104-127)."""
+    def step(self):
+        """One Muzero._update (Muzero.py:104-127) on a batch drawn from the replay ring, enqueued without a host round
+        trip: the host draws the random numbers from NumPy's global RandomState exactly as the reference does, the draw
+        itself (ReplayRing.priority_sample_device / uniform_sample_device), the learner step and the priority write-back
+        run on the device.  Returns the losses (value, reward, policy) as the learner's device buffer, which the next
+        update overwrites.  Errors the reference would raise accumulate in self.buffer.status."""
         if self.priority_replay:
-            states, rwds, actions, pi_probs, returns, indx, w = self.buffer.priority_sample(self.batch_s)
+            states, rwds, actions, pi_probs, returns, indx, w = self.buffer.priority_sample_device(self.batch_s)
         else:
-            states, rwds, actions, pi_probs, returns = self.buffer.uniform_sample(self.batch_s)
+            states, rwds, actions, pi_probs, returns = self.buffer.uniform_sample_device(self.batch_s)
             indx, w = None, None
-        new_p, v_loss, r_loss, p_loss = self.learner.update(states, rwds, actions, pi_probs, returns, w)
+        if "update" in vars(self.learner):
+            # Learner.update replaced on the instance (a hook that inspects every update): it is driven, read-back included
+            new_p, *losses = self.learner.update(states, rwds, actions, pi_probs, returns, w)
+            losses = torch.tensor(losses, dtype=torch.float32, device=self.learner.device)
+        else:
+            new_p, losses = self.learner.step(states, rwds, actions, pi_probs, returns, w)
         self._weights_dirty = True
-        self.buffer.update_priorities(indx, new_p)
-        return v_loss, r_loss, p_loss
+        self.buffer.update_priorities_device(indx, new_p)
+        return losses
+
+    def _read_back(self, losses):
+        """(value, reward, policy loss) and the replay ring's status word in one read-back."""
+        *vals, status = torch.cat([losses.to(torch.float64), self.buffer.status.to(torch.float64)]).tolist()
+        return tuple(vals), int(status)
+
+    def update(self):
+        """One update (step) and its read-back: -> (value loss, reward loss, policy loss) as Muzero._update returns them;
+        raises what the reference would have raised."""
+        losses, status = self._read_back(self.step())
+        ReplayRing.raise_for_status(status)
+        return losses
 
     def training_loop(self, n_loops, min_replay_size, print_acc=None, log=print):
         """-> list of (loop, mean episode length of the loop, value loss, reward loss, policy loss)."""
@@ -156,9 +183,14 @@ class BatchedMuzero:
             self._refresh_actor(adjust_temperature(self.episodes_done // max(1, self.B)))
             finished, mean_len, _ = self.play(self.moves_per_loop)
             losses = (float("nan"),) * 3
-            if self.rank == 0 and not self._mismatches and len(self.buffer) > min_replay_size:
+            if self.rank == 0 and not self._mismatches and len(self.buffer) > min_replay_size and self.n_update_x_loop > 0:
                 for _ in range(self.n_update_x_loop):
-                    losses = self.update()
+                    dev_losses = self.step()
+                # the loop's one read-back of its updates: the last update's losses and the replay ring's status word, so
+                # a draw the reference would reject raises here, at the end of the loop, rather than at its update
+                losses, self._replay_status = self._read_back(dev_losses)
+                if self.world == 1:
+                    ReplayRing.raise_for_status(self._replay_status)
             row = (n, mean_len, *losses)
             history.append(self._end_loop(row) if self.world > 1 else row)
             mean_len, losses = history[-1][1], history[-1][2:]

@@ -3,7 +3,7 @@
     python tools/learner_audit.py [--disks 3] [--games 1024] [--loops 400] [--out profiles/learner_audit_n3_g1024.json]
 
 Trains exactly as examples/train_hanoi.py does with the same arguments (same seeds, torch default init, 25 simulations,
-8 updates per loop, min_replay_size 5,000).  Before each Learner.update it snapshots the batch, parameters, Adam moments
+8 updates per loop, min_replay_size 5,000).  Before each Learner.step it snapshots the batch, parameters, Adam moments
 and step index; after it, it compares every gradient, the parameters, moments, new priorities and losses with the
 one-step float64 reference from that snapshot (float32 yardstick on the CPU) under the gates of
 tests/test_learner_reference.py.  Writes one JSON document: the card name and power limit, every update that failed a
@@ -52,25 +52,26 @@ def main():
     net = MuZeroNet(3 * args.disks, 6, LR, "cpu", TD_return=True)
     mz = BatchedMuzero(net.state_dict(), args.disks, 200, args.games, n_mcts_simulations=args.sims,
                        n_update_x_loop=args.updates_per_loop, seed=args.seed)
-    ln, orig, rows = mz.learner, mz.learner.update, []
+    # the hook sits on Learner.step, the entry point BatchedMuzero's updates call (Learner.update is step + read-back)
+    ln, orig, rows = mz.learner, mz.learner.step, []
     loop = [0]
 
     def audited(states, rwds, actions, pi_probs, returns, priority_w=None, apply_update=True):
         batch = [t.clone() for t in (states, rwds, actions, pi_probs, returns)]
         w = None if priority_w is None else priority_w.clone()
         before, step_index = snapshot(ln), ln.step_index + 1
-        out = orig(states, rwds, actions, pi_probs, returns, priority_w, apply_update)
-        kern = dict(grads=ln.grad_dict(), **snapshot(ln), priorities=None if out[0] is None else torch.from_numpy(out[0]),
-                    losses=np.array(out[1:]))
+        new_p, losses = orig(states, rwds, actions, pi_probs, returns, priority_w, apply_update)
+        kern = dict(grads=ln.grad_dict(), **snapshot(ln), priorities=None if new_p is None else new_p.cpu(),
+                    losses=np.array(losses.cpu().tolist()))
         stats, ref = lref.compare_update(kern, before, step_index, batch, w, LR, ref_device="cuda")
         worst, bad = lref.check(stats, GATES)
         rows.append(dict(update=step_index, loop=loop[0], hazard_rows=int(lref.hazard_rows(ref).sum()), failing=bad,
                          worst={c: max(v) for c, v in worst.items()}))
         if bad:
             print(f"update {step_index} (loop {loop[0]}): {len(bad)} tensors fail: {bad[:6]}", flush=True)
-        return out
+        return new_p, losses
 
-    ln.update = audited
+    ln.step = audited
 
     def log(msg):
         print(msg, flush=True)
