@@ -206,10 +206,9 @@ __global__ void __launch_bounds__(256) episode_unroll(
           for (int e = 1; e < ex_at; ++e) y = __dmul_rn(y, x);
           wv[a] = y;
         }
-        double rest = 0.0;  // np.sum of 6 doubles: first element + (0 + the rest, left to right)
+        double tot = wv[0];  // np.sum of 6 doubles: left to right (NumPy sums arrays shorter than 8 sequentially)
 #pragma unroll
-        for (int a = 1; a < 6; ++a) rest = __dadd_rn(rest, wv[a]);
-        const double tot = __dadd_rn(wv[0], rest);
+        for (int a = 1; a < 6; ++a) tot = __dadd_rn(tot, wv[a]);
 #pragma unroll
         for (int a = 0; a < 6; ++a) buf_pi[o * 6 + a] = (float)__ddiv_rn(wv[a], tot);
       } else {  // absorbing padding (Muzero.py:296-307): reward 0, return 0, one random action, uniform policy
@@ -267,10 +266,9 @@ __global__ void __launch_bounds__(128) episode_unroll_warp(
         for (int e = 1; e < ex_at; ++e) y = __dmul_rn(y, x);
         wv[a] = y;
       }
-      double rest = 0.0;  // np.sum of 6 doubles: first element + (0 + the rest, left to right)
+      double tot = wv[0];  // np.sum of 6 doubles: left to right (NumPy sums arrays shorter than 8 sequentially)
 #pragma unroll
-      for (int a = 1; a < 6; ++a) rest = __dadd_rn(rest, wv[a]);
-      const double tot = __dadd_rn(wv[0], rest);
+      for (int a = 1; a < 6; ++a) tot = __dadd_rn(tot, wv[a]);
 #pragma unroll
       for (int a = 0; a < 6; ++a) st.pi[a] = (float)__ddiv_rn(wv[a], tot);
       stage[t] = st;

@@ -698,11 +698,11 @@ __device__ __forceinline__ RootPolicy root_policy_eval(const hmz_node_t* root, d
       w[a] = pow(x, ex);
     }
   }
-  // np.sum of 6 doubles: first element + (0 + the rest, left to right)
-  double rest = 0.0;
+  // np.sum of 6 doubles: left to right (NumPy sums arrays shorter than 8 sequentially; the order matters once the
+  // powers pass 2^53, e.g. exponent 5 with about 1,000 visits)
+  double total = w[0];
 #pragma unroll
-  for (int a = 1; a < 6; ++a) rest = __dadd_rn(rest, w[a]);
-  const double total = __dadd_rn(w[0], rest);
+  for (int a = 1; a < 6; ++a) total = __dadd_rn(total, w[a]);
 #pragma unroll
   for (int a = 0; a < 6; ++a) out.prob[a] = __ddiv_rn(w[a], total);
   int act = 0;
