@@ -7,7 +7,7 @@ import os
 import threading
 
 PKG_DIR = os.path.dirname(os.path.abspath(__file__))
-# HMZ_LIB_PATH (tooling): load another build of the library, e.g. an A/B variant produced by tools/build_variant.sh
+# HMZ_LIB_PATH (tooling): load another build of the library, e.g. an A/B variant that build.py wrote under HMZ_VARIANT
 LIB_PATH = os.environ.get("HMZ_LIB_PATH") or os.path.join(PKG_DIR, "libhmz.so")
 
 OK, ERR_INVALID, ERR_CUDA, ERR_UNSUPPORTED = 0, -1, -2, -3

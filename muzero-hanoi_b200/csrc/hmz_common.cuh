@@ -46,28 +46,10 @@ struct ProfScope {
 __device__ __forceinline__ void pdl_wait() { asm volatile("griddepcontrol.wait;" ::: "memory"); }
 __device__ __forceinline__ void pdl_launch_dependents() { asm volatile("griddepcontrol.launch_dependents;" ::: "memory"); }
 
-// HMZ_PDL (tuning switch): bit 0 = the network kernels, bit 1 = the tree kernel launch as programmatic dependents,
-// bit 2 = the tree kernel loads what the previous tree kernel wrote BEFORE it waits for the network kernel (the
-// network kernel then signals its dependents only after its own wait, see pdl_prewait()).
-inline int pdl_mask() {
-  static const int mask = getenv("HMZ_PDL") ? atoi(getenv("HMZ_PDL")) : 7;
-  return mask;
-}
-inline int pdl_prewait() { return (pdl_mask() >> 2) & 1; }
-// Where a kernel signals its dependents (tuning switches).  HMZ_PDL_NET_AT: -1 = at the start of the network
-// kernel (after its wait when bit 2 of HMZ_PDL is set), k in 0..3 = when the last pass starts network k, 4 = at exit.
-// HMZ_PDL_TREE_AT: 0 = at the start of the tree kernel, 1 = after the backup, 2 = after the select walk, 3 = at exit.
-inline int pdl_net_at() {
-  static const int v = getenv("HMZ_PDL_NET_AT") ? atoi(getenv("HMZ_PDL_NET_AT")) : -1;
-  return v;
-}
-inline int pdl_tree_at() {
-  static const int v = getenv("HMZ_PDL_TREE_AT") ? atoi(getenv("HMZ_PDL_TREE_AT")) : 0;
-  return v;
-}
-
+// Launches `kernel` as a programmatic dependent of its stream predecessor.  The network kernels and the tree
+// kernel launch this way; each signals its own dependents early (see net_tc_body and tree_phase).
 template <typename... KArgs, typename... Args>
-inline cudaError_t launch_pdl(int kind_bit, void (*kernel)(KArgs...), dim3 grid, dim3 block, size_t smem, cudaStream_t stream,
+inline cudaError_t launch_pdl(void (*kernel)(KArgs...), dim3 grid, dim3 block, size_t smem, cudaStream_t stream,
                               Args... args) {
   cudaLaunchConfig_t cfg = {};
   cfg.gridDim = grid;
@@ -78,7 +60,7 @@ inline cudaError_t launch_pdl(int kind_bit, void (*kernel)(KArgs...), dim3 grid,
   attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
   attr[0].val.programmaticStreamSerializationAllowed = 1;
   cfg.attrs = attr;
-  cfg.numAttrs = (pdl_mask() & kind_bit) ? 1 : 0;
+  cfg.numAttrs = 1;
   return cudaLaunchKernelEx(&cfg, kernel, static_cast<KArgs>(args)...);
 }
 

@@ -12,39 +12,25 @@
 namespace hmz {
 
 // ------------------------------------------------------------------------------ kernels
-// One thread owns U vec4 groups per grid-stride iteration, spaced a block apart so that every load / store instruction
-// of a warp covers one contiguous 512-byte (words, rewards) or 128-byte (actions, flags) span; all U groups' loads are
-// issued before the first use.  Measured on the B200 (tools/gpu_round.sh envsweep, 2^24 envs): U = 1 4.19-4.26 TB/s,
-// U = 2 4.0, U = 4 3.9 — more bytes in flight per thread do not help (2,048 resident threads per SM already cover the
-// latency-bandwidth product), so U = 1 is the default (HMZ_ENV_UNROLL / HMZ_ENV_CTAS are tuning switches).
-template <bool kObs, int U>
+// One thread owns one vec4 group per grid-stride iteration, so that every load / store instruction of a warp covers one
+// contiguous 512-byte (words, rewards) or 128-byte (actions, flags) span.  Measured on the B200 (2^24 envs), with U vec4
+// groups per thread and iteration: U = 1 4.19-4.26 TB/s, U = 2 4.0, U = 4 3.9 — more bytes in flight per thread do not
+// help (2,048 resident threads per SM already cover the latency-bandwidth product); the unrolled forms have been removed.
+template <bool kObs>
 __global__ void __launch_bounds__(256) env_step_vec4(uint4* __restrict__ words, const uchar4* __restrict__ actions,
                                                     float4* __restrict__ rewards, uchar4* __restrict__ flags,
                                                     uint4* __restrict__ obs_words, int64_t n_vec, EnvCfg c) {
-  const int64_t tile = (int64_t)U * blockDim.x;
-  for (int64_t base = blockIdx.x * tile + threadIdx.x; base < n_vec; base += (int64_t)gridDim.x * tile) {
-    uint4 w[U];
-    uchar4 a[U];
-#pragma unroll
-    for (int k = 0; k < U; ++k) {
-      const int64_t i = base + (int64_t)k * blockDim.x;
-      if (i < n_vec) {  // every byte is touched exactly once per launch: streaming loads / stores
-        w[k] = __ldcs(words + i);
-        a[k] = __ldcs(actions + i);
-      }
-    }
-#pragma unroll
-    for (int k = 0; k < U; ++k) {
-      const int64_t i = base + (int64_t)k * blockDim.x;
-      if (i >= n_vec) continue;
-      const StepOut o0 = step_word(w[k].x, a[k].x, c), o1 = step_word(w[k].y, a[k].y, c), o2 = step_word(w[k].z, a[k].z, c),
-                    o3 = step_word(w[k].w, a[k].w, c);
-      __stcs(words + i, make_uint4(o0.word, o1.word, o2.word, o3.word));
-      __stcs(rewards + i, make_float4(o0.reward, o1.reward, o2.reward, o3.reward));
-      __stcs(flags + i, make_uchar4((unsigned char)o0.flags, (unsigned char)o1.flags, (unsigned char)o2.flags,
-                                    (unsigned char)o3.flags));
-      if (kObs) __stcs(obs_words + i, make_uint4(o0.obs_word, o1.obs_word, o2.obs_word, o3.obs_word));
-    }
+  for (int64_t i = blockIdx.x * (int64_t)blockDim.x + threadIdx.x; i < n_vec; i += (int64_t)gridDim.x * blockDim.x) {
+    // every byte is touched exactly once per launch: streaming loads / stores
+    const uint4 w = __ldcs(words + i);
+    const uchar4 a = __ldcs(actions + i);
+    const StepOut o0 = step_word(w.x, a.x, c), o1 = step_word(w.y, a.y, c), o2 = step_word(w.z, a.z, c),
+                  o3 = step_word(w.w, a.w, c);
+    __stcs(words + i, make_uint4(o0.word, o1.word, o2.word, o3.word));
+    __stcs(rewards + i, make_float4(o0.reward, o1.reward, o2.reward, o3.reward));
+    __stcs(flags + i, make_uchar4((unsigned char)o0.flags, (unsigned char)o1.flags, (unsigned char)o2.flags,
+                                  (unsigned char)o3.flags));
+    if (kObs) __stcs(obs_words + i, make_uint4(o0.obs_word, o1.obs_word, o2.obs_word, o3.obs_word));
   }
 }
 
@@ -62,33 +48,21 @@ __global__ void __launch_bounds__(256) env_step_scalar(uint32_t* __restrict__ wo
   }
 }
 
-template <int U>
 __global__ void __launch_bounds__(256) env_step_random_vec4(uint4* __restrict__ words, uchar4* __restrict__ actions,
                                                            float4* __restrict__ rewards, uchar4* __restrict__ flags,
                                                            int64_t n_vec, EnvCfg c, uint32_t seed_lo, uint32_t seed_hi,
                                                            uint32_t step_lo, uint32_t step_hi) {
-  const int64_t tile = (int64_t)U * blockDim.x;
-  for (int64_t base = blockIdx.x * tile + threadIdx.x; base < n_vec; base += (int64_t)gridDim.x * tile) {
-    uint4 w[U];
-#pragma unroll
-    for (int k = 0; k < U; ++k) {
-      const int64_t i = base + (int64_t)k * blockDim.x;
-      if (i < n_vec) w[k] = __ldcs(words + i);
-    }
-#pragma unroll
-    for (int k = 0; k < U; ++k) {
-      const int64_t i = base + (int64_t)k * blockDim.x;
-      if (i >= n_vec) continue;
-      const Philox4 r = philox4x32_10((uint32_t)i, (uint32_t)(i >> 32), step_lo, step_hi, seed_lo, seed_hi);
-      uint32_t a0, a1, a2, a3;
-      const StepOut o0 = step_random_word(w[k].x, r.x, c, a0), o1 = step_random_word(w[k].y, r.y, c, a1),
-                    o2 = step_random_word(w[k].z, r.z, c, a2), o3 = step_random_word(w[k].w, r.w, c, a3);
-      __stcs(words + i, make_uint4(o0.word, o1.word, o2.word, o3.word));
-      __stcs(actions + i, make_uchar4((unsigned char)a0, (unsigned char)a1, (unsigned char)a2, (unsigned char)a3));
-      __stcs(rewards + i, make_float4(o0.reward, o1.reward, o2.reward, o3.reward));
-      __stcs(flags + i, make_uchar4((unsigned char)o0.flags, (unsigned char)o1.flags, (unsigned char)o2.flags,
-                                    (unsigned char)o3.flags));
-    }
+  for (int64_t i = blockIdx.x * (int64_t)blockDim.x + threadIdx.x; i < n_vec; i += (int64_t)gridDim.x * blockDim.x) {
+    const uint4 w = __ldcs(words + i);
+    const Philox4 r = philox4x32_10((uint32_t)i, (uint32_t)(i >> 32), step_lo, step_hi, seed_lo, seed_hi);
+    uint32_t a0, a1, a2, a3;
+    const StepOut o0 = step_random_word(w.x, r.x, c, a0), o1 = step_random_word(w.y, r.y, c, a1),
+                  o2 = step_random_word(w.z, r.z, c, a2), o3 = step_random_word(w.w, r.w, c, a3);
+    __stcs(words + i, make_uint4(o0.word, o1.word, o2.word, o3.word));
+    __stcs(actions + i, make_uchar4((unsigned char)a0, (unsigned char)a1, (unsigned char)a2, (unsigned char)a3));
+    __stcs(rewards + i, make_float4(o0.reward, o1.reward, o2.reward, o3.reward));
+    __stcs(flags + i, make_uchar4((unsigned char)o0.flags, (unsigned char)o1.flags, (unsigned char)o2.flags,
+                                  (unsigned char)o3.flags));
   }
 }
 
@@ -229,16 +203,6 @@ int make_env_cfg(EnvCfg& c, int n_disks, int max_steps, int goal_peg, int auto_r
   return HMZ_OK;
 }
 
-// Tuning switches (read once): vec4 groups per thread and iteration (1, 2 or 4) and resident CTAs per SM the grid is sized for.
-static int env_unroll() {
-  static const int u = getenv("HMZ_ENV_UNROLL") ? atoi(getenv("HMZ_ENV_UNROLL")) : 1;
-  return u == 2 || u == 4 ? u : 1;
-}
-static int env_ctas_per_sm() {
-  static const int v = getenv("HMZ_ENV_CTAS") ? atoi(getenv("HMZ_ENV_CTAS")) : 8;
-  return v >= 1 && v <= 8 ? v : 8;
-}
-
 static bool aligned16(const void* p) { return (reinterpret_cast<uintptr_t>(p) & 15u) == 0; }
 static bool aligned4(const void* p) { return (reinterpret_cast<uintptr_t>(p) & 3u) == 0; }
 
@@ -306,20 +270,9 @@ int hmz_env_step(uint32_t* words, const uint8_t* actions, float* rewards, uint8_
              (!obs_words || aligned16(obs_words));
   int64_t n_vec = vec ? n / 4 : 0;
   if (n_vec > 0) {
-    const int u = env_unroll();
-    unsigned grid = grid_for(n_vec, 256 * u, env_ctas_per_sm());
-    uint4* w4 = (uint4*)words;
-    const uchar4* a4 = (const uchar4*)actions;
-    float4* r4 = (float4*)rewards;
-    uchar4* f4 = (uchar4*)flags;
-    uint4* o4 = (uint4*)obs_words;
-#define HMZ_ENV_LAUNCH(OBS, U) env_step_vec4<OBS, U><<<grid, 256, 0, st>>>(w4, a4, r4, f4, o4, n_vec, c)
-    if (obs_words) {
-      if (u == 1) HMZ_ENV_LAUNCH(true, 1); else if (u == 2) HMZ_ENV_LAUNCH(true, 2); else HMZ_ENV_LAUNCH(true, 4);
-    } else {
-      if (u == 1) HMZ_ENV_LAUNCH(false, 1); else if (u == 2) HMZ_ENV_LAUNCH(false, 2); else HMZ_ENV_LAUNCH(false, 4);
-    }
-#undef HMZ_ENV_LAUNCH
+    const unsigned grid = grid_for(n_vec, 256, 8);
+    (obs_words ? env_step_vec4<true> : env_step_vec4<false>)<<<grid, 256, 0, st>>>(
+        (uint4*)words, (const uchar4*)actions, (float4*)rewards, (uchar4*)flags, (uint4*)obs_words, n_vec, c);
     if (int rc = check_launch("env_step_vec4")) return rc;
   }
   if (n_vec * 4 < n) {
@@ -372,15 +325,9 @@ int hmz_env_step_random(uint32_t* words, uint8_t* actions, float* rewards, uint8
   if (int rc = make_env_cfg(c, n_disks, max_steps, goal_peg, 1, reset_word)) return rc;
   if (n % 4 != 0 || !aligned16(words) || !aligned4(actions) || !aligned16(rewards) || !aligned4(flags))
     return fail(HMZ_ERR_INVALID, "hmz_env_step_random: n_envs must be a multiple of 4 and buffers 16-byte aligned");
-  const int u = env_unroll();
-  const unsigned grid = grid_for(n / 4, 256 * u, env_ctas_per_sm());
-#define HMZ_ENV_LAUNCH(U)                                                                                              \
-  env_step_random_vec4<U><<<grid, 256, 0, (cudaStream_t)stream>>>((uint4*)words, (uchar4*)actions, (float4*)rewards, \
-                                                                  (uchar4*)flags, n / 4, c, (uint32_t)seed,          \
-                                                                  (uint32_t)(seed >> 32), (uint32_t)step_index,      \
-                                                                  (uint32_t)(step_index >> 32))
-  if (u == 1) HMZ_ENV_LAUNCH(1); else if (u == 2) HMZ_ENV_LAUNCH(2); else HMZ_ENV_LAUNCH(4);
-#undef HMZ_ENV_LAUNCH
+  env_step_random_vec4<<<grid_for(n / 4, 256, 8), 256, 0, (cudaStream_t)stream>>>(
+      (uint4*)words, (uchar4*)actions, (float4*)rewards, (uchar4*)flags, n / 4, c, (uint32_t)seed, (uint32_t)(seed >> 32),
+      (uint32_t)step_index, (uint32_t)(step_index >> 32));
   return check_launch("env_step_random_vec4");
 }
 

@@ -27,17 +27,9 @@ namespace hmz {
 
 namespace tc {
 namespace v4 {
-// HMZ_TC_MAXNREG (tuning switch): cap the kernel at fewer registers so that tree-kernel blocks of other search
-// groups can share the SM (704 threads x 64 registers leave 20 K registers = two 128-thread blocks at 80);
-// measured: no gain, the default keeps 80 registers
-#ifdef HMZ_TC_MAXNREG
-#define HMZ_TC_BOUNDS __maxnreg__(HMZ_TC_MAXNREG)
-#else
-#define HMZ_TC_BOUNDS __launch_bounds__(kLaunchThreads, 1)
-#endif
 // The stand-alone kernels: one launch per network evaluation of a whole batch (grid = min(tile pairs, SMs)).
 template <bool kInitial>
-__global__ void HMZ_TC_BOUNDS net_tc(const __grid_constant__ TcArgs a) {
+__global__ void __launch_bounds__(kLaunchThreads, 1) net_tc(const __grid_constant__ TcArgs a) {
   extern __shared__ uint8_t smem_raw[];
   net_tc_body<kInitial, false>(a, PersistCtl{}, smem_raw, (int)blockIdx.x, (int)gridDim.x);
 }
@@ -135,28 +127,18 @@ static int tc_prepare(int* smem_bytes) {
   if (done_dev != dev) {
     cudaError_t e = cudaFuncSetAttribute(tc::v4::net_tc<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, *smem_bytes);
     if (e == cudaSuccess) e = cudaFuncSetAttribute(tc::v4::net_tc<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, *smem_bytes);
-    const int carve = getenv("HMZ_TC_CARVEOUT") ? atoi(getenv("HMZ_TC_CARVEOUT")) : -1;  // tuning switch, default: unset
-    if (e == cudaSuccess && carve >= 0) e = cudaFuncSetAttribute(tc::v4::net_tc<false>, cudaFuncAttributePreferredSharedMemoryCarveout, carve);
-    if (e == cudaSuccess && carve >= 0) e = cudaFuncSetAttribute(tc::v4::net_tc<true>, cudaFuncAttributePreferredSharedMemoryCarveout, carve);
     if (e != cudaSuccess) return fail(HMZ_ERR_CUDA, "cudaFuncSetAttribute(net_tc): %s", cudaGetErrorString(e));
     done_dev = dev;
   }
   return HMZ_OK;
 }
 
-// Tile pairs per CTA the recurrent launch aims for (tuning switch HMZ_TC_PASSES, default 1): with several search groups in
-// flight a CTA that runs two passes pays the kernel's prologue (barrier init, TMEM allocation, first weight blocks,
-// ~1.9 us of a ~12.5 us single-pass CTA) once for both, at the price of a longer launch.
-static int tc_passes() {
-  static const int v = getenv("HMZ_TC_PASSES") ? atoi(getenv("HMZ_TC_PASSES")) : 1;
-  return v < 1 ? 1 : v;
-}
-static unsigned tc_grid(int64_t n, int* n_pairs, int passes = 1) {
+// One tile pair per CTA while there are SMs for it (DESIGN §9: two passes per CTA did not pay).
+static unsigned tc_grid(int64_t n, int* n_pairs) {
   const int64_t pairs = (n + 2 * tc::kM - 1) / (2 * tc::kM);
   const int sms = sm_count();
   *n_pairs = (int)pairs;
-  const int64_t want = (pairs + passes - 1) / passes;
-  return (unsigned)(want < sms ? want : sms);
+  return (unsigned)(pairs < sms ? pairs : sms);
 }
 
 int tc_net_recurrent(const void* weights, const void* lat_in, int64_t in_rows_per_item, const uint16_t* in_row,
@@ -165,11 +147,10 @@ int tc_net_recurrent(const void* weights, const void* lat_in, int64_t in_rows_pe
                      int64_t weight_stride, bool allow_head_split) {
   int smem = 0, n_pairs = 0;
   if (int rc = tc_prepare(&smem)) return rc;
-  unsigned grid = tc_grid(n, &n_pairs, tc_passes());
+  unsigned grid = tc_grid(n, &n_pairs);
   tc::v4::TcArgs a{};
-  // small batches: three CTAs per tile pair, one head each (TcArgs::head_split); HMZ_TC_SPLIT=0 switches it off
-  static const int split_on = getenv("HMZ_TC_SPLIT") ? atoi(getenv("HMZ_TC_SPLIT")) : 1;
-  a.head_split = (split_on && allow_head_split && 3 * n_pairs <= sm_count()) ? 3 : 1;
+  // small batches: three CTAs per tile pair, one head each (TcArgs::head_split)
+  a.head_split = (allow_head_split && 3 * n_pairs <= sm_count()) ? 3 : 1;
   if (a.head_split == 3) grid = 3u * (unsigned)n_pairs;
   a.wsec = (const uint8_t*)weights;
   a.block_set = block_set;
@@ -187,9 +168,9 @@ int tc_net_recurrent(const void* weights, const void* lat_in, int64_t in_rows_pe
   a.v_out = v;
   a.n = n;
   a.n_pairs = n_pairs;
-  a.timeline = tc_timeline_enabled() | (pdl_prewait() << 1) | ((pdl_net_at() + 1) << 2);
+  a.timeline = tc_timeline_enabled();
   a.gantt = gantt_next(0, gantt_context_tag());
-  cudaError_t e = launch_pdl(1, tc::v4::net_tc<false>, dim3(grid), dim3(tc::v4::kLaunchThreads), (size_t)smem, stream, a);
+  cudaError_t e = launch_pdl(tc::v4::net_tc<false>, dim3(grid), dim3(tc::v4::kLaunchThreads), (size_t)smem, stream, a);
   if (e != cudaSuccess) return fail(HMZ_ERR_CUDA, "net_tc<recurrent> launch: %s", cudaGetErrorString(e));
   return check_launch("net_tc<recurrent>");
 }
@@ -216,8 +197,7 @@ int tc_net_initial(const void* weights, int n_disks, const uint32_t* words, void
   a.n = n;
   a.n_pairs = n_pairs;
   a.head_split = 1;
-  a.timeline = (pdl_prewait() << 1) | ((pdl_net_at() + 1) << 2);
-  cudaError_t e = launch_pdl(1, tc::v4::net_tc<true>, dim3(grid), dim3(tc::v4::kLaunchThreads), (size_t)smem, stream, a);
+  cudaError_t e = launch_pdl(tc::v4::net_tc<true>, dim3(grid), dim3(tc::v4::kLaunchThreads), (size_t)smem, stream, a);
   if (e != cudaSuccess) return fail(HMZ_ERR_CUDA, "net_tc<initial> launch: %s", cudaGetErrorString(e));
   return check_launch("net_tc<initial>");
 }

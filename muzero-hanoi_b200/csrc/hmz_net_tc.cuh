@@ -350,7 +350,7 @@ struct TcArgs {
   int head_split;             // 3: small batches (3 x tile pairs <= SMs) — CTAs 3 p, 3 p + 1, 3 p + 2 all run the dynamics network
                               // of pair p and then ONE head each (reward + the latent rows / value / policy): the per-simulation
                               // chain of a pass shrinks from four networks to two while idle SMs do the redundant work; else 1
-  int timeline;               // tooling / PDL switches of the stand-alone kernels
+  int timeline;               // tooling (HMZ_TC_TIMELINE): bit 0 = record phase marks, bits 8+ = the traced pass
   unsigned long long* gantt;  // tooling (hmz_debug_gantt), nullable
   const uint16_t* block_set;  // nullable (stand-alone kernels only): weight set of each tile pair (hmz_multi_t), at
   int64_t weight_stride;      // wsec + block_set[pair] * weight_stride
@@ -378,20 +378,13 @@ struct PersistCtl {
   int rotate;                 // 1: a CTA's residue class of tile pairs rotates by n_pairs % n_cta per simulation, so that with a CTA
                               // count that does not divide the pair count every CTA gets the extra pass equally often
 };
-#ifdef HMZ_PERSIST_STATS  // tooling build (tools/build_variant.py): role statistics of the persistent kernel
+#ifdef HMZ_PERSIST_STATS  // tooling build (HMZ_VARIANT with HMZ_NVCC_EXTRA=-DHMZ_PERSIST_STATS): role statistics of the persistent kernel
 constexpr bool kPersistStats = true;
 #else
 constexpr bool kPersistStats = false;
 #endif
-// Back-off between two polls of a hand-off word (ns; 0 = poll back to back).  Tuning switch.
-#ifdef HMZ_PERSIST_SLEEP_NS
-#define HMZ_PERSIST_SLEEP_NS_SET 1  // (hmz_build_flags reports a non-default value)
-#else
-#define HMZ_PERSIST_SLEEP_NS 64
-#endif
-__device__ __forceinline__ void persist_backoff() {
-  if (HMZ_PERSIST_SLEEP_NS > 0) __nanosleep(HMZ_PERSIST_SLEEP_NS);
-}
+// Back-off between two polls of a hand-off word.
+__device__ __forceinline__ void persist_backoff() { __nanosleep(64); }
 constexpr int kSlicesPerPair = 16;       // warps (16 searches each) per 256-search tile pair
 __device__ __forceinline__ uint32_t ld_relaxed_u32(const uint32_t* p) {
   uint32_t v;
@@ -486,7 +479,7 @@ __device__ __forceinline__ void net_tc_body(const TcArgs& a, const PersistCtl& p
   float* __restrict__ v_out = a.v_out;
   const int64_t n = a.n;
   const int n_pairs = a.n_pairs;
-  const int timeline = a.timeline;  // (persistent passes: only the tooling bits 0 and 8+ are set)
+  const int timeline = a.timeline;
   // passes of this CTA: its tile pairs, once (stand-alone) or once per simulation (persistent)
   // (pair, sim) sequence of this CTA: in simulation s it owns the pairs first_pair(s), first_pair(s) + n_cta, ...
   const int rot = (kPersist && pc.rotate) ? n_pairs % n_cta : 0;
@@ -566,14 +559,9 @@ __device__ __forceinline__ void net_tc_body(const TcArgs& a, const PersistCtl& p
   // The dependents (the next tree kernel) are signalled only AFTER this kernel's own wait: that kernel reads
   // what the previous tree kernel wrote before it waits for this one, so it must not start before the
   // previous tree kernel has completed.  (The loader warp waits after its first four weight blocks.)
-  const bool late_signal = !kPersist && (timeline & 2) != 0;  // HMZ_PDL bit 2
-  const int signal_net = kPersist ? 8 : ((timeline >> 2) & 7) - 1;  // HMZ_PDL_NET_AT: -1 = here (8: never)
-  if (!kPersist) {
-    if (!late_signal && signal_net < 0) pdl_launch_dependents();
-    if (warp != kLoaderWarp && (late_signal || (warp != kMmaWarp && warp != kMmaWarp1))) {
-      pdl_wait();
-      if (late_signal && signal_net < 0) pdl_launch_dependents();
-    }
+  if (!kPersist && warp != kLoaderWarp) {
+    pdl_wait();
+    pdl_launch_dependents();
   }
   TL4_CTA(62);
 
@@ -590,9 +578,9 @@ __device__ __forceinline__ void net_tc_body(const TcArgs& a, const PersistCtl& p
       for (int i = 0; i < 8; ++i) {
         if (kInitial && (i >> 1) == 1) continue;  // no reward head at the root
         if (!runs(i >> 1)) continue;
-        if (late_signal && pass == 0 && issued == (split == 1 ? 4 : 2)) {  // the first blocks are in flight: now order after the preceding kernel
+        if (!kPersist && pass == 0 && issued == (split == 1 ? 4 : 2)) {  // the first blocks are in flight: now order after the preceding kernel
           pdl_wait();
-          if (signal_net < 0) pdl_launch_dependents();
+          pdl_launch_dependents();
         }
         ++issued;
         const int kind = i & 1, slot = (i >> 1) & 1;
@@ -621,7 +609,6 @@ __device__ __forceinline__ void net_tc_body(const TcArgs& a, const PersistCtl& p
       for (int net = 0; net < 4; ++net) {  // dynamics / representation, reward, value, policy
         if (kInitial && net == 1) continue;
         if (!runs(net)) continue;
-        if (t == 0 && net == signal_net && pass == n_pass - 1) pdl_launch_dependents();
         // ---- first layer: H[0:256) = [A | AX] x W1'^T
         {
           const uint32_t slot = (uint32_t)net & 1u, use = slot ? use1 : use0;  // both layers of a network use slot (net & 1)

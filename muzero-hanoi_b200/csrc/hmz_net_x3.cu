@@ -755,9 +755,8 @@ int net_recurrent(const void* weights, const void* lat_in, int64_t in_rows_per_i
   a.n = n;
   a.n_tiles = (int)((n + kM - 1) / kM);
   const int sms = sm_count();
-  // small batches: three CTAs per tile, one head each (HMZ_TC_SPLIT=0 switches it off)
-  static const int split_on = getenv("HMZ_TC_SPLIT") ? atoi(getenv("HMZ_TC_SPLIT")) : 1;
-  a.head_split = (split_on && allow_head_split && 3 * a.n_tiles <= sms) ? 3 : 1;
+  // small batches: three CTAs per tile, one head each
+  a.head_split = (allow_head_split && 3 * a.n_tiles <= sms) ? 3 : 1;
   static const int tl = getenv("HMZ_X3_TIMELINE") ? atoi(getenv("HMZ_X3_TIMELINE")) : 0;
   a.timeline = tl;
   const unsigned grid = a.head_split == 3 ? 3u * (unsigned)a.n_tiles : (unsigned)(a.n_tiles < sms ? a.n_tiles : sms);

@@ -26,10 +26,7 @@
 
 namespace hmz {
 
-#ifndef HMZ_PERSIST_THREADS
-#define HMZ_PERSIST_THREADS 768
-#endif
-constexpr int kPersistThreads = HMZ_PERSIST_THREADS;  // 24 warps; at this block size ptxas may use 80 registers per thread
+constexpr int kPersistThreads = 768;  // 24 warps; at this block size ptxas may use 80 registers per thread
 constexpr int kPersistWarps = kPersistThreads / 32;
 
 struct PersistArgs {
@@ -58,11 +55,7 @@ __device__ __forceinline__ void tree_role(const PersistArgs& a, uint8_t* smem_ra
     reinterpret_cast<double*>(s_cnt)[i] = reinterpret_cast<const double*>(a.cnt_table)[i];
   for (int i = threadIdx.x; i < a.table_rows; i += blockDim.x) s_ucb[i] = a.ucb_table[i];
   __syncthreads();
-#ifdef HMZ_PERSIST_GLOBAL_TABLES  // A/B switch: read the tables from global memory through L1 instead
-  const SmemTables tb{a.cnt_table, a.ucb_table, a.table_rows};
-#else
   const SmemTables tb{s_cnt, s_ucb, a.table_rows};
-#endif
   const int lane = threadIdx.x & 31, half = lane & 1;
   const tc::v4::PersistCtl& pc = a.ctl;
   const bool stats = tc::v4::kPersistStats && pc.stats != nullptr && lane == 0;
@@ -137,10 +130,7 @@ __global__ void __launch_bounds__(kPersistThreads, 1) search_persistent(const __
 //                 the tree launch for `sim` poll it before their backup (acquire)
 // A network CTA needs a whole SM, so under the launch-per-simulation schedule the two kernel families take turns on the
 // machine (DESIGN.md §4); here the network CTAs keep their SMs and the tree blocks never wait for an SM to drain.
-static int server_mlp_ctas() {
-  static const int v = getenv("HMZ_SERVER_MLP") ? atoi(getenv("HMZ_SERVER_MLP")) : 72;
-  return v;
-}
+constexpr int kServerMlpCtas = 72;  // resident network CTAs (fewer when the device has fewer than 80 SMs or pairs)
 
 // Dynamic shared memory of search_persistent, opted in once per host thread and device.
 static int persist_prepare(int* smem_out) {
@@ -212,7 +202,7 @@ int server_mlp_launch(const hmz_search_t* s, const void* weights, int n_simulati
   PersistArgs a{};
   a.n_pairs = (int)tile_pairs(s->n_searches);
   a.n_sims = n_simulations;
-  int n_mlp = server_mlp_ctas();
+  int n_mlp = kServerMlpCtas;
   if (n_mlp > sm_count() - 8) n_mlp = sm_count() - 8;
   if (n_mlp > a.n_pairs) n_mlp = a.n_pairs;
   if (n_mlp < 1) return fail(HMZ_ERR_UNSUPPORTED, "server schedule needs at least 9 SMs");
@@ -245,20 +235,11 @@ int persist_read_timeline(unsigned long long* host_out) {  // this translation u
 int persist_read_stats(unsigned long long* host_out) {
   return cudaMemcpyFromSymbol(host_out, g_persist_stats, sizeof(unsigned long long) * 16) == cudaSuccess ? HMZ_OK : HMZ_ERR_CUDA;
 }
-static int persist_mlp_override() {
-  static const int v = getenv("HMZ_PERSIST_MLP") ? atoi(getenv("HMZ_PERSIST_MLP")) : 0;
-  return v;
-}
-static int persist_sm_limit() {
-  static const int v = getenv("HMZ_PERSIST_SMS") ? atoi(getenv("HMZ_PERSIST_SMS")) : 0;
-  return v;
-}
 
 // How many CTAs play the MLP role: the MLP side needs ceil(n_pairs / n_mlp) passes of ~8 us per simulation round, the
 // tree side ~14 us per phase for as many slices as its 24 warps per CTA can hold at once; take the split that minimises
 // the longer of the two (ties: fewer MLP CTAs).
 static int choose_n_mlp(int n_pairs, int sms) {
-  if (persist_mlp_override() > 0) return persist_mlp_override() < sms ? (persist_mlp_override() < n_pairs ? persist_mlp_override() : n_pairs) : sms - 1;
   const double t_mlp = 8.0, t_tree = 14.0;
   int best = 1;
   double best_cost = 1e30;
@@ -289,8 +270,7 @@ int persist_launch(const hmz_search_t* s, const void* weights, int n_simulations
                    const CountRow* cnt_table, const TreeScratch& scratch, void* ctl_mem, cudaStream_t stream) {
   int smem = 0;
   if (int rc = persist_prepare(&smem)) return rc;
-  int sms = sm_count();
-  if (persist_sm_limit() > 1 && persist_sm_limit() < sms) sms = persist_sm_limit();
+  const int sms = sm_count();
   PersistArgs a{};
   const int64_t B = s->n_searches;
   a.n_pairs = (int)tile_pairs(B);

@@ -5,8 +5,6 @@
 // hmz_tree.cuh.  These kernels are latency-bound gathers (one 128-byte record per tree level, one
 // 16-byte slot per backup step); there is no contraction here and nothing for tensor cores to do.
 #include <cstdlib>
-#include <cstring>
-#include <vector>
 
 #include "hmz_common.cuh"
 #include "hmz_net_tc.cuh"
@@ -16,10 +14,7 @@ namespace hmz {
 
 // Warps never synchronise with each other, so the block size only sets the granularity at which finished
 // work frees its registers for the next block: a block lives as long as the DEEPEST of its walks.
-#ifndef HMZ_TREE_THREADS
-#define HMZ_TREE_THREADS 128
-#endif
-constexpr int kTreeThreads = HMZ_TREE_THREADS;       // 16 searches per warp
+constexpr int kTreeThreads = 128;                    // 16 searches per warp
 constexpr int kSearchesPerBlock = kTreeThreads / 2;  // one lane pair per search
 constexpr int kLatentWidth = HMZ_LATENT;
 
@@ -80,12 +75,9 @@ __global__ void __launch_bounds__(kTreeThreads) search_select(hmz_search_t s, in
 }
 
 // The fused hot-loop kernel of the launch-per-simulation schedule: tree_phase() (hmz_tree.cuh) for one lane pair per
-// search, launched as a programmatic dependent of the network kernel.
-#ifndef HMZ_TREE_MIN_BLOCKS
-#define HMZ_TREE_MIN_BLOCKS (640 / HMZ_TREE_THREADS)  // 20 warps per SM (96 registers)
-#endif
+// search, launched as a programmatic dependent of the network kernel.  Five blocks per SM: 20 warps at 96 registers.
 template <bool kTL, bool kTrusted>
-__global__ void __launch_bounds__(kTreeThreads, HMZ_TREE_MIN_BLOCKS) search_backup_select(hmz_search_t s, int sim, const double* __restrict__ ucb_table,
+__global__ void __launch_bounds__(kTreeThreads, 5) search_backup_select(hmz_search_t s, int sim, const double* __restrict__ ucb_table,
                                                                      double discount, TreeScratch sc, int do_select) {
   if (threadIdx.x == 0) gantt_mark(sc.gantt, 0);
   tree_phase<kTL, kTrusted, true>(s, sim, ucb_table, discount, sc, do_select, (blockIdx.x * (int64_t)blockDim.x + threadIdx.x) >> 1,
@@ -263,20 +255,17 @@ static int ensure_rcp_table() {
 // kernels the largest L1 split and every alternation between the two kernels re-partitions the SM's L1 / shared
 // memory.  Pinning the tree kernels to an explicit split removes ~1.8 us from every kernel switch (measured:
 // 50.4 -> 46.7 us per simulation with serial launches; any explicit value from 0 to 75 % behaves the same, 100 %
-// starves the tree kernel's L1).  HMZ_TREE_CARVEOUT = percent of shared memory (default 25, -1 = leave unset).
-static int tree_carveout() {
-  static const int pct = getenv("HMZ_TREE_CARVEOUT") ? atoi(getenv("HMZ_TREE_CARVEOUT")) : 25;
-  return pct;
-}
+// starves the tree kernel's L1).
+constexpr int kTreeCarveoutPct = 25;  // percent of the SM's L1 / shared memory given to shared memory
 static int ensure_tree_attrs() {
   static thread_local int done_dev = -1;
   int dev = 0;
   if (cudaGetDevice(&dev) != cudaSuccess) return fail(HMZ_ERR_CUDA, "cudaGetDevice failed (no CUDA device?)");
-  if (done_dev == dev || tree_carveout() < 0) return HMZ_OK;
-  cudaError_t e = cudaFuncSetAttribute(search_backup_select<false, false>, cudaFuncAttributePreferredSharedMemoryCarveout, tree_carveout());
-  if (e == cudaSuccess) e = cudaFuncSetAttribute(search_backup_select<false, true>, cudaFuncAttributePreferredSharedMemoryCarveout, tree_carveout());
-  if (e == cudaSuccess) e = cudaFuncSetAttribute(search_backup_select<true, true>, cudaFuncAttributePreferredSharedMemoryCarveout, tree_carveout());
-  if (e == cudaSuccess) e = cudaFuncSetAttribute(search_select, cudaFuncAttributePreferredSharedMemoryCarveout, tree_carveout());
+  if (done_dev == dev) return HMZ_OK;
+  cudaError_t e = cudaFuncSetAttribute(search_backup_select<false, false>, cudaFuncAttributePreferredSharedMemoryCarveout, kTreeCarveoutPct);
+  if (e == cudaSuccess) e = cudaFuncSetAttribute(search_backup_select<false, true>, cudaFuncAttributePreferredSharedMemoryCarveout, kTreeCarveoutPct);
+  if (e == cudaSuccess) e = cudaFuncSetAttribute(search_backup_select<true, true>, cudaFuncAttributePreferredSharedMemoryCarveout, kTreeCarveoutPct);
+  if (e == cudaSuccess) e = cudaFuncSetAttribute(search_select, cudaFuncAttributePreferredSharedMemoryCarveout, kTreeCarveoutPct);
   if (e != cudaSuccess) return fail(HMZ_ERR_CUDA, "cudaFuncSetAttribute(carveout): %s", cudaGetErrorString(e));
   done_dev = dev;
   return HMZ_OK;
@@ -388,39 +377,12 @@ int hmz_debug_tree_timeline(long long search, unsigned long long* host_out) {
   return HMZ_OK;
 }
 
-// Non-default compile-time tuning switches of this build ("" for a clean build), so that tests and bench lines can
-// tell a tuned library from the shipped one.  None of them changes results.
+// Non-default compile-time switches of this build ("" for a clean build), so that tests and bench lines can tell a
+// tooling or A/B build from the shipped one.  None of them changes results.
 const char* hmz_build_flags(void) {
   return ""
-#if HMZ_TREE_THREADS != 128
-         " HMZ_TREE_THREADS"
-#endif
-#if HMZ_TREE_MIN_BLOCKS != (640 / HMZ_TREE_THREADS)
-         " HMZ_TREE_MIN_BLOCKS"
-#endif
-#if HMZ_PREFETCH_SECTORS != 0
-         " HMZ_PREFETCH_SECTORS"
-#endif
-#if HMZ_L2_HINTS != 0
-         " HMZ_L2_HINTS"
-#endif
-#ifdef HMZ_NO_LATENT_PREFETCH
-         " HMZ_NO_LATENT_PREFETCH"
-#endif
-#ifdef HMZ_TC_MAXNREG
-         " HMZ_TC_MAXNREG"
-#endif
 #ifdef HMZ_PERSIST_STATS
          " HMZ_PERSIST_STATS"
-#endif
-#ifdef HMZ_PERSIST_THREADS
-         " HMZ_PERSIST_THREADS"
-#endif
-#ifdef HMZ_PERSIST_SLEEP_NS_SET
-         " HMZ_PERSIST_SLEEP_NS"
-#endif
-#ifdef HMZ_PERSIST_GLOBAL_TABLES
-         " HMZ_PERSIST_GLOBAL_TABLES"
 #endif
 #ifdef HMZ_VARIANT
          " HMZ_VARIANT"
@@ -649,12 +611,12 @@ static int run_one_sim(const hmz_search_t* s, const SimScratch& sc, const void* 
   }
   if (skip & 2) return HMZ_OK;
   ProfScope prof_scope(HMZ_PROF_EXPAND_BACKUP, stream);
-  const int do_select = (sim + 1 < n_simulations ? 1 : 0) | (pdl_prewait() << 1) | ((pdl_tree_at() & 3) << 2);
+  const int do_select = sim + 1 < n_simulations ? 1 : 0;
   const float *cr = sc.r, *cp = sc.p, *cv = sc.v;
   TreeScratch ts{sc.lp, sc.la, sc.depth, sc.path, sc.wild, cr, cp, cv,
                  s->capture ? s->capture + ((size_t)sim * (size_t)capture_stride + (size_t)capture_lo) * 8 : nullptr,
                  gantt_next(1, gantt_context_tag()), sets.budget};
-  cudaError_t e = launch_pdl(2, g_tree_tl_search >= 0 ? search_backup_select<true, true> : search_backup_select<false, true>,
+  cudaError_t e = launch_pdl(g_tree_tl_search >= 0 ? search_backup_select<true, true> : search_backup_select<false, true>,
                              dim3(search_grid(B)), dim3(kTreeThreads), 0, st, *s, sim, ucb_table, discount, ts, do_select);
   if (e != cudaSuccess) return fail(HMZ_ERR_CUDA, "search_backup_select launch: %s", cudaGetErrorString(e));
   return check_launch("search_backup_select");
@@ -692,19 +654,19 @@ static int search_run_server(const hmz_search_t* s, const void* weights, int n_s
   int rc = server_mlp_launch(s, weights, n_simulations, whole, sc0.ctl, (int)(per / 256), fork[groups], &sctl);
   // A tree launch that is resident before its pairs' network outputs exist holds its SM slots spinning: the group's
   // stream waits (cuStreamWaitValue32, resolved through the runtime so that libcuda is not a link dependency) until the
-  // network CTAs have finished every pair of the group for the previous simulation.  HMZ_SERVER_GATE=0: spin only.
+  // network CTAs have finished every pair of the group for the previous simulation.  Without that entry point the tree
+  // warps only spin.
   typedef int (*WaitValue32)(cudaStream_t, unsigned long long, unsigned int, unsigned int);
   static WaitValue32 wait_value = nullptr;
-  static int gate = -1;
-  if (gate < 0) {
-    gate = getenv("HMZ_SERVER_GATE") ? atoi(getenv("HMZ_SERVER_GATE")) : 1;
+  static bool resolved = false;
+  if (!resolved) {
     void* fn = nullptr;
     cudaDriverEntryPointQueryResult qr;
-    if (gate && (cudaGetDriverEntryPoint("cuStreamWaitValue32", &fn, cudaEnableDefault, &qr) != cudaSuccess || qr != cudaDriverEntryPointSuccess || !fn)) {
-      gate = 0;
+    if (cudaGetDriverEntryPoint("cuStreamWaitValue32", &fn, cudaEnableDefault, &qr) == cudaSuccess && qr == cudaDriverEntryPointSuccess)
+      wait_value = (WaitValue32)fn;
+    else
       cudaGetLastError();
-    }
-    wait_value = (WaitValue32)fn;
+    resolved = true;
   }
   hmz_search_t sub[16];
   SimScratch sc[16];
@@ -721,7 +683,7 @@ static int search_run_server(const hmz_search_t* s, const void* weights, int n_s
       TreeScratch ts{sc[g].lp, sc[g].la, sc[g].depth, sc[g].path, sc[g].wild, sc[g].r, sc[g].p, sc[g].v,
                      (s->capture && k > 0) ? s->capture + ((size_t)(k - 1) * (size_t)B + (size_t)(g * per)) * 8 : nullptr,
                      gantt_next(1, gantt_context_tag())};
-      if (gate && k > 0) {
+      if (wait_value && k > 0) {
         const unsigned int pairs_g = (unsigned int)((sub[g].n_searches + 255) / 256);
         if (wait_value(fork[g], (unsigned long long)(uintptr_t)(sctl.group_done + (size_t)g * 8), pairs_g * (unsigned int)k, 0u /* >= */) != 0)
           rc = fail(HMZ_ERR_CUDA, "cuStreamWaitValue32 failed");
@@ -781,8 +743,8 @@ static int search_run_groups(const hmz_search_t* s, const hmz_multi_t* m, const 
   return rc;
 }
 
-static int search_run_direct(const hmz_search_t* s, const void* weights, int mode, int n_simulations, const double* ucb_table,
-                             double discount, void* stream) {
+int hmz_search_run(const hmz_search_t* s, const void* weights, int mode, int n_simulations, const double* ucb_table,
+                   double discount, void* stream) {
   if (int rc = check_search(s, "hmz_search_run")) return rc;
   if (s->n_searches == 0 || n_simulations == 0) return HMZ_OK;
   if (!weights || !ucb_table || !s->workspace || !s->latents || n_simulations < 0 ||
@@ -808,96 +770,6 @@ static int search_run_direct(const hmz_search_t* s, const void* weights, int mod
   if (s->schedule < 0 || s->schedule > 16)
     return fail(HMZ_ERR_INVALID, "hmz_search_run: schedule %d is neither a group count in [0, 16] nor HMZ_SCHEDULE_PERSISTENT", s->schedule);
   return search_run_groups(s, nullptr, weights, mode, n_simulations, ucb_table, discount, stream);
-}
-
-// ---- optional CUDA-graph replay of the whole search (HMZ_GRAPH=1) -------------------------------------------
-// The launch sequence of one hmz_search_run call (groups x simulations x 2 kernels, programmatic edges
-// included) is captured once per distinct argument set on an internal stream and replayed; the caller's stream
-// is joined around the replay with events.  Tooling / tuning switch: off by default.
-namespace {
-struct GraphEntry {
-  unsigned long long key[8];
-  cudaGraphExec_t exec;
-  long long kernels;
-};
-struct GraphCache {
-  int dev = -1;
-  cudaStream_t stream = nullptr;
-  cudaEvent_t fork = nullptr, join = nullptr;
-  std::vector<GraphEntry> entries;
-};
-int graph_mode() {
-  static const int on = getenv("HMZ_GRAPH") ? atoi(getenv("HMZ_GRAPH")) : 0;
-  return on;
-}
-}  // namespace
-
-static int search_run_graph(const hmz_search_t* s, const void* weights, int mode, int n_simulations, const double* ucb_table,
-                            double discount, void* stream) {
-  static thread_local GraphCache gc;
-  int dev = 0;
-  if (cudaGetDevice(&dev) != cudaSuccess) return fail(HMZ_ERR_CUDA, "cudaGetDevice failed");
-  if (gc.dev != dev) {
-    gc = GraphCache();
-    gc.dev = dev;
-    if (cudaStreamCreateWithFlags(&gc.stream, cudaStreamNonBlocking) != cudaSuccess ||
-        cudaEventCreateWithFlags(&gc.fork, cudaEventDisableTiming) != cudaSuccess ||
-        cudaEventCreateWithFlags(&gc.join, cudaEventDisableTiming) != cudaSuccess)
-      return fail(HMZ_ERR_CUDA, "graph stream / event creation failed");
-  }
-  unsigned long long dbits;
-  memcpy(&dbits, &discount, 8);
-  const unsigned long long key[8] = {(unsigned long long)(uintptr_t)s->nodes, (unsigned long long)(uintptr_t)s->latents,
-                                     (unsigned long long)(uintptr_t)s->workspace, (unsigned long long)(uintptr_t)weights,
-                                     (unsigned long long)s->n_searches | ((unsigned long long)n_simulations << 40),
-                                     (unsigned long long)(uintptr_t)ucb_table, dbits,
-                                     (unsigned long long)s->n_records | ((unsigned long long)mode << 32) |
-                                         ((unsigned long long)s->root_prior_is_f64 << 40) | ((unsigned long long)s->latent_dtype << 44) |
-                                         ((unsigned long long)s->schedule << 48) ^ (unsigned long long)(uintptr_t)s->capture};
-  GraphEntry* hit = nullptr;
-  for (auto& e : gc.entries)
-    if (memcmp(e.key, key, sizeof(key)) == 0) hit = &e;
-  if (!hit) {
-    if (int rc = check_search(s, "hmz_search_run")) return rc;  // one-time uploads happen outside the capture
-    const long long before = g_launches.load();
-    if (cudaStreamBeginCapture(gc.stream, cudaStreamCaptureModeThreadLocal) != cudaSuccess)
-      return fail(HMZ_ERR_CUDA, "cudaStreamBeginCapture failed: %s", cudaGetErrorString(cudaGetLastError()));
-    const int rc = search_run_direct(s, weights, mode, n_simulations, ucb_table, discount, (void*)gc.stream);
-    cudaGraph_t graph = nullptr;
-    const cudaError_t e = cudaStreamEndCapture(gc.stream, &graph);
-    if (rc != HMZ_OK) {
-      if (graph) cudaGraphDestroy(graph);
-      return rc;
-    }
-    if (e != cudaSuccess || !graph) return fail(HMZ_ERR_CUDA, "cudaStreamEndCapture failed: %s", cudaGetErrorString(e));
-    GraphEntry ne;
-    memcpy(ne.key, key, sizeof(key));
-    ne.kernels = g_launches.load() - before;
-    g_launches.store(before);  // capturing launched nothing
-    const cudaError_t ei = cudaGraphInstantiate(&ne.exec, graph, 0);
-    cudaGraphDestroy(graph);
-    if (ei != cudaSuccess) return fail(HMZ_ERR_CUDA, "cudaGraphInstantiate failed: %s", cudaGetErrorString(ei));
-    if (gc.entries.size() >= 8) {  // tiny cache: drop the oldest
-      cudaGraphExecDestroy(gc.entries.front().exec);
-      gc.entries.erase(gc.entries.begin());
-    }
-    gc.entries.push_back(ne);
-    hit = &gc.entries.back();
-  }
-  cudaStream_t caller = (cudaStream_t)stream;
-  if (cudaEventRecord(gc.fork, caller) != cudaSuccess || cudaStreamWaitEvent(gc.stream, gc.fork, 0) != cudaSuccess ||
-      cudaGraphLaunch(hit->exec, gc.stream) != cudaSuccess || cudaEventRecord(gc.join, gc.stream) != cudaSuccess ||
-      cudaStreamWaitEvent(caller, gc.join, 0) != cudaSuccess)
-    return fail(HMZ_ERR_CUDA, "graph replay failed: %s", cudaGetErrorString(cudaGetLastError()));
-  g_launches.fetch_add(hit->kernels);
-  return HMZ_OK;
-}
-
-int hmz_search_run(const hmz_search_t* s, const void* weights, int mode, int n_simulations, const double* ucb_table,
-                   double discount, void* stream) {
-  if (graph_mode() && s && s->n_searches > 0 && n_simulations > 0 && g_prof_on.load() == 0 && g_tree_tl_search < 0)
-    return search_run_graph(s, weights, mode, n_simulations, ucb_table, discount, stream);
-  return search_run_direct(s, weights, mode, n_simulations, ucb_table, discount, stream);
 }
 
 int hmz_search_run_multi(const hmz_search_t* s, const hmz_multi_t* m, const void* weights, int mode, const double* ucb_table,

@@ -73,22 +73,6 @@ __device__ __forceinline__ void ld256(const void* p, uint4& lo, uint4& hi) {
                : "l"(p)
                : "memory");
 }
-#ifndef HMZ_L2_HINTS
-#define HMZ_L2_HINTS 0
-#endif
-// the same with L2 eviction priorities (the .L2:: qualifiers exist for the 256-bit forms only): root records are
-// re-read by every simulation (evict_last), freshly expanded records are not needed soon (evict_first)
-__device__ __forceinline__ void ld256_keep(const void* p, uint4& lo, uint4& hi) {
-  asm volatile("ld.global.L2::evict_last.v8.u32 {%0, %1, %2, %3, %4, %5, %6, %7}, [%8];"
-               : "=r"(lo.x), "=r"(lo.y), "=r"(lo.z), "=r"(lo.w), "=r"(hi.x), "=r"(hi.y), "=r"(hi.z), "=r"(hi.w)
-               : "l"(p)
-               : "memory");
-}
-__device__ __forceinline__ void st256_stream(void* p, const uint4& lo, const uint4& hi) {
-  asm volatile("st.global.L2::evict_first.v8.u32 [%0], {%1, %2, %3, %4, %5, %6, %7, %8};" ::"l"(p), "r"(lo.x), "r"(lo.y), "r"(lo.z),
-               "r"(lo.w), "r"(hi.x), "r"(hi.y), "r"(hi.z), "r"(hi.w)
-               : "memory");
-}
 __device__ __forceinline__ void st256(void* p, const uint4& lo, const uint4& hi) {
   asm volatile("st.global.v8.u32 [%0], {%1, %2, %3, %4, %5, %6, %7, %8};" ::"l"(p), "r"(lo.x), "r"(lo.y), "r"(lo.z), "r"(lo.w),
                "r"(hi.x), "r"(hi.y), "r"(hi.z), "r"(hi.w)
@@ -105,13 +89,8 @@ __device__ __forceinline__ void write_fresh_half_vals(hmz_node_t* rec, int half,
                                                       int parent_action) {
   uint4* dst = reinterpret_cast<uint4*>(&rec->h[half]);
   const uint4 empty = make_uint4(0u, 0u, 0u, 0xFFFF0000u);  // W = 0, rwd = 0, N = 0, child = HMZ_NO_CHILD
-#if HMZ_L2_HINTS & 2
-#define HMZ_ST_FRESH st256_stream
-#else
-#define HMZ_ST_FRESH st256
-#endif
-  HMZ_ST_FRESH(dst, empty, empty);
-  HMZ_ST_FRESH(dst + 2, empty,
+  st256(dst, empty, empty);
+  st256(dst + 2, empty,
         make_uint4(__float_as_uint(pr0), __float_as_uint(pr1), __float_as_uint(pr2),
                    half == 0 ? ((uint32_t)parent | ((uint32_t)parent_action << 16)) : 0u));
 }
@@ -221,16 +200,6 @@ __device__ __forceinline__ void minmax_update(double x, double& mn, double& mx) 
   if (x < mn) mn = x;
 }
 
-#ifndef HMZ_PREFETCH_SECTORS
-#define HMZ_PREFETCH_SECTORS 0
-#endif
-// Request a 128-byte node record into L1 without a destination register.
-__device__ __forceinline__ void prefetch_record(const void* rec) {
-#pragma unroll
-  for (int k = 0; k < HMZ_PREFETCH_SECTORS; ++k)
-    asm volatile("prefetch.global.L1 [%0];" ::"l"(reinterpret_cast<const char*>(rec) + 32 * k * (4 / HMZ_PREFETCH_SECTORS)));
-}
-
 // Reference-order evaluation of one child (the slow, always-exact form): used when an operand falls
 // outside the range the straight-line form below is proven for.
 static __device__ __noinline__ float child_score_exact(double W, float rwd, int n, float prior, double prior64, bool use64, double tn,
@@ -288,16 +257,8 @@ __device__ __forceinline__ Leaf select_leaf(const hmz_node_t* nodes, const doubl
     double tn = 0.0;
     if (active) {
       const uint4* hp = reinterpret_cast<const uint4*>(&nodes[e].h[half]);
-#if HMZ_L2_HINTS & 1
-      if (e == 0) {
-        ld256_keep(hp, q0, q1);
-        ld256_keep(hp + 2, q2, q3);
-      } else
-#endif
-      {
-        ld256(hp, q0, q1);
-        ld256(hp + 2, q2, q3);
-      }
+      ld256(hp, q0, q1);
+      ld256(hp + 2, q2, q3);
       if (depth == 0) tree_mark<kTL>(41, tl_on);
       tn = tb.ucb(ucb_table, n_parent);
       if (use64) {  // only the (noised) root has float64 priors; requested together with the record
@@ -307,11 +268,6 @@ __device__ __forceinline__ Leaf select_leaf(const hmz_node_t* nodes, const doubl
     }
     if (depth < 8) tree_mark<kTL>(8 + 2 * depth, tl_on, q0.w ^ q1.w ^ q2.w ^ q3.w);
     Slot c[3] = {Slot::unpack(q0), Slot::unpack(q1), Slot::unpack(q2)};
-#if HMZ_PREFETCH_SECTORS > 0
-#pragma unroll
-    for (int j = 0; j < 3; ++j)
-      if (active && c[j].child != (int)HMZ_NO_CHILD) prefetch_record(&nodes[c[j].child]);
-#endif
     const float prior[3] = {__uint_as_float(q3.x), __uint_as_float(q3.y), __uint_as_float(q3.z)};
     double y[3], yw[3], dn[3], dn1[3];
 #pragma unroll
@@ -532,11 +488,12 @@ struct ServerCtl {
 // usually shares its prefix.  With path elements (slot + entry per level, recorded by the previous walk) the backup needs
 // one round trip for its inputs; without them (split-phase API) it walks the parent links.
 //   b_raw, half   the search this lane pair owns (b_raw >= n_searches: masked, but the lane stays for the warp-uniform walk)
-//   do_select     bit 0: select simulation sim + 1 afterwards; bits 1-3: programmatic-launch switches (kPdl only);
-//                 bit 4: no backup (with sim = -1: the first selection of a search)
+//   do_select     bit 0: select simulation sim + 1 afterwards; bit 4: no backup (with sim = -1: the first selection
+//                 of a search)
 //   kTrusted      `wild_flags[search]` is the sticky "a backup wrote an untame W or Q" flag of is_tame(); the walk then
 //                 skips its per-operand range tests
-//   kPdl          stand-alone kernel launched as a programmatic dependent of the network kernel
+//   kPdl          stand-alone kernel launched as a programmatic dependent of the network kernel: it signals its own
+//                 dependents at entry and waits for the network kernel after loading what the previous tree kernel wrote
 // ALL 32 lanes of the warp must call it.
 template <bool kTL, bool kTrusted, bool kPdl, class TB>
 __device__ __forceinline__ void tree_phase(const hmz_search_t& s, int sim, const double* __restrict__ ucb_table, double discount,
@@ -550,9 +507,7 @@ __device__ __forceinline__ void tree_phase(const hmz_search_t& s, int sim, const
   const float* p = sc.p;
   const float* v = sc.v;
   float* capture = sc.capture;
-  const int signal_at = (do_select >> 2) & 3;  // HMZ_PDL_TREE_AT
-  if (kPdl && signal_at == 0) pdl_launch_dependents();
-  if (kPdl && !(do_select & 2)) pdl_wait();  // HMZ_PDL bit 2 off: nothing is read before the wait
+  if (kPdl) pdl_launch_dependents();
   const bool valid = b_raw < s.n_searches;  // out-of-range pairs stay for the warp-uniform walk, masked
   const int64_t b = valid ? b_raw : s.n_searches - 1;
   const bool tl = kTL && valid && b == (g_tree_timeline_search & 0xFFFFFFFFll) && sim == (int)(g_tree_timeline_search >> 32) && half == 0;
@@ -631,7 +586,6 @@ __device__ __forceinline__ void tree_phase(const hmz_search_t& s, int sim, const
       tree_mark<kTL>(3, tl, (uint32_t)__double2loint(mn));
     }
   }
-  if (kPdl && signal_at == 1) pdl_launch_dependents();
   if (!(do_select & 1)) return;
   // lane 0's slot stores must be visible to its partner's loads in the walk below (a shuffle orders nothing in memory)
   __syncwarp();
@@ -643,12 +597,10 @@ __device__ __forceinline__ void tree_phase(const hmz_search_t& s, int sim, const
   const double* rp = s.root_prior_is_f64 ? s.root_prior + b * 6 : nullptr;
   const bool sel = valid && sim + 1 < budget;  // (a search past its budget stays in the warp-uniform walk, masked)
   const Leaf leaf = select_leaf<kTL, kTrusted, TB>(nodes, rp, mn, mx, sim + 1, ucb_table, discount, half, nullptr, 0, path, tl, sel, wild, tb);
-  if (kPdl && signal_at == 2) pdl_launch_dependents();
   if (half == 0 && sel) {
     leaf_parent[b] = (uint16_t)leaf.parent;
     leaf_action[b] = (uint8_t)leaf.action;
     leaf_depth[b] = (uint16_t)leaf.depth;
-#ifndef HMZ_NO_LATENT_PREFETCH
     // The network kernel that follows gathers the parent's latent row (written many simulations ago, long gone
     // from L2): ask for it now, a whole kernel launch ahead of its use.
     if (s.latents != nullptr) {
@@ -657,7 +609,6 @@ __device__ __forceinline__ void tree_phase(const hmz_search_t& s, int sim, const
       asm volatile("prefetch.global.L2 [%0];" ::"l"(row));
       if (row_bytes == 256) asm volatile("prefetch.global.L2 [%0];" ::"l"(row + 128));
     }
-#endif
     if (tl) {
       g_tree_timeline[4] = (unsigned long long)leaf.depth;
       tree_mark<kTL>(5, tl);

@@ -2,7 +2,6 @@
 # One gpurun call = one round of GPU evidence.  Usage (from the repo root, under gpurun):
 #   bash tools/gpu_round.sh tests          GPU test-suite + a short default bench line
 #   bash tools/gpu_round.sh bench          default bench line only (20 steps)
-#   bash tools/gpu_round.sh envsweep       env kernels over HMZ_ENV_UNROLL x HMZ_ENV_CTAS
 #   bash tools/gpu_round.sh memcheck       compute-sanitizer --tool memcheck over smoke()
 #   bash tools/gpu_round.sh microbench     TMEM / tcgen05.mma micro-benchmarks, kernel families alone, clock64 timelines
 #   bash tools/gpu_round.sh x3             the fast parity mode's kernel: probe, timeline, bench line, ncu --set full
@@ -33,9 +32,6 @@ for stage in "$@"; do
       ;;
     persistsweep)
       : > gpurun_out/persist_sweep.txt
-      for m in ${MLP_LIST:-40 48 56 64 72 80 96}; do
-        HMZ_PERSIST_MLP=$m MOVES=8 timeout 120 python tools/persist_probe.py >> gpurun_out/persist_sweep.txt 2>&1
-      done
       HMZ_LIB_PATH=muzero-hanoi_b200/variants/libhmz_stats.so HMZ_PERSIST_STATS=1 MOVES=4 timeout 120 python tools/persist_probe.py >> gpurun_out/persist_sweep.txt 2>&1
       for b in 8192 16384 32768; do
         B=$b SCHEDULES=64,0,1 MOVES=8 timeout 120 python tools/persist_probe.py >> gpurun_out/persist_sweep.txt 2>&1
@@ -61,14 +57,6 @@ for stage in "$@"; do
     reference)
       timeout 600 python bench.py --impl reference --steps 20 --warmup 3 > gpurun_out/bench_reference.json 2> gpurun_out/bench_reference.log
       echo "reference rc=$?"; head -c 400 gpurun_out/bench_reference.json
-      ;;
-    envsweep)
-      : > gpurun_out/env_sweep.txt
-      for u in 1 2 4; do for c in 3 4 8; do
-        echo "HMZ_ENV_UNROLL=$u HMZ_ENV_CTAS=$c" >> gpurun_out/env_sweep.txt
-        HMZ_ENV_UNROLL=$u HMZ_ENV_CTAS=$c timeout 120 python tools/env_probe.py >> gpurun_out/env_sweep.txt 2>&1
-      done; done
-      cat gpurun_out/env_sweep.txt
       ;;
     memcheck)
       timeout 900 compute-sanitizer --tool memcheck --error-exitcode 7 python -c "import __graft_entry__ as g; g.smoke()" > gpurun_out/memcheck_smoke.log 2>&1
@@ -112,7 +100,6 @@ for stage in "$@"; do
       SCHEDULE=128 timeout 200 python tools/gantt.py > gpurun_out/gantt_server.txt 2>&1
       SERVER=128 timeout 200 python tools/tc_timeline.py > gpurun_out/timeline_net_tc_server.txt 2>&1
       SCHEDULES=0,64,128,136 MOVES=10 timeout 200 python tools/persist_probe.py > gpurun_out/schedules.txt 2>&1
-      for m in 64 68 72 76 80; do HMZ_SERVER_MLP=$m SCHEDULES=128 MOVES=8 timeout 200 python tools/persist_probe.py 2>&1 | sed "s/^/HMZ_SERVER_MLP=$m /" >> gpurun_out/schedules.txt; done
       timeout 600 python bench.py --steps 10 --warmup 3 --no-cpu-baseline --no-env --no-configs --schedule server > gpurun_out/bench_server.json 2> gpurun_out/bench_server.log
       TORCH_INIT=1 SEARCHES=17,30000,5000 timeout 120 python tools/tree_timeline.py > gpurun_out/timeline_tree.txt 2>&1
       ;;

@@ -30,7 +30,7 @@ for sched in [int(x) for x in os.environ.get("SCHEDULES", "64").split(",")]:
     e1.record()
     torch.cuda.synchronize()
     ms = e0.elapsed_time(e1) / moves
-    line = f"B={B} S={S} mode={MODE} schedule={sched} HMZ_PERSIST_MLP={os.environ.get('HMZ_PERSIST_MLP', '-')}: {ms:.3f} ms/move, {B * S / ms / 1e6:.1f} M sims/s, {ms / S * 1e3:.2f} us/round"
+    line = f"B={B} S={S} mode={MODE} schedule={sched}: {ms:.3f} ms/move, {B * S / ms / 1e6:.1f} M sims/s, {ms / S * 1e3:.2f} us/round"
     if sched == 64 and os.environ.get("HMZ_PERSIST_STATS"):
         buf = (C.c_ulonglong * 16)()
         _lib.check(lib.hmz_debug_persist_stats(buf))

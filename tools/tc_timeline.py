@@ -32,40 +32,27 @@ torch.cuda.synchronize()
 buf = (C.c_ulonglong * 96)()
 _lib.check(READ(buf))
 marks = np.array(list(buf), dtype=np.int64)
-if os.environ.get("HMZ_TC_V3"):
-    names = {0: "ctl start", 1: "ctl gather seen", 2: "ctl Wg1 landed", 3: "ctl L1 issued", 4: "ctl L1 complete", 5: "ctl Wg2 landed",
-             6: "ctl g-hid h0 written", 7: "ctl g-hid h1 written", 8: "ctl L2 complete", 9: "ctl latent tiles written", 32: "hid gather done", 63: "end",
-             48: "small saw L2", 49: "hid latent done (arrived)", 56: "hid latent: tmem loaded", 57: "hid latent: minmax exchanged", 58: "hid latent: stores issued"}
-    for hd, nm in enumerate("rpv"):
-        for j, what in enumerate(["W1 landed", "first MMA complete", "W2 landed", "hid h0 written", "hid h1 written", "second MMA complete"]):
-            names[10 + hd * 6 + j] = f"ctl {nm}: {what}"
-        names[50 + hd * 2] = f"small {nm}: saw second layer"
-        names[51 + hd * 2] = f"small {nm}: output done"
-    for ly, nm in enumerate("grpv"):
-        names[33 + ly * 3] = f"hid {nm}: saw first layer"
-        names[34 + ly * 3] = f"hid {nm}: epilogue done"
-        names[35 + ly * 3] = f"hid {nm}: saw second layer"
-else:  # v4: two tiles per CTA
-    names = {60: "CTA: kernel entry", 61: "CTA: barriers + TMEM ready", 62: "CTA: past the PDL wait", 63: "CTA: all warps done",
-             64: "T0 hid: pass start", 66: "out: pass published"}
-    for i, net in enumerate("grvp"):  # network order of a pass: dynamics, reward, value, policy
-        for t in range(2):
-            names[i * 4 + t] = f"T{t} mma {net}: L1 inputs ready"
-            names[i * 4 + 2 + t] = f"T{t} mma {net}: L2 inputs ready (A1 written)"
-            names[16 + i * 2 + t] = f"T{t} mma {net}: L1 issue point reached"
+# two tiles per CTA
+names = {60: "CTA: kernel entry", 61: "CTA: barriers + TMEM ready", 62: "CTA: past the PDL wait", 63: "CTA: all warps done",
+         64: "T0 hid: pass start", 66: "out: pass published"}
+for i, net in enumerate("grvp"):  # network order of a pass: dynamics, reward, value, policy
     for t in range(2):
-        names[86 + t * 8] = f"T{t} hid: raw latent published"
-        names[44 + t * 8] = f"T{t} hid: saw dynamics L2 complete"
-        names[40 + t * 8] = f"T{t} hid: minmax exchanged"
-        names[41 + t * 8] = f"T{t} hid: hn tile written"
-        names[42 + t * 8] = f"T{t} hid: hn published"
-        names[43 + t * 8] = f"T{t} hid: copy-out barrier passed"
-        names[80 + t * 8] = f"T{t} hid: gather done"
-        for ly, nm in enumerate("grvp"):
-            names[81 + t * 8 + ly] = f"T{t} hid {nm}: A1 half 0 written"
-        names[85 + t * 8] = f"T{t} hid: latent done"
-        for hd, nm in enumerate("rvp"):
-            names[70 + hd * 2 + t] = f"T{t} out {nm}: done"
+        names[i * 4 + t] = f"T{t} mma {net}: L1 inputs ready"
+        names[i * 4 + 2 + t] = f"T{t} mma {net}: L2 inputs ready (A1 written)"
+        names[16 + i * 2 + t] = f"T{t} mma {net}: L1 issue point reached"
+for t in range(2):
+    names[86 + t * 8] = f"T{t} hid: raw latent published"
+    names[44 + t * 8] = f"T{t} hid: saw dynamics L2 complete"
+    names[40 + t * 8] = f"T{t} hid: minmax exchanged"
+    names[41 + t * 8] = f"T{t} hid: hn tile written"
+    names[42 + t * 8] = f"T{t} hid: hn published"
+    names[43 + t * 8] = f"T{t} hid: copy-out barrier passed"
+    names[80 + t * 8] = f"T{t} hid: gather done"
+    for ly, nm in enumerate("grvp"):
+        names[81 + t * 8 + ly] = f"T{t} hid {nm}: A1 half 0 written"
+    names[85 + t * 8] = f"T{t} hid: latent done"
+    for hd, nm in enumerate("rvp"):
+        names[70 + hd * 2 + t] = f"T{t} out {nm}: done"
 if os.environ.get("SERVER"):
     for k in (60, 61, 62, 63):
         names.pop(k, None)
