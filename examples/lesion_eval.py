@@ -1,8 +1,9 @@
-"""The reference's lesion experiment (acting_experiments/acting_ablations.py) on a network trained a moment ago:
-train 3-disk Hanoi on the device, then measure the planning error (moves beyond the optimum) from random starts for
-several MCTS budgets, intact and with the policy / value / reward heads re-initialised.
+"""The reference's lesion experiment (acting_experiments/acting_ablations.py) on a network trained a moment ago (or
+loaded with --checkpoint): train 3-disk Hanoi on the device, then measure the planning error (moves beyond the optimum)
+from random starts for several MCTS budgets, intact and with the policy / value / reward heads re-initialised.
 
     python examples/lesion_eval.py [--loops 300] [--episodes 2048]
+    python examples/lesion_eval.py --checkpoint muzero_model.pt      # a trained network instead of training one
 """
 import argparse
 import copy
@@ -15,23 +16,37 @@ import torch
 
 from muzero_hanoi_b200 import acting
 from muzero_hanoi_b200.engine import PackedWeights
+from muzero_hanoi_b200.learner import split_flat
 from muzero_hanoi_b200.networks import MuZeroNet
-from muzero_hanoi_b200.trainer import BatchedMuzero
+from muzero_hanoi_b200.trainer import BatchedMuzero, check_checkpoint
 
 
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--loops", type=int, default=300)
     ap.add_argument("--episodes", type=int, default=2048)
+    ap.add_argument("--checkpoint", metavar="PATH", help="evaluate this network instead of training one: the reference's "
+                    "muzero_model.pt (BatchedMuzero.export_reference) or a BatchedMuzero.save file")
     args = ap.parse_args()
     torch.manual_seed(1)
     np.random.seed(1)
     N = 3
     net = MuZeroNet(3 * N, 6, 0.002, "cpu", TD_return=True)
-    mz = BatchedMuzero(net.state_dict(), N, 200, 512, n_update_x_loop=8, seed=1)
-    hist = mz.training_loop(args.loops, min_replay_size=5000)
-    print("trained: mean episode length of the last 20 loops %.1f" % np.mean([h[1] for h in hist[-20:]]))
-    net.load_state_dict({k: v.cpu() for k, v in mz.learner.state_dict().items()})
+    if args.checkpoint:
+        ck = torch.load(args.checkpoint, map_location="cpu")
+        if "Muzero_net" in ck:  # the reference's file, loaded as the lesion scripts load it (acting_ablations.py:350-360)
+            net.load_state_dict(ck["Muzero_net"])
+        else:
+            check_checkpoint(ck)
+            if ck["config"]["N"] != N:
+                raise ValueError(f"{args.checkpoint}: a network of N={ck['config']['N']}, this experiment is N={N}")
+            net.load_state_dict(split_flat(ck["learner"]["params"], N))
+        print("loaded %s" % args.checkpoint)
+    else:
+        mz = BatchedMuzero(net.state_dict(), N, 200, 512, n_update_x_loop=8, seed=1)
+        hist = mz.training_loop(args.loops, min_replay_size=5000)
+        print("trained: mean episode length of the last 20 loops %.1f" % np.mean([h[1] for h in hist[-20:]]))
+        net.load_state_dict({k: v.cpu() for k, v in mz.learner.state_dict().items()})
     budgets = [5, 10, 30, 80]
     settings = [("intact", (False, False, False)), ("policy lesion", (True, False, False)), ("value lesion", (False, True, False)),
                 ("reward lesion", (False, False, True)), ("policy + value lesion", (True, True, False))]
