@@ -353,7 +353,9 @@ int hmz_debug_div_check(uint64_t n_samples, uint64_t seed, unsigned long long* c
  * the global id of its first game).  Parity mode passes the reference's own draws to hmz_search_begin_p0 /
  * hmz_search_root_policy instead.
  */
-/* np.random.dirichlet(alpha * ones(6)) (MCTS/mcts.py:148-149): out float64 [n][6]. */
+/* np.random.dirichlet(alpha * ones(6)) (MCTS/mcts.py:148-149): out float64 [n][6].  counter < 2^56
+ * (HMZ_ERR_INVALID otherwise): the gamma streams keep the draw's block number in the low 8 bits of Philox counter
+ * word 3, so counter bits 56-63 have no room there. */
 int hmz_rng_dirichlet(double* out, int64_t n, double alpha, uint64_t seed, uint64_t counter, uint64_t item_offset, void* stream);
 /* One uniform double in [0, 1) per item (the draw of np.random.choice, MCTS/mcts.py:120). */
 int hmz_rng_uniform(double* out, int64_t n, uint64_t seed, uint64_t counter, uint64_t item_offset, void* stream);
@@ -383,7 +385,8 @@ typedef struct hmz_move_record {
  * into the root prior (hmz_search_begin_p0) and the sampling uniform, keyed by (seed, game_offset + game, move_index);
  * hmz_search_run; ONE kernel for the root policy + sampled action (hmz_search_root_policy), the move record, the
  * episode store (hmz_episode_record / _close) and hmz_env_step with auto-reset — enqueued on `stream` without any host
- * synchronisation.  All pointers are caller-owned device buffers. */
+ * synchronisation.  All pointers are caller-owned device buffers.  move_index < 2^56 (HMZ_ERR_INVALID otherwise), the
+ * counter domain of hmz_rng_dirichlet. */
 typedef struct hmz_selfplay {
   hmz_search_t search;      /* root_prior_is_f64 must equal (dirichlet_alpha > 0 && exploration_eps > 0) */
   const void* weights;      /* hmz_weights_pack blob */

@@ -14,6 +14,9 @@ namespace hmz {
 
 static_assert(sizeof(hmz_move_record_t) == 32, "wire record (include/hmz.h) must be 32 bytes");
 
+// Counters of the Dirichlet streams stay below 2^56: bits 32-55 become bits 8-31 of c3 below, bits 56-63 would be lost.
+constexpr uint64_t kDirichletCounterLimit = 1ull << 56;
+
 struct PhiloxStream {  // sequential 32-bit draws from one (key, item) Philox stream
   uint32_t c0, c1, c2, c3, k0, k1;
   Philox4 buf;
@@ -279,6 +282,8 @@ extern "C" {
 
 int hmz_rng_dirichlet(double* out, int64_t n, double alpha, uint64_t seed, uint64_t counter, uint64_t item_offset, void* stream) {
   ProfScope prof_scope(HMZ_PROF_OTHER, stream);
+  if (counter >= kDirichletCounterLimit)
+    return fail(HMZ_ERR_INVALID, "hmz_rng_dirichlet: counter %llu is not below 2^56", (unsigned long long)counter);
   if (n == 0) return HMZ_OK;
   if (!out || n < 0 || !(alpha > 0.0)) return fail(HMZ_ERR_INVALID, "hmz_rng_dirichlet: bad arguments");
   rng_dirichlet<<<grid_for(n, 256, 4), 256, 0, (cudaStream_t)stream>>>(out, n, alpha, seed, counter, item_offset);
@@ -314,6 +319,8 @@ int hmz_debug_philox(const uint32_t* counters_keys, uint32_t* out, int n_blocks,
 // Four launches around the search: no host synchronisation, everything on `stream`.
 int hmz_selfplay_move(const hmz_selfplay_t* sp, uint64_t move_index, void* stream) {
   if (!sp) return fail(HMZ_ERR_INVALID, "hmz_selfplay_move: null descriptor");
+  if (move_index >= kDirichletCounterLimit)
+    return fail(HMZ_ERR_INVALID, "hmz_selfplay_move: move_index %llu is not below 2^56", (unsigned long long)move_index);
   const hmz_search_t* s = &sp->search;
   const int64_t B = s->n_searches;
   if (B == 0) return HMZ_OK;

@@ -87,3 +87,20 @@ def test_weight_sets_blob_layout(lib, mode):
         assert np.array_equal(blob[k * ws.stride: k * ws.stride + need], pack_host(sd, 4, mode))
         assert not blob[k * ws.stride + need: (k + 1) * ws.stride].any()
     assert not np.array_equal(blob[:need], blob[ws.stride: ws.stride + need])
+
+
+def test_dirichlet_counter_domain_without_gpu(lib):
+    """The Dirichlet streams keep the draw's block in the low 8 bits of Philox counter word 3, above counter bits 32-55:
+    hmz_rng_dirichlet and hmz_selfplay_move reject counters from 2^56 on, before any CUDA call."""
+    from muzero_hanoi_b200 import _lib
+
+    for counter in (1 << 56, (1 << 64) - 1):
+        assert lib.hmz_rng_dirichlet(None, 0, 0.25, 0, counter, 0, None) == _lib.ERR_INVALID and b"2^56" in lib.hmz_last_error()
+        assert lib.hmz_selfplay_move(ctypes.byref(_lib.SelfPlayDesc()), counter, None) == _lib.ERR_INVALID
+        assert b"2^56" in lib.hmz_last_error()
+    assert lib.hmz_rng_dirichlet(None, 4, 0.25, 0, (1 << 56) - 1, 0, None) == _lib.ERR_INVALID
+    assert b"bad arguments" in lib.hmz_last_error()  # the largest counter allowed passes the domain check
+    sp = _lib.SelfPlayDesc()
+    sp.search.n_searches = 4
+    assert lib.hmz_selfplay_move(ctypes.byref(sp), (1 << 56) - 1, None) == _lib.ERR_INVALID
+    assert b"null buffer" in lib.hmz_last_error()

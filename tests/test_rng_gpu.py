@@ -3,7 +3,9 @@
 The reference draws np.random.dirichlet (MCTS/mcts.py:149) and np.random.choice (:120) from NumPy's global Mersenne
 twister; the batched engine cannot reproduce that stream (parity mode takes the draws as INPUTS instead), so the
 on-device generator is validated for what it is: Philox4x32-10 against the published known-answer vectors, the uniform
-and Dirichlet laws by their moments, and the keying by GLOBAL game id (results invariant to the sharding, SURVEY.md §8e).
+and Dirichlet moments, and the keying by GLOBAL game id (results invariant to the sharding, SURVEY.md §8e).  Every draw
+is also compared element by element with oracle/move_ref.py's restatement, and the laws with their exact CDFs, in
+tests/test_move_reference_{cpu,gpu}.py.
 """
 import ctypes as C
 
@@ -12,19 +14,9 @@ import pytest
 import torch
 
 from oracle import cport, port
+from oracle.move_ref import philox_host as _philox_host
 
 pytestmark = pytest.mark.gpu
-
-
-def _philox_host(c, k):
-    """Philox4x32-10 (Salmon, Moraes, Dror, Shaw 2011) restated with Python integers."""
-    M0, M1, W0, W1 = 0xD2511F53, 0xCD9E8D57, 0x9E3779B9, 0xBB67AE85
-    c, k = list(c), list(k)
-    for _ in range(10):
-        p0, p1 = M0 * c[0], M1 * c[2]
-        c = [(p1 >> 32) ^ c[1] ^ k[0], p1 & 0xFFFFFFFF, (p0 >> 32) ^ c[3] ^ k[1], p0 & 0xFFFFFFFF]
-        k = [(k[0] + W0) & 0xFFFFFFFF, (k[1] + W1) & 0xFFFFFFFF]
-    return c
 
 
 # Random123 kat_vectors, philox4x32 with 10 rounds: (counter, key) -> output
